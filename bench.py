@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the classic-control hot path on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline (`value`, `roofline`, `e2e`): a "step" is ONE mgym_step launch over 2^24 CartPole-v1 envs per GPU with
@@ -100,7 +100,13 @@ def parse_args():
     ap.add_argument("--only-configs", default="", help="comma-separated sub-config names (default: all)")
     ap.add_argument("--config-seconds", type=float, default=0.2, help="one timed window of a sub-config (3 are taken)")
     ap.add_argument("--scale", type=float, default=1.0, help="shrink every sub-config (smoke runs on small GPUs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0's envs, a fixed "
+                         "sample of at most 2^20 of them) as DIR/<name>.npy, so that two builds can be compared")
+    args = ap.parse_args()
+    if args.dump_outputs is not None and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native: the reference arm returns no arrays")
+    return args
 
 
 # -------------------------------------------------------------------------------------------------
@@ -487,6 +493,34 @@ def run_mixed_suite(ctx, m, args, native_comm):
     return out, launches
 
 
+DUMP_MAX_ENVS = 1 << 20  # 16 + 4 + 4 + 4 + 8 bytes per sampled env: 36 MB at most
+DUMP_SAMPLE_SEED = 0x5EED
+
+
+def dump_step_outputs(torch, info, n, env_index_base, out_dir):
+    """The StepInfo a caller of env.step received from the last timed step -- observation, reward, terminated,
+    truncated -- for a fixed, seeded sample of the envs (every env when n <= DUMP_MAX_ENVS), as float32 .npy files,
+    plus the global index of each sampled env (float64, exact below 2^53)."""
+    import numpy as np
+
+    if n <= DUMP_MAX_ENVS:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(n, DUMP_MAX_ENVS, replace=False))
+    sel = torch.from_numpy(idx).to(info.reward.device)
+    obs, reward, done, truncated = info
+    arrays = {
+        "obs": obs.index_select(1, sel).cpu().numpy(),
+        "reward": reward.index_select(0, sel).cpu().numpy(),
+        "terminated": done.index_select(0, sel).to(torch.float32).cpu().numpy(),
+        "truncated": truncated.index_select(0, sel).to(torch.float32).cpu().numpy(),
+        "env_index": (idx + env_index_base).astype(np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def measure_host_link(ctx, nbytes=256 << 20, reps=4):
     """Pinned-memory copy ceilings of THIS box, all ranks copying at once: D2H alone, H2D alone, and both directions
     concurrently on two streams.  GB/s per GPU (max-over-ranks time) and aggregated over the ranks."""
@@ -578,11 +612,12 @@ def run_native(args, rank, local_rank, world):
     gen.manual_seed(1234 + rank)
     pool = [torch.randint(0, 2, (n,), dtype=torch.uint8, device=device, generator=gen) for _ in range(16)]
     step_i = [0]
+    last = [None]
 
     def one_step():
         # the public call: Gym::step.  For CartPole the returned observation is a view of the resident state rows
         # (obs_out = NULL in the C call), reward and flags go to the env's own buffers.
-        env.step(pool[step_i[0] & 15])
+        last[0] = env.step(pool[step_i[0] & 15])
         step_i[0] += 1
 
     warmup = max(args.warmup, 3)
@@ -592,6 +627,9 @@ def run_native(args, rank, local_rank, world):
     ms_max, clocks = ctx.timed(one_step, args.steps)
     ms_max *= 1e3
     gpu_launches = args.steps
+    if args.dump_outputs is not None and rank == 0:
+        # before anything else runs on this env: the returned tensors are views of buffers the next step overwrites
+        dump_step_outputs(torch, last[0], n, begin, args.dump_outputs)
 
     # the statistics collective: torch.distributed (NCCL) and, at N > 1, the C ABI's own NCCL entry point
     native_comm, native = None, "not run (single rank: no communicator)"
@@ -711,6 +749,7 @@ def run_native(args, rank, local_rank, world):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the benchmark may run from a read-only checkout: it writes nothing into the tree
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

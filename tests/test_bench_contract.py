@@ -67,6 +67,37 @@ def test_clock_records_are_cut_from_one_sampler_by_wall_clock_window():
     assert short["samples"] == 1 and "nearest" in short["note"]
 
 
+def test_dump_outputs_writes_a_fixed_sample_of_the_last_step(tmp_path):
+    """--dump-outputs: what env.step returned, as float32/float64 .npy files under 64 MB, the same sample every run."""
+    import numpy as np
+
+    torch = __import__("pytest").importorskip("torch")
+    from modurl_gym_b200.vec_env import StepInfo
+
+    b = _bench_module()
+    n, base = 3 * b.DUMP_MAX_ENVS + 5, 7 << 24
+    gen = torch.Generator().manual_seed(1)
+    obs, reward = torch.rand((4, n), generator=gen), torch.rand(n, generator=gen)
+    flags = torch.randint(0, 4, (n,), dtype=torch.uint8, generator=gen)
+    for d in ("a", "b"):
+        b.dump_step_outputs(torch, StepInfo(obs, reward, flags), n, base, str(tmp_path / d))
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["env_index.npy", "obs.npy", "reward.npy", "terminated.npy", "truncated.npy"]
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert np.array_equal(got[f[:-4]], np.load(tmp_path / "b" / f))
+        assert got[f[:-4]].dtype in (np.float32, np.float64)
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    idx = got["env_index"].astype(np.int64) - base
+    assert len(idx) == b.DUMP_MAX_ENVS and np.all(np.diff(idx) > 0) and idx[-1] < n
+    assert np.array_equal(got["obs"], obs.numpy()[:, idx]) and np.array_equal(got["reward"], reward.numpy()[idx])
+    assert np.array_equal(got["terminated"], (flags.numpy()[idx] & 1).astype(np.float32))
+    assert np.array_equal(got["truncated"], (flags.numpy()[idx] >> 1 & 1).astype(np.float32))
+    small = tmp_path / "small"
+    b.dump_step_outputs(torch, StepInfo(obs[:, :10], reward[:10], flags[:10]), 10, 0, str(small))
+    assert np.array_equal(np.load(small / "env_index.npy"), np.arange(10.0))
+
+
 def test_statistics_comparison_tolerates_only_the_float_sum():
     torch = __import__("pytest").importorskip("torch")
     b = _bench_module()
