@@ -168,6 +168,30 @@ impl GpuVecEnv {
         assert_eq!(state_soa.len(), sd * self.num_envs as usize, "state: state_dim * N floats");
         check(unsafe { sys::mgym_set_state(self.h, state_soa.as_ptr(), ptr::null(), ptr::null(), self.stream) })
     }
+    /// Number of per-env physics parameters of this kind (0 for Acrobot).
+    pub fn num_params(&self) -> usize { unsafe { sys::mgym_num_params(self.kind as i32).max(0) as usize } }
+    /// Per-env physics parameters from a HOST array of num_params * N floats, parameter-major; `None` returns to
+    /// the kind's constants.  Rejected values leave the handle untouched.
+    pub fn set_params(&mut self, params_soa: Option<&[f32]>) -> Result<(), MgymError> {
+        let p = match params_soa {
+            Some(p) => {
+                assert_eq!(p.len(), self.num_params() * self.num_envs as usize, "params: num_params * N floats");
+                p.as_ptr()
+            }
+            None => ptr::null(),
+        };
+        check(unsafe { sys::mgym_set_params(self.h, p, self.stream) })
+    }
+    pub fn get_params(&mut self) -> Result<Vec<f32>, MgymError> {
+        let mut v = vec![0f32; self.num_params() * self.num_envs as usize];
+        check(unsafe { sys::mgym_get_params(self.h, v.as_mut_ptr(), self.stream) })?;
+        Ok(v)
+    }
+    /// Draws each env's parameters (those with mask[i] != 0; `mask` a device u8[N] or null) from [low, high).
+    pub fn sample_params(&mut self, low: &[f32], high: &[f32], mask: *const u8, key: u64) -> Result<(), MgymError> {
+        assert!(low.len() == self.num_params() && high.len() == self.num_params(), "low, high: num_params each");
+        check(unsafe { sys::mgym_sample_params(self.h, low.as_ptr(), high.as_ptr(), mask, key, self.stream) })
+    }
     pub fn stats(&mut self) -> Result<sys::mgym_stats, MgymError> {
         let mut s = sys::mgym_stats::default();
         check(unsafe { sys::mgym_stats_get(self.h, &mut s, self.stream) })?;

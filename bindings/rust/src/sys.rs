@@ -80,6 +80,13 @@ extern "C" {
     pub fn mgym_sample_actions(env: *mut mgym_env, actions_out: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn mgym_step_host(env: *mut mgym_env, actions_host: *const c_void, obs_host: *mut f32,
                           reward_host: *mut f32, flags_host: *mut u8, stream: *mut c_void) -> c_int;
+    pub fn mgym_num_params(kind: c_int) -> c_int;
+    pub fn mgym_param_name(kind: c_int, i: c_int) -> *const c_char;
+    pub fn mgym_param_defaults(kind: c_int, out: *mut f32) -> c_int;
+    pub fn mgym_set_params(env: *mut mgym_env, params: *const f32, stream: *mut c_void) -> c_int;
+    pub fn mgym_get_params(env: *mut mgym_env, out: *mut f32, stream: *mut c_void) -> c_int;
+    pub fn mgym_sample_params(env: *mut mgym_env, low: *const f32, high: *const f32, mask: *const u8, key: u64,
+                              stream: *mut c_void) -> c_int;
     pub fn mgym_stats_get(env: *mut mgym_env, out: *mut mgym_stats, stream: *mut c_void) -> c_int;
     pub fn mgym_stats_reset(env: *mut mgym_env, stream: *mut c_void) -> c_int;
     pub fn mgym_stats_export(env: *mut mgym_env, device_vec5_out: *mut f64, stream: *mut c_void) -> c_int;

@@ -176,8 +176,9 @@ int mgym_get_obs(mgym_env *env, float *obs_out, void *stream); /* current observ
 float *mgym_state_ptr(mgym_env *env);
 
 /* Checkpoint / resume: the whole handle (state rows, counters, running returns, statistics, step and reset
- * indices) as one opaque HOST blob.  mgym_checkpoint_size gives the byte count; a handle created with the same
- * kind, num_envs and config continues bit-identically after mgym_checkpoint_load. */
+ * indices, per-env parameters if set) as one opaque HOST blob.  mgym_checkpoint_size gives the byte count; a handle
+ * created with the same kind, num_envs and config continues bit-identically after mgym_checkpoint_load, which
+ * restores exactly the parameters the blob carries (a blob without them clears the handle's). */
 size_t mgym_checkpoint_size(const mgym_env *env);
 int mgym_checkpoint_save(mgym_env *env, void *host_blob, size_t blob_bytes, void *stream);
 int mgym_checkpoint_load(mgym_env *env, const void *host_blob, size_t blob_bytes, void *stream);
@@ -204,6 +205,36 @@ int mgym_sample_actions(mgym_env *env, void *actions_out, void *stream);
  * H2D actions, step, D2H results, synchronises the stream.  Any output may be NULL. */
 int mgym_step_host(mgym_env *env, const void *actions_host, float *obs_host, float *reward_host,
                    uint8_t *flags_host, void *stream);
+
+/* ---- per-env physics parameters (domain randomisation, system identification) ------------
+ * A handle may carry one row per parameter, SoA float[P][N] (P = mgym_num_params), owned by the handle and
+ * allocated on first use.  Without them every env runs the kind's constants (the defaults below) on the same
+ * kernels as before, bit for bit; with them step, rollout and step_host read each env's own constants.
+ * Derived constants are computed per env in f32 in the host's operation order, so defaults set explicitly give
+ * the same bits as no parameters.  Termination thresholds, spaces, time limits and reset distributions do not
+ * depend on parameters.
+ *   CartPole-v1               gravity 9.8, masscart 1.0, masspole 0.1, length 0.5 (half-pole), force_mag 10.0,
+ *                             tau 0.02 (masses, length and tau > 0)
+ *   MountainCar-v0            force 0.001, gravity 0.0025
+ *   MountainCarContinuous-v0  power 0.0015, gravity 0.0025
+ *   Pendulum-v1               g 10.0, m 1.0, l 1.0 (m, l > 0)
+ *   Acrobot-v1                none (P = 0; mgym_set_params / mgym_sample_params return MGYM_ERR_BAD_ARGUMENT)
+ * Every parameter must be finite. */
+int mgym_num_params(int kind);                      /* P, or a negative status for an unknown kind */
+const char *mgym_param_name(int kind, int i);       /* NULL outside [0, P) */
+int mgym_param_defaults(int kind, float *out);      /* P floats */
+/* params: [P][N], host or device; NULL = back to the constants.  Checked before anything is copied: a rejected
+ * set returns MGYM_ERR_BAD_ARGUMENT and leaves the handle untouched.  Synchronises; not capturable. */
+int mgym_set_params(mgym_env *env, const float *params, void *stream);
+/* out: [P][N], host or device; the defaults when no parameters are set. */
+int mgym_get_params(mgym_env *env, float *out, void *stream);
+/* Draws parameter c of env i uniformly from [low[c], high[c]) (host arrays of P; f64 draw cast to f32, like the
+ * reset states): word c % 4 of the Philox block with counter (global env index, key mod 2^56) and tag 3 + c / 4,
+ * so the draws do not depend on sharding or launch geometry.  mask (device uint8[N] or NULL) limits the draw to
+ * envs with mask[i] != 0 -- per-episode randomisation is `mask = flags != 0` after a step.  Rows not set before
+ * start from the defaults.  Capturable into a CUDA graph once the rows exist (the key is the caller's). */
+int mgym_sample_params(mgym_env *env, const float *low, const float *high, const uint8_t *mask, uint64_t key,
+                       void *stream);
 
 /* ---- statistics --------------------------------------------------------------------- */
 int mgym_stats_get(mgym_env *env, mgym_stats_t *out, void *stream); /* synchronises */

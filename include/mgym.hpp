@@ -175,6 +175,25 @@ class GpuVecEnv {
     check(mgym_get_state(h_, state_soa.data(), steps.data(), sbt.data(), stream_));
     sync();
   }
+  // ---- per-env physics parameters (domain randomisation) ------------------------------------------------
+  static int num_params(int kind) { return mgym_num_params(kind); }
+  // params_soa: [P][N] on the host or the device; nullptr returns to the kind's constants
+  void set_params(const float* params_soa) {
+    check(mgym_set_params(h_, params_soa, stream_));
+  }
+  std::vector<float> get_params() {
+    std::vector<float> v((size_t)mgym_num_params(kind_) * n_);
+    check(mgym_get_params(h_, v.data(), stream_));
+    return v;
+  }
+  // low, high: P values each; mask_device: uint8[N] or nullptr
+  void sample_params(const std::vector<float>& low, const std::vector<float>& high,
+                     const uint8_t* mask_device = nullptr, uint64_t key = 0) {
+    if ((int)low.size() != mgym_num_params(kind_) || (int)high.size() != mgym_num_params(kind_))
+      throw Error(MGYM_ERR_BAD_ARGUMENT, "sample_params: low and high need num_params values each");
+    check(mgym_sample_params(h_, low.data(), high.data(), mask_device, key, stream_));
+  }
+
   mgym_stats_t stats() {
     mgym_stats_t s{};
     check(mgym_stats_get(h_, &s, stream_));

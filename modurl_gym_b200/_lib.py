@@ -81,6 +81,12 @@ SYMBOLS = {
     "mgym_rollout": (_i, [_vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mgym_sample_actions": (_i, [_vp, _vp, _vp]),
     "mgym_step_host": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "mgym_num_params": (_i, [_i]),
+    "mgym_param_name": (C.c_char_p, [_i, _i]),
+    "mgym_param_defaults": (_i, [_i, _vp]),
+    "mgym_set_params": (_i, [_vp, _vp, _vp]),
+    "mgym_get_params": (_i, [_vp, _vp, _vp]),
+    "mgym_sample_params": (_i, [_vp, _vp, _vp, _vp, _u64, _vp]),
     "mgym_stats_get": (_i, [_vp, C.POINTER(Stats), _vp]),
     "mgym_stats_reset": (_i, [_vp, _vp]),
     "mgym_stats_export": (_i, [_vp, _vp, _vp]),

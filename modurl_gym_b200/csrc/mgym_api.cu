@@ -54,6 +54,7 @@ struct mgym_env {
   uint64_t pool_len = 0;
   unsigned long long* stats = nullptr;  // 5 x 8 bytes
   uint32_t* bad_action = nullptr;
+  float* params = nullptr;  // per-env physics parameters [P][n] (mgym_set_params), null = the kind's constants
 
   uint64_t t = 0;         // steps executed since creation
   uint64_t n_resets = 0;  // explicit reset calls since creation
@@ -115,6 +116,21 @@ constexpr int kContinuous[MGYM_NUM_KINDS] = {0, 0, 1, 1, 0};
 constexpr int kNumActions[MGYM_NUM_KINDS] = {2, 3, 0, 0, 3};
 const char* const kNames[MGYM_NUM_KINDS] = {"CartPole-v1", "MountainCar-v0", "MountainCarContinuous-v0",
                                             "Pendulum-v1", "Acrobot-v1"};
+
+// Per-env physics parameters (mgym_set_params): count, names, defaults (the constants of make_consts and of the
+// device code) and the ones that must be > 0 (bit c = parameter c).  Acrobot has none.
+constexpr int kNumParams[MGYM_NUM_KINDS] = {6, 2, 2, 3, 0};
+const char* const kParamNames[MGYM_NUM_KINDS][6] = {
+    {"gravity", "masscart", "masspole", "length", "force_mag", "tau"},
+    {"force", "gravity"},
+    {"power", "gravity"},
+    {"g", "m", "l"},
+    {}};
+constexpr float kParamDefaults[MGYM_NUM_KINDS][6] = {
+    {9.8f, 1.0f, 0.1f, 0.5f, 10.0f, 0.02f}, {0.001f, 0.0025f}, {0.0015f, 0.0025f}, {10.0f, 1.0f, 1.0f}, {}};
+constexpr uint32_t kParamPositive[MGYM_NUM_KINDS] = {0x2Eu, 0u, 0u, 0x6u, 0u};
+static_assert(Env<0>::NP == 6 && Env<1>::NP == 2 && Env<2>::NP == 2 && Env<3>::NP == 3 && Env<4>::NP == 0,
+              "parameter tables and Env<KIND>::NP disagree");
 
 bool valid_kind(int kind) { return kind >= 0 && kind < MGYM_NUM_KINDS; }
 size_t counter_width(int cnt_mode) {
@@ -234,8 +250,8 @@ struct OccupancyCache {
 };
 OccupancyCache g_occupancy;
 
-int launch_persistent(void (*kernel)(KernelParams), const mgym_env* e, const KernelParams& p, uint64_t groups,
-                      cudaStream_t st) {
+template <typename KP>
+int launch_persistent(void (*kernel)(KP), const mgym_env* e, const KP& p, uint64_t groups, cudaStream_t st) {
   constexpr int threads = 256;
   int per_sm = g_occupancy.find(reinterpret_cast<const void*>(kernel), e->device);
   if (per_sm == 0) {
@@ -254,12 +270,12 @@ int launch_persistent(void (*kernel)(KernelParams), const mgym_env* e, const Ker
 }
 
 // TMA-staged step kernel (auto-reset, vector path, N a multiple of the 128-env warp tile)
-template <int KIND, int CNT, bool AUTO = true>
-int launch_step_tma(const mgym_env* ce, const KernelParams& p_in, cudaStream_t st) {
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false>
+int launch_step_tma(const mgym_env* ce, const KParams<PARAMS>& p_in, cudaStream_t st) {
   mgym_env* e = const_cast<mgym_env*>(ce);  // ticket accounting
-  KernelParams p = p_in;
-  using L = TmaLayout<KIND, CNT, AUTO>;
-  auto kernel = step_kernel_tma<KIND, CNT, AUTO>;
+  KParams<PARAMS> p = p_in;
+  using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
+  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS>;
   constexpr int threads = TMA_THREADS;
   // the opt-in to > 48 KB of dynamic shared memory and the occupancy are per device
   static int cached_per_sm[kMaxDevices] = {};
@@ -316,36 +332,36 @@ bool use_tma() {
   return v;
 }
 
-// kind x vector width x auto/manual x counter representation
-template <int KIND, int V, bool ROLLOUT>
-int dispatch_mode(const mgym_env* e, const KernelParams& p, cudaStream_t st) {
+// kind x vector width x auto/manual x counter representation (x per-env parameters)
+template <int KIND, int V, bool ROLLOUT, bool PARAMS = false>
+int dispatch_mode(const mgym_env* e, const KParams<PARAMS>& p, cudaStream_t st) {
   const uint64_t groups = p.n / V;
   const bool autor = e->cfg.auto_reset != 0;
   if constexpr (!ROLLOUT && V == 4) {
     // manual mode (the reference's protocol): counters are 32-bit, CartPole adds steps_beyond_terminated
-    if (!autor && use_tma() && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false>(e, p, st);
+    if (!autor && use_tma() && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
     if (autor && use_tma() && p.n % TMA_TILE == 0) {
       if constexpr (KIND == 0) {  // CartPole always counts (500-step truncation, cartpole.rs:297)
-        if (e->cnt_mode == CNT_U16) return launch_step_tma<KIND, CNT_U16>(e, p, st);
-        return launch_step_tma<KIND, CNT_S16>(e, p, st);
+        if (e->cnt_mode == CNT_U16) return launch_step_tma<KIND, CNT_U16, true, PARAMS>(e, p, st);
+        return launch_step_tma<KIND, CNT_S16, true, PARAMS>(e, p, st);
       } else {
         switch (e->cnt_mode) {
-          case CNT_S16: return launch_step_tma<KIND, CNT_S16>(e, p, st);
-          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY>(e, p, st);
-          default: return launch_step_tma<KIND, CNT_S32>(e, p, st);
+          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS>(e, p, st);
+          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS>(e, p, st);
+          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS>(e, p, st);
         }
       }
     }
     if (use_tma() && p.n > TMA_TILE) {
       // ragged size: whole 1024-env tiles on the TMA kernel, the remaining (< 1024) envs on the vector kernel
-      KernelParams head = p, tail = p;
+      KParams<PARAMS> head = p, tail = p;
       head.adv_dt = 0;  // device clock: the tail launch (last of the call) moves the step index on
       head.n = p.n - p.n % TMA_TILE;
       tail.first = p.first + head.n;
       tail.n = p.n - head.n;
-      int rc = dispatch_mode<KIND, 4, false>(e, head, st);
+      int rc = dispatch_mode<KIND, 4, false, PARAMS>(e, head, st);
       if (rc != MGYM_OK) return rc;
-      return dispatch_mode<KIND, 4, false>(e, tail, st);
+      return dispatch_mode<KIND, 4, false, PARAMS>(e, tail, st);
     }
   }
   // rollout_kernel's FULL form: complete warp tiles and all three trajectory outputs
@@ -355,11 +371,11 @@ int dispatch_mode(const mgym_env* e, const KernelParams& p, cudaStream_t st) {
   do {                                                                                                   \
     if constexpr (ROLLOUT) {                                                                             \
       if constexpr (AUTO_ && V == 4) {                                                                   \
-        if (full) return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true>, e, p, groups, st); \
+        if (full) return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS>, e, p, groups, st); \
       }                                                                                                  \
-      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false>, e, p, groups, st);           \
+      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS>, e, p, groups, st);   \
     } else {                                                                                             \
-      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_>, e, p, groups, st);                     \
+      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS>, e, p, groups, st);             \
     }                                                                                                    \
   } while (0)
   if (!autor) MGYM_LAUNCH(false, CNT_U32);
@@ -375,11 +391,25 @@ int dispatch_mode(const mgym_env* e, const KernelParams& p, cudaStream_t st) {
 #undef MGYM_LAUNCH
 }
 
+// A handle with per-env parameters runs the PARAMS instantiations (kinds that have parameters only).
+template <int KIND, bool ROLLOUT>
+int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
+  if constexpr (Env<KIND>::NP > 0) {
+    if (e->params) {
+      KernelParamsP pp;
+      static_cast<KernelParams&>(pp) = p;
+      pp.params = e->params;
+      return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true>(e, pp, st) : dispatch_mode<KIND, 1, ROLLOUT, true>(e, pp, st);
+    }
+  }
+  return vec4 ? dispatch_mode<KIND, 4, ROLLOUT>(e, p, st) : dispatch_mode<KIND, 1, ROLLOUT>(e, p, st);
+}
+
 template <bool ROLLOUT>
 int dispatch(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
 #define MGYM_KIND(K_)                                               \
   case K_:                                                          \
-    return vec4 ? dispatch_mode<K_, 4, ROLLOUT>(e, p, st) : dispatch_mode<K_, 1, ROLLOUT>(e, p, st)
+    return dispatch_kind<K_, ROLLOUT>(e, p, vec4, st)
   switch (e->kind) {
     MGYM_KIND(0);
     MGYM_KIND(1);
@@ -573,6 +603,7 @@ int mgym_destroy(mgym_env* e) {
   cudaFree(e->reset_pool);
   cudaFree(e->stats);
   cudaFree(e->bad_action);
+  cudaFree(e->params);
   cudaFree(e->h_actions);
   cudaFree(e->h_obs);
   cudaFree(e->h_reward);
@@ -866,7 +897,7 @@ struct CheckpointHeader {
   int32_t kind, cnt_mode, auto_reset, has_sbt, has_ret;
   int32_t is_euler, sutton_barto, max_episode_steps, track_stats;
   float goal_velocity;
-  uint32_t pad0;
+  uint32_t has_params;  // 1: the per-env parameter rows follow the statistics
   uint64_t n, seed, t, n_resets, env_index_base, pool_len;
 };
 constexpr uint32_t kCkptMagic = 0x4D47594Du;  // "MGYM"
@@ -883,18 +914,23 @@ CheckpointHeader checkpoint_header(const mgym_env* e) {
   h.goal_velocity = e->cfg.goal_velocity;
   h.n = e->n, h.seed = e->seed, h.t = e->t, h.n_resets = e->n_resets;
   h.env_index_base = e->cfg.env_index_base, h.pool_len = e->pool_len;
+  h.has_params = e->params ? 1u : 0u;
   return h;
 }
 
 size_t counter_bytes(const mgym_env* e) { return counter_width(e->cnt_mode) * (size_t)e->n; }
-}  // namespace
+size_t param_bytes(const mgym_env* e) { return sizeof(float) * kNumParams[e->kind] * (size_t)e->n; }
 
-size_t mgym_checkpoint_size(const mgym_env* e) {
-  if (!e) return 0;
+// size of a blob of this handle that carries parameter rows or not
+size_t checkpoint_bytes(const mgym_env* e, bool with_params) {
   const size_t n = (size_t)e->n;
   return sizeof(CheckpointHeader) + sizeof(float) * kStateDim[e->kind] * n + counter_bytes(e) +
-         (e->sbt ? sizeof(uint32_t) * n : 0) + (e->ep_return ? sizeof(float) * n : 0) + 5 * sizeof(unsigned long long);
+         (e->sbt ? sizeof(uint32_t) * n : 0) + (e->ep_return ? sizeof(float) * n : 0) + 5 * sizeof(unsigned long long) +
+         (with_params ? param_bytes(e) : 0);
 }
+}  // namespace
+
+size_t mgym_checkpoint_size(const mgym_env* e) { return e ? checkpoint_bytes(e, e->params != nullptr) : 0; }
 
 int mgym_checkpoint_save(mgym_env* e, void* blob, size_t blob_bytes, void* stream) {
   if (!e || !blob) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_checkpoint_save: NULL argument");
@@ -918,6 +954,7 @@ int mgym_checkpoint_save(mgym_env* e, void* blob, size_t blob_bytes, void* strea
   if ((rc = pull(e->sbt, e->sbt ? sizeof(uint32_t) * n : 0))) return rc;
   if ((rc = pull(e->ep_return, e->ep_return ? sizeof(float) * n : 0))) return rc;
   if ((rc = pull(e->stats, 5 * sizeof(unsigned long long)))) return rc;
+  if ((rc = pull(e->params, e->params ? param_bytes(e) : 0))) return rc;
   MGYM_CUDA(cudaStreamSynchronize(st));
   return MGYM_OK;
 }
@@ -945,8 +982,11 @@ int mgym_checkpoint_load(mgym_env* e, const void* blob, size_t blob_bytes, void*
                 h.track_stats, mine.track_stats, (double)h.goal_velocity, (double)mine.goal_velocity,
                 (unsigned long long)h.env_index_base, (unsigned long long)mine.env_index_base,
                 (unsigned long long)h.pool_len, (unsigned long long)mine.pool_len);
-  if (blob_bytes < mgym_checkpoint_size(e)) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_checkpoint_load: truncated blob");
+  // a blob restores exactly the parameters it carries; one without parameter rows clears the handle's
+  const bool with_params = h.has_params != 0 && kNumParams[e->kind] > 0;
+  if (blob_bytes < checkpoint_bytes(e, with_params)) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_checkpoint_load: truncated blob");
   DeviceGuard guard(e->device);
+  if (with_params && !e->params) MGYM_CUDA(cudaMalloc(&e->params, param_bytes(e)));
   cudaStream_t st = (cudaStream_t)stream;
   const size_t n = (size_t)e->n;
   const uint8_t* in = static_cast<const uint8_t*>(blob) + sizeof(h);
@@ -961,7 +1001,12 @@ int mgym_checkpoint_load(mgym_env* e, const void* blob, size_t blob_bytes, void*
   if ((rc = push(e->sbt, e->sbt ? sizeof(uint32_t) * n : 0))) return rc;
   if ((rc = push(e->ep_return, e->ep_return ? sizeof(float) * n : 0))) return rc;
   if ((rc = push(e->stats, 5 * sizeof(unsigned long long)))) return rc;
+  if ((rc = push(e->params, with_params ? param_bytes(e) : 0))) return rc;
   MGYM_CUDA(cudaStreamSynchronize(st));
+  if (!with_params) {
+    cudaFree(e->params);
+    e->params = nullptr;
+  }
   e->seed = h.seed;
   e->t = h.t;
   if (e->cfg.device_clock) {
@@ -1046,6 +1091,140 @@ int mgym_sample_actions(mgym_env* e, void* actions_out, void* stream) {
     case 3: sample_actions_kernel<3><<<blocks, 256, 0, st>>>((float*)actions_out, e->n, e->seed, base, e->t, td); break;
     default: sample_actions_kernel<4><<<blocks, 256, 0, st>>>((uint8_t*)actions_out, e->n, e->seed, base, e->t, td); break;
   }
+  MGYM_CUDA(cudaGetLastError());
+  return MGYM_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// per-env physics parameters
+// ---------------------------------------------------------------------------------------------
+int mgym_num_params(int kind) { return valid_kind(kind) ? kNumParams[kind] : MGYM_ERR_BAD_ARGUMENT; }
+
+const char* mgym_param_name(int kind, int i) {
+  return (valid_kind(kind) && i >= 0 && i < kNumParams[kind]) ? kParamNames[kind][i] : nullptr;
+}
+
+int mgym_param_defaults(int kind, float* out) {
+  if (!valid_kind(kind) || !out) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_param_defaults: bad argument");
+  for (int c = 0; c < kNumParams[kind]; ++c) out[c] = kParamDefaults[kind][c];
+  return MGYM_OK;
+}
+
+namespace {
+int no_params(const mgym_env* e, const char* what) {
+  return fail(MGYM_ERR_BAD_ARGUMENT,
+              "%s: %s has no per-env parameters (its RK4 runs on constants folded on the host; see DESIGN.md)", what,
+              kNames[e->kind]);
+}
+ParamVec param_defaults(int kind) {
+  ParamVec d{};
+  for (int c = 0; c < kNumParams[kind]; ++c) d.v[c] = kParamDefaults[kind][c];
+  return d;
+}
+// the handle's parameter rows, allocated and filled with the defaults on first use
+int ensure_params(mgym_env* e, cudaStream_t st) {
+  if (e->params) return MGYM_OK;
+  float* rows = nullptr;
+  MGYM_CUDA(cudaMalloc(&rows, param_bytes(e)));
+  fill_params_kernel<<<(unsigned)((e->n + 255) / 256), 256, 0, st>>>(rows, e->n, kNumParams[e->kind],
+                                                                     param_defaults(e->kind));
+  cudaError_t err = cudaGetLastError();
+  if (err != cudaSuccess) {
+    cudaFree(rows);
+    return fail(MGYM_ERR_CUDA, "ensure_params: %s", cudaGetErrorString(err));
+  }
+  e->params = rows;
+  return MGYM_OK;
+}
+}  // namespace
+
+int mgym_set_params(mgym_env* e, const float* params, void* stream) {
+  if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_set_params: env is NULL");
+  if (kNumParams[e->kind] == 0) return no_params(e, "mgym_set_params");
+  DeviceGuard guard(e->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = refuse_capture(e, st, "mgym_set_params", false)) return rc;
+  MGYM_CUDA(cudaStreamSynchronize(st));  // in-flight launches may still read the rows
+  if (!params) {
+    cudaFree(e->params);
+    e->params = nullptr;
+    return MGYM_OK;
+  }
+  const int np = kNumParams[e->kind];
+  const uint64_t n = e->n;
+  // the "must hold" conditions, checked before anything is copied: a rejected set leaves the handle untouched
+  bool bad = false;
+  if (is_host_pointer(params)) {  // host rows are scanned on the host, as mgym_step_host scans host actions
+    for (uint64_t i = 0; i < (uint64_t)np * n && !bad; ++i) {
+      const float x = params[i];
+      bad = !std::isfinite(x) || (((kParamPositive[e->kind] >> (i / n)) & 1u) && !(x > 0.0f));
+    }
+  } else {
+    uint64_t blocks = ((uint64_t)np * n + 255) / 256;
+    if (blocks > (uint64_t)e->num_sms * 8) blocks = (uint64_t)e->num_sms * 8;
+    MGYM_CUDA(cudaMemsetAsync(e->bad_action, 0, sizeof(uint32_t), st));
+    validate_params_kernel<<<(unsigned)blocks, 256, 0, st>>>(params, n, np, kParamPositive[e->kind], e->bad_action);
+    MGYM_CUDA(cudaGetLastError());
+    uint32_t flag = 0;
+    MGYM_CUDA(cudaMemcpyAsync(&flag, e->bad_action, sizeof(flag), cudaMemcpyDeviceToHost, st));
+    MGYM_CUDA(cudaStreamSynchronize(st));
+    bad = flag != 0;
+  }
+  if (bad)
+    return fail(MGYM_ERR_BAD_ARGUMENT,
+                "mgym_set_params: a %s parameter is not finite, or a mass, length or time step is not > 0; nothing "
+                "was changed", kNames[e->kind]);
+  if (!e->params) MGYM_CUDA(cudaMalloc(&e->params, param_bytes(e)));
+  MGYM_CUDA(cudaMemcpyAsync(e->params, params, param_bytes(e), cudaMemcpyDefault, st));
+  MGYM_CUDA(cudaStreamSynchronize(st));
+  return MGYM_OK;
+}
+
+int mgym_get_params(mgym_env* e, float* out, void* stream) {
+  if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_get_params: env is NULL");
+  if (kNumParams[e->kind] == 0) return MGYM_OK;  // nothing to write
+  if (!out) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_get_params: out is NULL");
+  DeviceGuard guard(e->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int np = kNumParams[e->kind];
+  const bool host = is_host_pointer(out);
+  if (e->params) {
+    MGYM_CUDA(cudaMemcpyAsync(out, e->params, param_bytes(e), cudaMemcpyDefault, st));
+    if (host) MGYM_CUDA(cudaStreamSynchronize(st));
+  } else if (host) {
+    for (int c = 0; c < np; ++c)
+      for (uint64_t i = 0; i < e->n; ++i) out[(uint64_t)c * e->n + i] = kParamDefaults[e->kind][c];
+  } else {
+    fill_params_kernel<<<(unsigned)((e->n + 255) / 256), 256, 0, st>>>(out, e->n, np, param_defaults(e->kind));
+    MGYM_CUDA(cudaGetLastError());
+  }
+  return MGYM_OK;
+}
+
+int mgym_sample_params(mgym_env* e, const float* low, const float* high, const uint8_t* mask, uint64_t key,
+                       void* stream) {
+  if (!e || !low || !high) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_sample_params: NULL argument");
+  if (kNumParams[e->kind] == 0) return no_params(e, "mgym_sample_params");
+  DeviceGuard guard(e->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int np = kNumParams[e->kind];
+  ParamBox box{};
+  for (int c = 0; c < np; ++c) {
+    const bool pos = (kParamPositive[e->kind] >> c) & 1u;
+    if (!std::isfinite(low[c]) || !std::isfinite(high[c]) || !(low[c] <= high[c]) || (pos && !(low[c] > 0.0f)))
+      return fail(MGYM_ERR_BAD_ARGUMENT,
+                  "mgym_sample_params: bad range for %s %s: [%g, %g] (finite, low <= high%s)", kNames[e->kind],
+                  kParamNames[e->kind][c], (double)low[c], (double)high[c], pos ? ", low > 0" : "");
+    box.lo[c] = (double)low[c];
+    box.range[c] = (double)high[c] - (double)low[c];
+  }
+  // capturable: the key is the caller's launch argument, nothing depends on host state once the rows exist
+  if (!e->params && is_capturing(st))
+    return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_sample_params: set or sample the parameters once before capturing "
+                "(the rows are allocated on first use)");
+  if (int rc = ensure_params(e, st)) return rc;
+  sample_params_kernel<<<(unsigned)((e->n + 255) / 256), 256, 0, st>>>(e->params, e->n, np, mask, e->seed,
+                                                                       e->cfg.env_index_base, key, box);
   MGYM_CUDA(cudaGetLastError());
   return MGYM_OK;
 }

@@ -112,6 +112,22 @@ struct KernelParams {
   PhiloxKeys keys;  // round keys of `seed`
   EnvConsts k;
 };
+// The launch parameters of the kernels instantiated with PARAMS: the handle's per-env physics parameters [NP][ld]
+// (mgym_set_params) on top.  A separate type, so that KernelParams -- and every kernel that takes it by value,
+// with the arguments after it -- stays exactly as it is.
+struct KernelParamsP : KernelParams {
+  const float* params;
+};
+template <bool PARAMS>
+using KParams = std::conditional_t<PARAMS, KernelParamsP, KernelParams>;
+
+// The per-env parameters of a lane's V envs, [NP][V] (r[c][v] = parameter c of slot v).  NP = 0: none.
+template <int NP_, int V>
+struct ParamRows {
+  static constexpr int NP = NP_;
+  float r[NP_ > 0 ? NP_ : 1][V];
+};
+using NoParams = ParamRows<0, 1>;
 
 __device__ __forceinline__ uint64_t launch_t(const KernelParams& p) { return p.t_dev ? *p.t_dev : p.t; }
 __device__ __forceinline__ uint64_t launch_work_base(const KernelParams& p) {
@@ -411,16 +427,41 @@ __device__ __noinline__ LaneIO<KIND, V> dynamics_reference_lane(LaneIO<KIND, V> 
 // TRUSTED (kinds with Env::HAS_TRUSTED): the caller has established Env::trusted_entry for every slot, which the
 // dynamics themselves then preserve, so the fast form runs without its per-step precondition test.
 // OBS_VALID (kinds with Env::HAS_OBS_CACHE): g.obs is the observation of the state in g.st on entry.
+// PR (ParamRows with NP > 0): every env steps with its own constants, prm.r[.][v] (Env::dynamics_p).
 template <int KIND, int V, bool AUTO, bool WANT_FINAL, bool TALLY_LEN = true, int RESET = RESET_IN_PLACE,
-          bool TRUSTED = false, bool OBS_VALID = false, bool BATCH_PAIRS = false>
+          bool TRUSTED = false, bool OBS_VALID = false, bool BATCH_PAIRS = false, typename PR = NoParams>
 __device__ __forceinline__ uint32_t step_group(const KernelParams& p, bool count, uint64_t base, uint64_t t,
                                            const typename Env<KIND>::act_t (&action)[V], bool track_ret,
-                                           Group<KIND, V>& g, StatAcc& acc) {
+                                           Group<KIND, V>& g, StatAcc& acc, const PR& prm = PR{}) {
   using E = Env<KIND>;
   float aux[V];
 #pragma unroll
   for (int v = 0; v < V; ++v) aux[v] = 0.0f;
-  if constexpr (E::HAS_BATCH) {
+  if constexpr (PR::NP > 0) {
+    static_assert(PR::NP == E::NP, "parameter rows of another kind");
+    // Kinds whose fast form does not depend on the constants (PARAM_FAST) keep it, behind the same test of the
+    // step's inputs as below; the others run the reference form with the env's constants.
+    bool fast = false;
+    if constexpr (E::PARAM_FAST) {
+      fast = true;
+      if constexpr (!(TRUSTED && E::HAS_TRUSTED)) {
+#pragma unroll
+        for (int v = 0; v < V; ++v) fast = fast & E::fast_ok(g.st[v], action[v], p.k);
+      }
+    }
+    constexpr bool CACHED = OBS_VALID && E::HAS_OBS_CACHE;
+#pragma unroll
+    for (int v = 0; v < V; ++v) {
+      float pe[E::NP];
+#pragma unroll
+      for (int c = 0; c < E::NP; ++c) pe[c] = prm.r[c][v];
+      const float sin_cached = CACHED ? g.obs[v][E::OD > 1 ? 1 : 0] : 0.0f;
+      if (fast)
+        E::template dynamics_p<true, CACHED>(g.st[v], action[v], p.k, pe, aux[v], sin_cached);
+      else
+        E::template dynamics_p<false, false>(g.st[v], action[v], p.k, pe, aux[v], 0.0f);
+    }
+  } else if constexpr (E::HAS_BATCH) {
     // Acrobot: the RK4 stages test their own intermediates, so the fast form runs first (it writes the state
     // unconditionally) and an env whose test failed is restored from here and redone with the reference form
     bool ok[V];
@@ -571,11 +612,12 @@ __device__ __forceinline__ typename CounterType<CNT>::type cnt_encode(uint32_t s
 // =============================================================================================
 // Mode 1: per-call step kernel
 // =============================================================================================
-template <int KIND, int V, bool AUTO, int CNT>
-__global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid_constant__ KernelParams p) {
+template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false>
+__global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid_constant__ KParams<PARAMS> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
+  using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   constexpr int SD = E::SD, OD = E::OD;
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
@@ -590,6 +632,15 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
     const uint64_t base = p.first + grp * V;
     Group<KIND, V> g;
     act_t action[V];
+    PR prm;
+    if constexpr (PARAMS) {
+#pragma unroll
+      for (int c = 0; c < E::NP; ++c) {
+        const Vec<float, V> r = ldv<float, V>(p.params + (uint64_t)c * p.ld + base);
+#pragma unroll
+        for (int v = 0; v < V; ++v) prm.r[c][v] = r.v[v];
+      }
+    }
     {
       Vec<float, V> s[SD];
 #pragma unroll
@@ -614,9 +665,11 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
       }
     }
     if (want_final)
-      step_group<KIND, V, AUTO, true>(p, true, base, t_now, action, track_ret, g, acc);
+      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, false, PR>(p, true, base, t_now, action,
+                                                                                    track_ret, g, acc, prm);
     else
-      step_group<KIND, V, AUTO, false>(p, true, base, t_now, action, track_ret, g, acc);
+      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, false, PR>(p, true, base, t_now, action,
+                                                                                     track_ret, g, acc, prm);
 
     {
       Vec<float, V> s[SD];
@@ -734,7 +787,10 @@ constexpr int TMA_THREADS = (TMA_CONSUMER_WARPS + 2) * 32;  // + one producer wa
 constexpr int TMA_RESET_BUFFERS = 2;                         // request queues in flight
 constexpr int TMA_TILE = TMA_CONSUMER_WARPS * 32 * 4;       // envs per CTA tile: 256 consumer threads x V=4
 
-template <int KIND, int CNT, bool AUTO = true>
+// PARAMS: the env's NP parameter rows travel with the tile (4 NP bytes per env more).  The stage count is then the
+// largest (up to TMA_STAGES) that still lets two CTAs share an SM: CartPole's 43 KB stage runs 2 stages x 2 CTAs
+// (4 tiles = 172 KB in flight per SM, against 4 x 2 x 19 KB without parameters).
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false>
 struct TmaLayout {
   using E = Env<KIND>;
   static constexpr uint32_t ROW = TMA_TILE * 4;  // one f32 row of a tile
@@ -747,14 +803,22 @@ struct TmaLayout {
   // manual CartPole also carries steps_beyond_terminated (cartpole.rs:27)
   static constexpr uint32_t OFF_SBT = OFF_RET + RET_BYTES;
   static constexpr uint32_t SBT_BYTES = (!AUTO && KIND == 0) ? ROW : 0;
-  static constexpr uint32_t STAGE_BYTES = (OFF_SBT + SBT_BYTES + 127u) & ~127u;
+  static constexpr uint32_t OFF_PAR = OFF_SBT + SBT_BYTES;
+  static constexpr uint32_t PAR_BYTES = PARAMS ? E::NP * ROW : 0;
+  static constexpr uint32_t STAGE_BYTES = (OFF_PAR + PAR_BYTES + 127u) & ~127u;
   static constexpr uint32_t BAR_BYTES = 128;  // full[STAGES], empty[STAGES], tile id of each stage
   static_assert(24 * TMA_STAGES <= 128, "barriers and tile ids must fit BAR_BYTES");
   // reset queues: per buffer {q_full, q_empty mbarriers, tile id, count} (32 B) + per finished env its uint16 index in
   // the tile and the uint32 length of the episode that ended (the reset stream is keyed by its start)
   static constexpr uint32_t QUEUE_STRIDE = 32 + TMA_TILE * 2 + TMA_TILE * 4;
   static constexpr uint32_t QUEUE_BYTES = TMA_RESET_BUFFERS * QUEUE_STRIDE;
-  static constexpr uint32_t OFF_QUEUE = BAR_BYTES + TMA_STAGES * STAGE_BYTES;
+  static constexpr int fit_stages() {
+    const uint32_t budget = 110u * 1024u - 256u - QUEUE_BYTES;  // per CTA, two CTAs per SM
+    const int s = (int)(budget / STAGE_BYTES);
+    return s > TMA_STAGES ? TMA_STAGES : (s < 1 ? 1 : s);
+  }
+  static constexpr int STAGES = PARAMS ? fit_stages() : TMA_STAGES;
+  static constexpr uint32_t OFF_QUEUE = BAR_BYTES + STAGES * STAGE_BYTES;
   static constexpr uint32_t SMEM_BYTES = 128 + OFF_QUEUE + QUEUE_BYTES;
 };
 
@@ -775,13 +839,15 @@ struct TmaLayout {
 // AUTO = false is the reference's own protocol (no same-step reset: the caller resets what finished,
 // cartpole.rs:468-470): the same pipeline with steps_beyond_terminated as one more row and nothing ever queued
 // for the reset warp.
-template <int KIND, int CNT, bool AUTO = true>
-__global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_tma(const __grid_constant__ KernelParams p) {
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false>
+__global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_tma(const __grid_constant__ KParams<PARAMS> p) {
   using E = Env<KIND>;
-  using L = TmaLayout<KIND, CNT, AUTO>;
+  using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
   constexpr int SD = E::SD, OD = E::OD, V = 4;
+  constexpr int TMA_STAGES = L::STAGES;  // shadows the global default: this kernel's own ring depth
+  using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   static_assert(AUTO || !cnt_is_stamp(CNT), "manual mode keeps the reference's own counters");
   static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
   extern __shared__ uint8_t smem_raw[];
@@ -835,7 +901,8 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_
     // tickets [work_base, work_base + n_tiles + gridDim.x): each CTA draws exactly one ticket past the end.
     if (lane == 0) {
       const act_t* actions = reinterpret_cast<const act_t*>(p.actions);
-      const uint32_t tx = SD * L::ROW + L::ACT_BYTES + L::CNT_BYTES + (track_ret ? L::ROW : 0u) + L::SBT_BYTES;
+      const uint32_t tx =
+          SD * L::ROW + L::ACT_BYTES + L::CNT_BYTES + (track_ret ? L::ROW : 0u) + L::SBT_BYTES + L::PAR_BYTES;
       for (uint32_t it = 0;; ++it) {
         const uint32_t s = it % TMA_STAGES, round = it / TMA_STAGES;
         tma::mbar_wait(empty0 + 8 * s, (round & 1u) ^ 1u);  // first round passes at once
@@ -857,6 +924,11 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_
           if (track_ret) tma::bulk_g2s(dst + L::OFF_RET, p.ep_return + e0, L::ROW, bar);
         }
         if constexpr (HAS_SBT) tma::bulk_g2s(dst + L::OFF_SBT, p.sbt + e0, L::ROW, bar);
+        if constexpr (PARAMS) {
+#pragma unroll
+          for (int c = 0; c < E::NP; ++c)
+            tma::bulk_g2s(dst + L::OFF_PAR + c * L::ROW, p.params + (uint64_t)c * p.ld + e0, L::ROW, bar);
+        }
       }
     }
     __syncwarp();
@@ -919,8 +991,17 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_
 
       Group<KIND, V> g;
       act_t action[V];
+      PR prm;
       {
         const uint8_t* st = smem_raw + (data0 + s * L::STAGE_BYTES - tma::smem_u32(smem_raw));
+        if constexpr (PARAMS) {
+#pragma unroll
+          for (int c = 0; c < E::NP; ++c) {
+            const Vec<float, V> r = ldv<float, V>(reinterpret_cast<const float*>(st + L::OFF_PAR + c * L::ROW) + tid * V);
+#pragma unroll
+            for (int v = 0; v < V; ++v) prm.r[c][v] = r.v[v];
+          }
+        }
         Vec<float, V> row[SD];
 #pragma unroll
         for (int c = 0; c < SD; ++c) row[c] = ldv<float, V>(reinterpret_cast<const float*>(st + c * L::ROW) + tid * V);
@@ -959,11 +1040,11 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_
       }
 #else
       if (want_final)
-        step_group<KIND, V, AUTO, true, true, RESET_BY_CALLER, false, false, MGYM_STEP_BATCH_PAIRS>(p, true, base, t_now, action, track_ret, g,
-                                                                                   acc);
+        step_group<KIND, V, AUTO, true, true, RESET_BY_CALLER, false, false, MGYM_STEP_BATCH_PAIRS, PR>(p, true, base, t_now, action, track_ret, g,
+                                                                                   acc, prm);
       else
-        step_group<KIND, V, AUTO, false, true, RESET_BY_CALLER, false, false, MGYM_STEP_BATCH_PAIRS>(p, true, base, t_now, action, track_ret,
-                                                                                    g, acc);
+        step_group<KIND, V, AUTO, false, true, RESET_BY_CALLER, false, false, MGYM_STEP_BATCH_PAIRS, PR>(p, true, base, t_now, action, track_ret,
+                                                                                    g, acc, prm);
 #endif
       // Everything about this lane's finished envs sits in one branch: statistics from the packed flags word,
       // counters cleared, and their index inside the tile appended to the reset queue.
@@ -1074,16 +1155,22 @@ constexpr int rollout_min_blocks() {
   return MGYM_ROLLOUT_MIN_BLOCKS > 0 ? MGYM_ROLLOUT_MIN_BLOCKS : (KIND == 4 ? 2 : 3);
 }
 
-template <int KIND, int V, bool AUTO, int CNT, bool FULL>
-__global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kernel(const __grid_constant__ KernelParams p) {
+// PARAMS: the NP parameters of each env are read once per warp tile into per-thread shared-memory slots (like the
+// prefetched reset states) and picked up by every step: held in registers across the loop they would cost the
+// occupancy the loop is built for.  The action ring is half as deep then, so that CartPole's slots (24 KB), its
+// prefetched resets (16 KB) and the ring stay within the 48 KB of static shared memory.
+template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false>
+__global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kernel(const __grid_constant__ KParams<PARAMS> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
+  using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   constexpr int SD = E::SD, OD = E::OD;
   static_assert(!FULL || (AUTO && V == 4), "the FULL form is built for the vector auto-reset path only");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
-  constexpr int ACT_RING = MGYM_ACT_RING;
+  constexpr int ACT_RING = PARAMS ? MGYM_ACT_RING / 2 : MGYM_ACT_RING;
+  __shared__ float par_slots[PARAMS ? E::NP * V : 1][PARAMS ? 256 : 1];  // [c * V + v][thread]
   static_assert((ACT_RING & (ACT_RING - 1)) == 0, "power of two");
   constexpr uint32_t RING_STRIDE = 256 * V * sizeof(act_t);  // one row of the CTA: 256 threads x V actions
   __shared__ __align__(16) act_t act_ring[V == 4 ? ACT_RING : 1][256 * V];
@@ -1145,6 +1232,17 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kerne
         const Vec<float, V> er = ldv<float, V>(p.ep_return + base);
 #pragma unroll
         for (int v = 0; v < V; ++v) g.ret[v] = er.v[v];
+      }
+    }
+    if constexpr (PARAMS) {  // this thread's own slots: no synchronisation with other threads needed
+#pragma unroll
+      for (int c = 0; c < E::NP; ++c) {
+        Vec<float, V> r;
+#pragma unroll
+        for (int v = 0; v < V; ++v) r.v[v] = 1.0f;  // inactive lanes step zero states with harmless constants
+        if (active) r = ldv<float, V>(p.params + (uint64_t)c * p.ld + base);
+#pragma unroll
+        for (int v = 0; v < V; ++v) par_slots[c * V + v][threadIdx.x] = r.v[v];
       }
     }
 
@@ -1252,8 +1350,17 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kerne
 #pragma unroll
         for (int v = 0; v < V; ++v) action[v] = a_cur.get(v);
       }
-      step_group<KIND, V, AUTO, false, false, RESET_BY_CALLER, TRUSTED, true>(p, active, base, t, action, track_ret, g,
-                                                                              acc);
+      PR prm;
+      if constexpr (PARAMS) {
+        // volatile loads: re-read every step, not hoisted into registers for the whole loop
+#pragma unroll
+        for (int c = 0; c < E::NP; ++c) {
+#pragma unroll
+          for (int v = 0; v < V; ++v) prm.r[c][v] = *static_cast<volatile const float*>(&par_slots[c * V + v][threadIdx.x]);
+        }
+      }
+      step_group<KIND, V, AUTO, false, false, RESET_BY_CALLER, TRUSTED, true, false, PR>(p, active, base, t, action,
+                                                                                         track_ret, g, acc, prm);
 
       // ---- trajectory stores (before the resets: reward and flags belong to the finishing step; the
       // observation is stored after them, it is the post-reset one) ----
@@ -1528,6 +1635,53 @@ __global__ void steps_from_counters_kernel(const typename CounterType<CNT>::type
   const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t_dev) t = *t_dev;
   if (i < n) steps[i] = cnt_decode<CNT>(in[i], t);
+}
+
+// ---- per-env parameters (mgym_set_params / mgym_sample_params / mgym_get_params) ----------------------------------
+constexpr int MAX_PARAMS = 8;
+struct ParamVec {
+  float v[MAX_PARAMS];
+};
+struct ParamBox {  // U[lo, lo + range) per parameter, in f64 like the reset draws
+  double lo[MAX_PARAMS], range[MAX_PARAMS];
+};
+
+// Is every parameter finite, and every parameter c with bit c of `positive` set > 0?  Runs before anything is
+// copied into the handle, like validate_actions_kernel.
+__global__ void validate_params_kernel(const float* params, uint64_t n, int np, uint32_t positive, uint32_t* bad) {
+  bool mine = false;
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (uint64_t)np * n;
+       i += (uint64_t)gridDim.x * blockDim.x) {
+    const float x = params[i];
+    const uint32_t c = (uint32_t)(i / n);
+    mine |= !isfinite(x) || (((positive >> c) & 1u) && !(x > 0.0f));
+  }
+  if (__any_sync(0xffffffffu, mine) && (threadIdx.x & 31) == 0) *bad = 1u;
+}
+
+__global__ void fill_params_kernel(float* out, uint64_t n, int np, ParamVec value) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  for (int c = 0; c < np; ++c) out[(uint64_t)c * n + i] = value.v[c];
+}
+
+// Parameter c of env i (global index g = env_base + i) is word c % 4 of the Philox block with counter (g, key) and
+// tag TAG_PARAMS + c / 4, mapped to U[lo, lo + range) as the reset states are: independent of sharding and launch
+// geometry.  mask (device [n] or null): only envs with mask[i] != 0 are redrawn.
+__global__ void sample_params_kernel(float* params, uint64_t n, int np, const uint8_t* mask, uint64_t seed,
+                                     uint64_t env_base, uint64_t key, ParamBox box) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n || (mask && !mask[i])) return;
+  const uint64_t g = env_base + i;
+  for (int b = 0; b * 4 < np; ++b) {
+    const uint4 w = philox_env(seed, g, key, TAG_PARAMS + (uint32_t)b);
+    const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int c = 4 * b + j;
+      if (c < np) params[(uint64_t)c * n + i] = uniform_f64_to_f32(ws[j], box.lo[c], box.range[c]);
+    }
+  }
 }
 
 // validate_actions: is every discrete action inside Discrete(num_actions)?  Runs BEFORE the step, so an invalid

@@ -290,6 +290,70 @@ class GpuVecEnv:
         assert pool.shape[0] == self.state_dim
         _lib.check(self._lib.mgym_set_reset_pool(self._h, _ptr(pool), pool.shape[1], self._stream()))
 
+    # -- per-env physics parameters (domain randomisation) ---------------------------------------
+    @staticmethod
+    def param_names(kind):
+        """Names of the per-env parameters of `kind` (name or index), in row order; () for Acrobot."""
+        lib = _lib.load()
+        k = KINDS[kind] if isinstance(kind, str) else int(kind)
+        n = lib.mgym_num_params(k)
+        if n < 0:
+            raise ValueError(f"unknown kind {kind!r}")
+        return tuple(lib.mgym_param_name(k, i).decode() for i in range(n))
+
+    @staticmethod
+    def param_defaults(kind):
+        """The kind's constants, in the order of param_names(kind)."""
+        lib = _lib.load()
+        k = KINDS[kind] if isinstance(kind, str) else int(kind)
+        names = GpuVecEnv.param_names(k)
+        out = (C.c_float * max(1, len(names)))()
+        _lib.check(lib.mgym_param_defaults(k, out))
+        return tuple(float(out[i]) for i in range(len(names)))
+
+    def set_params(self, params):
+        """Per-env physics parameters.  params: a [P, N] tensor (rows in param_names order), a dict name -> scalar or
+        [N] tensor (unnamed parameters keep their current values), or None to return to the kind's constants.
+        Rejected values (not finite, or a non-positive mass / length / time step) raise and change nothing."""
+        if params is None:
+            _lib.check(self._lib.mgym_set_params(self._h, None, self._stream()))
+            return
+        names = self.param_names(self.kind)
+        if isinstance(params, dict):
+            unknown = set(params) - set(names)
+            if unknown:
+                raise KeyError(f"{sorted(unknown)} are not parameters of {self.kind}: {names}")
+            rows = self.get_params()
+            for c, name in enumerate(names):
+                if name in params:
+                    rows[c] = torch.as_tensor(params[name], dtype=torch.float32, device=self.device)
+            params = rows
+        params = torch.as_tensor(params, dtype=torch.float32).to(self.device).contiguous()
+        if tuple(params.shape) != (len(names), self.num_envs):
+            raise ValueError(f"params must have shape {(len(names), self.num_envs)}")
+        _lib.check(self._lib.mgym_set_params(self._h, _ptr(params), self._stream()))
+
+    def get_params(self, out=None):
+        """The per-env parameters as [P, N] (the defaults while none are set)."""
+        if out is None:
+            out = torch.empty((len(self.param_names(self.kind)), self.num_envs), dtype=torch.float32,
+                              device=self.device)
+        _lib.check(self._lib.mgym_get_params(self._h, _ptr(out), self._stream()))
+        return out
+
+    def sample_params(self, low, high, mask=None, key=0):
+        """Draw every env's parameters (or those with mask != 0) uniformly from [low, high) (P values each):
+        Philox-keyed by (global env index, key), so independent of sharding.  Capturable into a CUDA graph once
+        parameters exist; per-episode randomisation is sample_params(..., mask=info.flags != 0, key=step)."""
+        np_ = len(self.param_names(self.kind))
+        if len(low) != np_ or len(high) != np_:
+            raise ValueError(f"low and high need {np_} values each")
+        lo = (C.c_float * max(1, np_))(*[float(x) for x in low])
+        hi = (C.c_float * max(1, np_))(*[float(x) for x in high])
+        if mask is not None:
+            mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+        _lib.check(self._lib.mgym_sample_params(self._h, lo, hi, _ptr(mask), int(key), self._stream()))
+
     @property
     def step_index(self):
         return int(self._lib.mgym_step_index(self._h))
