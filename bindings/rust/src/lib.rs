@@ -192,6 +192,25 @@ impl GpuVecEnv {
         assert!(low.len() == self.num_params() && high.len() == self.num_params(), "low, high: num_params each");
         check(unsafe { sys::mgym_sample_params(self.h, low.as_ptr(), high.as_ptr(), mask, key, self.stream) })
     }
+    /// Per-episode redraw: every reset of an env draws its parameters from [low, high) (num_params values each);
+    /// `None` stops redrawing.  Rejected ranges leave the handle untouched.
+    pub fn set_param_redraw(&mut self, ranges: Option<(&[f32], &[f32])>) -> Result<(), MgymError> {
+        let (lo, hi) = match ranges {
+            Some((low, high)) => {
+                assert!(low.len() == self.num_params() && high.len() == self.num_params(), "low, high: num_params each");
+                (low.as_ptr(), high.as_ptr())
+            }
+            None => (ptr::null(), ptr::null()),
+        };
+        check(unsafe { sys::mgym_set_param_redraw(self.h, lo, hi, self.stream) })
+    }
+    /// The redraw ranges (low, high), or `None` when the handle does not redraw.
+    pub fn param_redraw(&self) -> Result<Option<(Vec<f32>, Vec<f32>)>, MgymError> {
+        let (mut lo, mut hi) = (vec![0f32; self.num_params()], vec![0f32; self.num_params()]);
+        let mut on: std::os::raw::c_int = 0;
+        check(unsafe { sys::mgym_get_param_redraw(self.h, &mut on, lo.as_mut_ptr(), hi.as_mut_ptr()) })?;
+        Ok(if on != 0 { Some((lo, hi)) } else { None })
+    }
     pub fn stats(&mut self) -> Result<sys::mgym_stats, MgymError> {
         let mut s = sys::mgym_stats::default();
         check(unsafe { sys::mgym_stats_get(self.h, &mut s, self.stream) })?;

@@ -87,6 +87,8 @@ extern "C" {
     pub fn mgym_get_params(env: *mut mgym_env, out: *mut f32, stream: *mut c_void) -> c_int;
     pub fn mgym_sample_params(env: *mut mgym_env, low: *const f32, high: *const f32, mask: *const u8, key: u64,
                               stream: *mut c_void) -> c_int;
+    pub fn mgym_set_param_redraw(env: *mut mgym_env, low: *const f32, high: *const f32, stream: *mut c_void) -> c_int;
+    pub fn mgym_get_param_redraw(env: *const mgym_env, enabled: *mut c_int, low: *mut f32, high: *mut f32) -> c_int;
     pub fn mgym_stats_get(env: *mut mgym_env, out: *mut mgym_stats, stream: *mut c_void) -> c_int;
     pub fn mgym_stats_reset(env: *mut mgym_env, stream: *mut c_void) -> c_int;
     pub fn mgym_stats_export(env: *mut mgym_env, device_vec5_out: *mut f64, stream: *mut c_void) -> c_int;

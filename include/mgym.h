@@ -176,9 +176,10 @@ int mgym_get_obs(mgym_env *env, float *obs_out, void *stream); /* current observ
 float *mgym_state_ptr(mgym_env *env);
 
 /* Checkpoint / resume: the whole handle (state rows, counters, running returns, statistics, step and reset
- * indices, per-env parameters if set) as one opaque HOST blob.  mgym_checkpoint_size gives the byte count; a handle
- * created with the same kind, num_envs and config continues bit-identically after mgym_checkpoint_load, which
- * restores exactly the parameters the blob carries (a blob without them clears the handle's). */
+ * indices, per-env parameters and redraw ranges if set) as one opaque HOST blob.  mgym_checkpoint_size gives the byte
+ * count; a handle created with the same kind, num_envs and config continues bit-identically after
+ * mgym_checkpoint_load, which restores exactly the parameters and ranges the blob carries (a blob without them clears
+ * the handle's). */
 size_t mgym_checkpoint_size(const mgym_env *env);
 int mgym_checkpoint_save(mgym_env *env, void *host_blob, size_t blob_bytes, void *stream);
 int mgym_checkpoint_load(mgym_env *env, const void *host_blob, size_t blob_bytes, void *stream);
@@ -231,10 +232,30 @@ int mgym_get_params(mgym_env *env, float *out, void *stream);
 /* Draws parameter c of env i uniformly from [low[c], high[c]) (host arrays of P; f64 draw cast to f32, like the
  * reset states): word c % 4 of the Philox block with counter (global env index, key mod 2^56) and tag 3 + c / 4,
  * so the draws do not depend on sharding or launch geometry.  mask (device uint8[N] or NULL) limits the draw to
- * envs with mask[i] != 0 -- per-episode randomisation is `mask = flags != 0` after a step.  Rows not set before
- * start from the defaults.  Capturable into a CUDA graph once the rows exist (the key is the caller's). */
+ * envs with mask[i] != 0 (e.g. `mask = flags != 0` after a step; mgym_set_param_redraw does per-episode draws
+ * on the device instead).  Rows not set before start from the defaults.  Capturable into a CUDA graph once the rows
+ * exist (the key is the caller's). */
 int mgym_sample_params(mgym_env *env, const float *low, const float *high, const uint8_t *mask, uint64_t key,
                        void *stream);
+/* Per-episode redraw (domain randomisation per episode): with ranges set, EVERY reset of an env also draws its
+ * parameters, parameter c uniformly from [low[c], high[c]) with the mapping of mgym_sample_params, from the Philox
+ * block with the counter of the new episode's reset state:
+ *   auto-reset in mgym_step / mgym_step_host / mgym_rollout   (global env index, step at which the finished episode
+ *                                                              began), tags 5 (parameters 0-3) and 6 (4-7)
+ *   mgym_reset / mgym_reset_masked, reset call index r        (global env index, r), tags 7 and 8
+ * so the draws do not depend on launch geometry, sharding or the mix of step and rollout calls.  The finishing step
+ * runs on the old parameters.  Nothing else redraws: not mgym_set_state, not a manual-mode (auto_reset = 0) step, and
+ * a reset pool (mgym_set_reset_pool) replaces only the reset STATES.  low[c] == high[c] draws exactly low[c].
+ * low, high: host arrays of P (finite, low <= high, low > 0 for masses, lengths and tau), or both NULL = off.
+ * Checked before anything changes: a rejected call leaves the handle untouched.  Setting ranges allocates the rows
+ * with the defaults if none are set and leaves the current episodes alone; `mgym_set_param_redraw(lo, hi);
+ * mgym_reset()` starts every env on drawn parameters.  mgym_set_params(NULL) clears the ranges with the rows,
+ * mgym_set_params(rows) keeps them; checkpoints carry them.  Acrobot: MGYM_ERR_BAD_ARGUMENT.  Not capturable.
+ * CUDA graphs: the ranges are launch parameters of the captured step / rollout, so a graph replays the ranges it was
+ * captured with -- recapture after changing them. */
+int mgym_set_param_redraw(mgym_env *env, const float *low, const float *high, void *stream);
+/* *enabled = 0 / 1; low, high (P floats each, may be NULL) receive the ranges when enabled. */
+int mgym_get_param_redraw(const mgym_env *env, int *enabled, float *low, float *high);
 
 /* ---- statistics --------------------------------------------------------------------- */
 int mgym_stats_get(mgym_env *env, mgym_stats_t *out, void *stream); /* synchronises */

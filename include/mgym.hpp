@@ -193,6 +193,23 @@ class GpuVecEnv {
       throw Error(MGYM_ERR_BAD_ARGUMENT, "sample_params: low and high need num_params values each");
     check(mgym_sample_params(h_, low.data(), high.data(), mask_device, key, stream_));
   }
+  // per-episode redraw: every reset draws the env's parameters from [low, high) (num_params values each)
+  void set_param_redraw(const std::vector<float>& low, const std::vector<float>& high) {
+    if ((int)low.size() != mgym_num_params(kind_) || (int)high.size() != mgym_num_params(kind_))
+      throw Error(MGYM_ERR_BAD_ARGUMENT, "set_param_redraw: low and high need num_params values each");
+    check(mgym_set_param_redraw(h_, low.data(), high.data(), stream_));
+  }
+  void clear_param_redraw() { check(mgym_set_param_redraw(h_, nullptr, nullptr, stream_)); }
+  // true and the ranges when the handle redraws; false (low, high untouched) otherwise
+  bool param_redraw(std::vector<float>* low = nullptr, std::vector<float>* high = nullptr) const {
+    const int np = mgym_num_params(kind_);
+    std::vector<float> lo((size_t)(np > 0 ? np : 0)), hi(lo.size());
+    int on = 0;
+    check(mgym_get_param_redraw(h_, &on, lo.data(), hi.data()));
+    if (on && low) *low = lo;
+    if (on && high) *high = hi;
+    return on != 0;
+  }
 
   mgym_stats_t stats() {
     mgym_stats_t s{};

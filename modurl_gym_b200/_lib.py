@@ -87,6 +87,8 @@ SYMBOLS = {
     "mgym_set_params": (_i, [_vp, _vp, _vp]),
     "mgym_get_params": (_i, [_vp, _vp, _vp]),
     "mgym_sample_params": (_i, [_vp, _vp, _vp, _vp, _u64, _vp]),
+    "mgym_set_param_redraw": (_i, [_vp, _vp, _vp, _vp]),
+    "mgym_get_param_redraw": (_i, [_vp, C.POINTER(_i), _vp, _vp]),
     "mgym_stats_get": (_i, [_vp, C.POINTER(Stats), _vp]),
     "mgym_stats_reset": (_i, [_vp, _vp]),
     "mgym_stats_export": (_i, [_vp, _vp, _vp]),

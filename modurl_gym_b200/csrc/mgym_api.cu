@@ -55,6 +55,9 @@ struct mgym_env {
   unsigned long long* stats = nullptr;  // 5 x 8 bytes
   uint32_t* bad_action = nullptr;
   float* params = nullptr;  // per-env physics parameters [P][n] (mgym_set_params), null = the kind's constants
+  // per-episode redraw ranges (mgym_set_param_redraw): every reset draws the env's parameters from U[lo, hi)
+  bool redraw = false;
+  float redraw_lo[MAX_PARAMS] = {}, redraw_hi[MAX_PARAMS] = {};
 
   uint64_t t = 0;         // steps executed since creation
   uint64_t n_resets = 0;  // explicit reset calls since creation
@@ -270,12 +273,12 @@ int launch_persistent(void (*kernel)(KP), const mgym_env* e, const KP& p, uint64
 }
 
 // TMA-staged step kernel (auto-reset, vector path, N a multiple of the 128-env warp tile)
-template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false>
-int launch_step_tma(const mgym_env* ce, const KParams<PARAMS>& p_in, cudaStream_t st) {
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false>
+int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cudaStream_t st) {
   mgym_env* e = const_cast<mgym_env*>(ce);  // ticket accounting
-  KParams<PARAMS> p = p_in;
+  KParams<PARAMS, REDRAW> p = p_in;
   using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
-  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS>;
+  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS, REDRAW>;
   constexpr int threads = TMA_THREADS;
   // the opt-in to > 48 KB of dynamic shared memory and the occupancy are per device
   static int cached_per_sm[kMaxDevices] = {};
@@ -332,36 +335,39 @@ bool use_tma() {
   return v;
 }
 
-// kind x vector width x auto/manual x counter representation (x per-env parameters)
-template <int KIND, int V, bool ROLLOUT, bool PARAMS = false>
-int dispatch_mode(const mgym_env* e, const KParams<PARAMS>& p, cudaStream_t st) {
+// kind x vector width x auto/manual x counter representation (x per-env parameters (x per-episode redraw: auto-reset
+// handles only, the host never asks for a manual form of it))
+template <int KIND, int V, bool ROLLOUT, bool PARAMS = false, bool REDRAW = false>
+int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStream_t st) {
   const uint64_t groups = p.n / V;
   const bool autor = e->cfg.auto_reset != 0;
   if constexpr (!ROLLOUT && V == 4) {
     // manual mode (the reference's protocol): counters are 32-bit, CartPole adds steps_beyond_terminated
-    if (!autor && use_tma() && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
+    if constexpr (!REDRAW) {
+      if (!autor && use_tma() && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
+    }
     if (autor && use_tma() && p.n % TMA_TILE == 0) {
       if constexpr (KIND == 0) {  // CartPole always counts (500-step truncation, cartpole.rs:297)
-        if (e->cnt_mode == CNT_U16) return launch_step_tma<KIND, CNT_U16, true, PARAMS>(e, p, st);
-        return launch_step_tma<KIND, CNT_S16, true, PARAMS>(e, p, st);
+        if (e->cnt_mode == CNT_U16) return launch_step_tma<KIND, CNT_U16, true, PARAMS, REDRAW>(e, p, st);
+        return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW>(e, p, st);
       } else {
         switch (e->cnt_mode) {
-          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS>(e, p, st);
-          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS>(e, p, st);
-          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS>(e, p, st);
+          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW>(e, p, st);
+          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS, REDRAW>(e, p, st);
+          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS, REDRAW>(e, p, st);
         }
       }
     }
     if (use_tma() && p.n > TMA_TILE) {
       // ragged size: whole 1024-env tiles on the TMA kernel, the remaining (< 1024) envs on the vector kernel
-      KParams<PARAMS> head = p, tail = p;
+      KParams<PARAMS, REDRAW> head = p, tail = p;
       head.adv_dt = 0;  // device clock: the tail launch (last of the call) moves the step index on
       head.n = p.n - p.n % TMA_TILE;
       tail.first = p.first + head.n;
       tail.n = p.n - head.n;
-      int rc = dispatch_mode<KIND, 4, false, PARAMS>(e, head, st);
+      int rc = dispatch_mode<KIND, 4, false, PARAMS, REDRAW>(e, head, st);
       if (rc != MGYM_OK) return rc;
-      return dispatch_mode<KIND, 4, false, PARAMS>(e, tail, st);
+      return dispatch_mode<KIND, 4, false, PARAMS, REDRAW>(e, tail, st);
     }
   }
   // rollout_kernel's FULL form: complete warp tiles and all three trajectory outputs
@@ -371,14 +377,17 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS>& p, cudaStream_t st) 
   do {                                                                                                   \
     if constexpr (ROLLOUT) {                                                                             \
       if constexpr (AUTO_ && V == 4) {                                                                   \
-        if (full) return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS>, e, p, groups, st); \
+        if (full)                                                                                        \
+          return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS, REDRAW>, e, p, groups, st); \
       }                                                                                                  \
-      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS>, e, p, groups, st);   \
+      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS, REDRAW>, e, p, groups, st); \
     } else {                                                                                             \
-      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS>, e, p, groups, st);             \
+      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS, REDRAW>, e, p, groups, st);     \
     }                                                                                                    \
   } while (0)
-  if (!autor) MGYM_LAUNCH(false, CNT_U32);
+  if constexpr (!REDRAW) {
+    if (!autor) MGYM_LAUNCH(false, CNT_U32);
+  }
   if constexpr (KIND == 0) {
     if (e->cnt_mode == CNT_U16) MGYM_LAUNCH(true, CNT_U16);
     MGYM_LAUNCH(true, CNT_S16);
@@ -391,7 +400,18 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS>& p, cudaStream_t st) 
 #undef MGYM_LAUNCH
 }
 
-// A handle with per-env parameters runs the PARAMS instantiations (kinds that have parameters only).
+// The handle's redraw ranges as the f64 box the kernels map Philox words into (the mapping of mgym_sample_params)
+ParamBox redraw_box(const mgym_env* e) {
+  ParamBox box{};
+  for (int c = 0; c < MAX_PARAMS; ++c) {
+    box.lo[c] = (double)e->redraw_lo[c];
+    box.range[c] = (double)e->redraw_hi[c] - (double)e->redraw_lo[c];
+  }
+  return box;
+}
+
+// A handle with per-env parameters runs the PARAMS instantiations (kinds that have parameters only), an auto-reset
+// one with redraw ranges the PARAMS + REDRAW instantiations (manual-mode steps never reset).
 template <int KIND, bool ROLLOUT>
 int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
   if constexpr (Env<KIND>::NP > 0) {
@@ -399,6 +419,13 @@ int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStrea
       KernelParamsP pp;
       static_cast<KernelParams&>(pp) = p;
       pp.params = e->params;
+      if (e->redraw && e->cfg.auto_reset) {
+        KernelParamsR pr;
+        static_cast<KernelParamsP&>(pr) = pp;
+        pr.redraw = redraw_box(e);
+        return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true, true>(e, pr, st)
+                    : dispatch_mode<KIND, 1, ROLLOUT, true, true>(e, pr, st);
+      }
       return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true>(e, pp, st) : dispatch_mode<KIND, 1, ROLLOUT, true>(e, pp, st);
     }
   }
@@ -512,6 +539,18 @@ int validate_device_actions(mgym_env* e, const void* actions, uint64_t count, cu
   MGYM_CUDA(cudaMemcpyAsync(&bad, e->bad_action, sizeof(bad), cudaMemcpyDeviceToHost, st));
   MGYM_CUDA(cudaStreamSynchronize(st));
   return bad ? invalid_action(e) : MGYM_OK;
+}
+
+// Redraw ranges (mgym_set_param_redraw, checkpoints): finite, low <= high, low > 0 for the kind's positive
+// parameters.  Names the first offending parameter.
+int check_redraw_ranges(int kind, const float* low, const float* high, const char* what) {
+  for (int c = 0; c < kNumParams[kind]; ++c) {
+    const bool pos = (kParamPositive[kind] >> c) & 1u;
+    if (!std::isfinite(low[c]) || !std::isfinite(high[c]) || !(low[c] <= high[c]) || (pos && !(low[c] > 0.0f)))
+      return fail(MGYM_ERR_BAD_ARGUMENT, "%s: bad range for %s %s: [%g, %g] (finite, low <= high%s); nothing was changed",
+                  what, kNames[kind], kParamNames[kind][c], (double)low[c], (double)high[c], pos ? ", low > 0" : "");
+  }
+  return MGYM_OK;
 }
 
 }  // namespace
@@ -753,6 +792,11 @@ int mgym_reset_masked(mgym_env* e, const uint8_t* mask, float* obs_out, void* st
     case 3: rc = launch_reset_kind<3>(e, p, mask, st); break;
     default: rc = launch_reset_kind<4>(e, p, mask, st); break;
   }
+  if (rc == MGYM_OK && e->redraw) {  // the reset envs' parameters, keyed like their reset states
+    reset_redraw_params_kernel<<<(unsigned)((e->n + 255) / 256), 256, 0, st>>>(
+        e->params, e->n, kNumParams[e->kind], mask, e->seed, e->cfg.env_index_base, e->n_resets, redraw_box(e));
+    MGYM_CUDA(cudaGetLastError());
+  }
   if (rc == MGYM_OK) e->n_resets += 1;
   return rc;
 }
@@ -897,7 +941,8 @@ struct CheckpointHeader {
   int32_t kind, cnt_mode, auto_reset, has_sbt, has_ret;
   int32_t is_euler, sutton_barto, max_episode_steps, track_stats;
   float goal_velocity;
-  uint32_t has_params;  // 1: the per-env parameter rows follow the statistics
+  uint32_t has_params;  // bit 0: the per-env parameter rows follow the statistics; bit 1: the redraw ranges (P low, then
+                        // P high values) follow the rows
   uint64_t n, seed, t, n_resets, env_index_base, pool_len;
 };
 constexpr uint32_t kCkptMagic = 0x4D47594Du;  // "MGYM"
@@ -914,23 +959,26 @@ CheckpointHeader checkpoint_header(const mgym_env* e) {
   h.goal_velocity = e->cfg.goal_velocity;
   h.n = e->n, h.seed = e->seed, h.t = e->t, h.n_resets = e->n_resets;
   h.env_index_base = e->cfg.env_index_base, h.pool_len = e->pool_len;
-  h.has_params = e->params ? 1u : 0u;
+  h.has_params = (e->params ? 1u : 0u) | (e->redraw ? 2u : 0u);
   return h;
 }
 
 size_t counter_bytes(const mgym_env* e) { return counter_width(e->cnt_mode) * (size_t)e->n; }
 size_t param_bytes(const mgym_env* e) { return sizeof(float) * kNumParams[e->kind] * (size_t)e->n; }
+size_t range_bytes(const mgym_env* e) { return 2 * sizeof(float) * kNumParams[e->kind]; }
 
-// size of a blob of this handle that carries parameter rows or not
-size_t checkpoint_bytes(const mgym_env* e, bool with_params) {
+// size of a blob of this handle that carries parameter rows (and redraw ranges) or not
+size_t checkpoint_bytes(const mgym_env* e, bool with_params, bool with_ranges) {
   const size_t n = (size_t)e->n;
   return sizeof(CheckpointHeader) + sizeof(float) * kStateDim[e->kind] * n + counter_bytes(e) +
          (e->sbt ? sizeof(uint32_t) * n : 0) + (e->ep_return ? sizeof(float) * n : 0) + 5 * sizeof(unsigned long long) +
-         (with_params ? param_bytes(e) : 0);
+         (with_params ? param_bytes(e) : 0) + (with_ranges ? range_bytes(e) : 0);
 }
 }  // namespace
 
-size_t mgym_checkpoint_size(const mgym_env* e) { return e ? checkpoint_bytes(e, e->params != nullptr) : 0; }
+size_t mgym_checkpoint_size(const mgym_env* e) {
+  return e ? checkpoint_bytes(e, e->params != nullptr, e->redraw) : 0;
+}
 
 int mgym_checkpoint_save(mgym_env* e, void* blob, size_t blob_bytes, void* stream) {
   if (!e || !blob) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_checkpoint_save: NULL argument");
@@ -956,6 +1004,11 @@ int mgym_checkpoint_save(mgym_env* e, void* blob, size_t blob_bytes, void* strea
   if ((rc = pull(e->stats, 5 * sizeof(unsigned long long)))) return rc;
   if ((rc = pull(e->params, e->params ? param_bytes(e) : 0))) return rc;
   MGYM_CUDA(cudaStreamSynchronize(st));
+  if (e->redraw) {
+    const size_t np = (size_t)kNumParams[e->kind];
+    memcpy(out, e->redraw_lo, sizeof(float) * np);
+    memcpy(out + sizeof(float) * np, e->redraw_hi, sizeof(float) * np);
+  }
   return MGYM_OK;
 }
 
@@ -983,8 +1036,18 @@ int mgym_checkpoint_load(mgym_env* e, const void* blob, size_t blob_bytes, void*
                 (unsigned long long)h.env_index_base, (unsigned long long)mine.env_index_base,
                 (unsigned long long)h.pool_len, (unsigned long long)mine.pool_len);
   // a blob restores exactly the parameters it carries; one without parameter rows clears the handle's
-  const bool with_params = h.has_params != 0 && kNumParams[e->kind] > 0;
-  if (blob_bytes < checkpoint_bytes(e, with_params)) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_checkpoint_load: truncated blob");
+  const bool with_params = (h.has_params & 1u) != 0 && kNumParams[e->kind] > 0;
+  const bool with_ranges = with_params && (h.has_params & 2u) != 0;
+  if (blob_bytes < checkpoint_bytes(e, with_params, with_ranges))
+    return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_checkpoint_load: truncated blob");
+  float lo[MAX_PARAMS] = {}, hi[MAX_PARAMS] = {};
+  if (with_ranges) {  // checked like mgym_set_param_redraw, before anything changes
+    const size_t np = (size_t)kNumParams[e->kind];
+    const uint8_t* r = static_cast<const uint8_t*>(blob) + checkpoint_bytes(e, true, false);
+    memcpy(lo, r, sizeof(float) * np);
+    memcpy(hi, r + sizeof(float) * np, sizeof(float) * np);
+    if (int rc = check_redraw_ranges(e->kind, lo, hi, "mgym_checkpoint_load")) return rc;
+  }
   DeviceGuard guard(e->device);
   if (with_params && !e->params) MGYM_CUDA(cudaMalloc(&e->params, param_bytes(e)));
   cudaStream_t st = (cudaStream_t)stream;
@@ -1007,6 +1070,10 @@ int mgym_checkpoint_load(mgym_env* e, const void* blob, size_t blob_bytes, void*
     cudaFree(e->params);
     e->params = nullptr;
   }
+  // exactly the ranges the blob carries: a blob without them turns redraw off
+  e->redraw = with_ranges;
+  memcpy(e->redraw_lo, lo, sizeof(lo));
+  memcpy(e->redraw_hi, hi, sizeof(hi));
   e->seed = h.seed;
   e->t = h.t;
   if (e->cfg.device_clock) {
@@ -1145,9 +1212,10 @@ int mgym_set_params(mgym_env* e, const float* params, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = refuse_capture(e, st, "mgym_set_params", false)) return rc;
   MGYM_CUDA(cudaStreamSynchronize(st));  // in-flight launches may still read the rows
-  if (!params) {
+  if (!params) {  // back to the constants: the redraw ranges go with the rows
     cudaFree(e->params);
     e->params = nullptr;
+    e->redraw = false;
     return MGYM_OK;
   }
   const int np = kNumParams[e->kind];
@@ -1226,6 +1294,38 @@ int mgym_sample_params(mgym_env* e, const float* low, const float* high, const u
   sample_params_kernel<<<(unsigned)((e->n + 255) / 256), 256, 0, st>>>(e->params, e->n, np, mask, e->seed,
                                                                        e->cfg.env_index_base, key, box);
   MGYM_CUDA(cudaGetLastError());
+  return MGYM_OK;
+}
+
+int mgym_set_param_redraw(mgym_env* e, const float* low, const float* high, void* stream) {
+  if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_set_param_redraw: env is NULL");
+  if (kNumParams[e->kind] == 0) return no_params(e, "mgym_set_param_redraw");
+  if (!low != !high)
+    return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_set_param_redraw: low and high must both be given, or both be NULL");
+  DeviceGuard guard(e->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = refuse_capture(e, st, "mgym_set_param_redraw", false)) return rc;
+  if (!low) {
+    e->redraw = false;
+    return MGYM_OK;
+  }
+  if (int rc = check_redraw_ranges(e->kind, low, high, "mgym_set_param_redraw")) return rc;
+  if (int rc = ensure_params(e, st)) return rc;  // rows with the defaults: the current episodes keep their constants
+  for (int c = 0; c < MAX_PARAMS; ++c) {
+    e->redraw_lo[c] = c < kNumParams[e->kind] ? low[c] : 0.0f;
+    e->redraw_hi[c] = c < kNumParams[e->kind] ? high[c] : 0.0f;
+  }
+  e->redraw = true;
+  return MGYM_OK;
+}
+
+int mgym_get_param_redraw(const mgym_env* e, int* enabled, float* low, float* high) {
+  if (!e || !enabled) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_get_param_redraw: NULL argument");
+  *enabled = e->redraw ? 1 : 0;
+  for (int c = 0; e->redraw && c < kNumParams[e->kind]; ++c) {
+    if (low) low[c] = e->redraw_lo[c];
+    if (high) high[c] = e->redraw_hi[c];
+  }
   return MGYM_OK;
 }
 

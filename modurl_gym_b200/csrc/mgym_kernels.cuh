@@ -118,8 +118,40 @@ struct KernelParams {
 struct KernelParamsP : KernelParams {
   const float* params;
 };
-template <bool PARAMS>
-using KParams = std::conditional_t<PARAMS, KernelParamsP, KernelParams>;
+constexpr int MAX_PARAMS = 8;
+struct ParamBox {  // U[lo, lo + range) per parameter, in f64 like the reset draws
+  double lo[MAX_PARAMS], range[MAX_PARAMS];
+};
+// The launch parameters of the kernels instantiated with REDRAW (auto-reset forms only): the handle's redraw ranges
+// (mgym_set_param_redraw), by value, on top of the rows -- every auto-reset then writes the new episode's parameters
+// into the rows.  A captured launch replays the ranges it was captured with.
+struct KernelParamsR : KernelParamsP {
+  ParamBox redraw;
+};
+template <bool PARAMS, bool REDRAW = false>
+using KParams = std::conditional_t<REDRAW, KernelParamsR, std::conditional_t<PARAMS, KernelParamsP, KernelParams>>;
+
+// The parameters of global env g for the episode whose reset state has counter (g, t): word c % 4 of the Philox
+// block (g, t) with tag tag0 + c / 4, mapped to U[lo, lo + range) as mgym_sample_params maps them.  Parameter c is
+// stored to dst[c * stride].
+template <int NP>
+__device__ __forceinline__ void redraw_params(const PhiloxKeys& ks, const ParamBox& box, uint64_t g, uint64_t t,
+                                              uint32_t tag0, float* dst, uint64_t stride) {
+#pragma unroll
+  for (int b = 0; b * 4 < NP; ++b) {
+    const uint4 w = philox_env(ks, g, t, tag0 + (uint32_t)b);
+    const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+    for (int j = 0; j < 4 && 4 * b + j < NP; ++j)
+      dst[(uint64_t)(4 * b + j) * stride] = uniform_f64_to_f32(ws[j], box.lo[4 * b + j], box.range[4 * b + j]);
+  }
+}
+// Where redraw_pending puts the redrawn parameters: parameter c of slot v at base[c * cstride + v * vstride]
+// (the parameter rows in global memory for the per-call step, the per-thread shared-memory slots in the rollout).
+struct RedrawDst {
+  float* base;
+  uint64_t cstride, vstride;
+};
 
 // The per-env parameters of a lane's V envs, [NP][V] (r[c][v] = parameter c of slot v).  NP = 0: none.
 template <int NP_, int V>
@@ -321,6 +353,24 @@ struct ResetPrefetch {
   uint32_t valid = 0;      // bit v: slot v holds the state for the END of env v's current episode
 };
 
+// The parameters of the new episodes of the slots in `pending` (p is a KernelParamsR), one slot per lane per pass,
+// from Philox whatever the source of the reset state, stored to `rd`.  Runs right before reset_pending (it reads the
+// counts AFTER the finishing step, which reset_pending clears).
+template <int KIND, int V>
+__device__ __forceinline__ void redraw_pending(const KernelParams& p, uint64_t base, uint64_t t, uint32_t pending,
+                                               const Group<KIND, V>& g, const RedrawDst& rd) {
+  const ParamBox& box = static_cast<const KernelParamsR&>(p).redraw;
+  while (pending) {
+    const int sel = __ffs(pending) - 1;
+    pending &= pending - 1;
+    uint32_t count = g.steps[0];
+#pragma unroll
+    for (int v = 1; v < V; ++v) count = (v == sel) ? g.steps[v] : count;
+    redraw_params<Env<KIND>::NP>(p.keys, box, p.env_base + base + sel, episode_start(t, count), TAG_REDRAW_AUTO,
+                                 rd.base + (uint64_t)sel * rd.vstride, rd.cstride);
+  }
+}
+
 // Draws the reset states of the slots in `pending` (bit v = slot v), one slot per lane per pass.  g.steps[] are the
 // counts AFTER the finishing step (they are cleared here).
 template <int KIND, int V>
@@ -428,8 +478,11 @@ __device__ __noinline__ LaneIO<KIND, V> dynamics_reference_lane(LaneIO<KIND, V> 
 // dynamics themselves then preserve, so the fast form runs without its per-step precondition test.
 // OBS_VALID (kinds with Env::HAS_OBS_CACHE): g.obs is the observation of the state in g.st on entry.
 // PR (ParamRows with NP > 0): every env steps with its own constants, prm.r[.][v] (Env::dynamics_p).
+// REDRAW (RESET_IN_PLACE, p is a KernelParamsR): the reset also redraws the finished envs' parameter rows in global
+// memory (the step itself ran on the old ones, in prm).
 template <int KIND, int V, bool AUTO, bool WANT_FINAL, bool TALLY_LEN = true, int RESET = RESET_IN_PLACE,
-          bool TRUSTED = false, bool OBS_VALID = false, bool BATCH_PAIRS = false, typename PR = NoParams>
+          bool TRUSTED = false, bool OBS_VALID = false, bool BATCH_PAIRS = false, typename PR = NoParams,
+          bool REDRAW = false>
 __device__ __forceinline__ uint32_t step_group(const KernelParams& p, bool count, uint64_t base, uint64_t t,
                                            const typename Env<KIND>::act_t (&action)[V], bool track_ret,
                                            Group<KIND, V>& g, StatAcc& acc, const PR& prm = PR{}) {
@@ -579,6 +632,10 @@ __device__ __forceinline__ uint32_t step_group(const KernelParams& p, bool count
       }
     }
   }
+  if constexpr (AUTO && RESET == RESET_IN_PLACE && REDRAW) {
+    const RedrawDst rd{const_cast<float*>(static_cast<const KernelParamsP&>(p).params) + base, p.ld, 1};
+    redraw_pending<KIND, V>(p, base, t, pending, g, rd);
+  }
   if constexpr (AUTO && RESET == RESET_IN_PLACE) reset_pending<KIND, V>(p, base, t, pending, g);
   return 0u;
 }
@@ -612,13 +669,15 @@ __device__ __forceinline__ typename CounterType<CNT>::type cnt_encode(uint32_t s
 // =============================================================================================
 // Mode 1: per-call step kernel
 // =============================================================================================
-template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false>
-__global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid_constant__ KParams<PARAMS> p) {
+// REDRAW: every reset also redraws the env's parameter rows (mgym_set_param_redraw; auto-reset with rows only).
+template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false, bool REDRAW = false>
+__global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
   using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   constexpr int SD = E::SD, OD = E::OD;
+  static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
   StatAcc acc;
@@ -665,11 +724,12 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
       }
     }
     if (want_final)
-      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, false, PR>(p, true, base, t_now, action,
-                                                                                    track_ret, g, acc, prm);
+      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, false, PR, REDRAW>(p, true, base, t_now, action,
+                                                                                            track_ret, g, acc, prm);
     else
-      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, false, PR>(p, true, base, t_now, action,
-                                                                                     track_ret, g, acc, prm);
+      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, false, PR, REDRAW>(p, true, base, t_now,
+                                                                                             action, track_ret, g, acc,
+                                                                                             prm);
 
     {
       Vec<float, V> s[SD];
@@ -839,8 +899,14 @@ struct TmaLayout {
 // AUTO = false is the reference's own protocol (no same-step reset: the caller resets what finished,
 // cartpole.rs:468-470): the same pipeline with steps_beyond_terminated as one more row and nothing ever queued
 // for the reset warp.
-template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false>
-__global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_tma(const __grid_constant__ KParams<PARAMS> p) {
+//
+// REDRAW (mgym_set_param_redraw): the reset warp also draws the new episode's parameters of each queued env (one more
+// Philox block, two for CartPole) and writes them into the rows in global memory.  The consumers stepped that tile
+// with the staged (old) rows; no other tile of the launch holds the env, and the next launch's producer reads the
+// rows only after griddepcontrol.wait.  Stage layout and stage count are those of the PARAMS form.
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false>
+__global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS)
+    step_kernel_tma(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
   using E = Env<KIND>;
   using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
   using act_t = typename E::act_t;
@@ -848,6 +914,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_
   constexpr int SD = E::SD, OD = E::OD, V = 4;
   constexpr int TMA_STAGES = L::STAGES;  // shadows the global default: this kernel's own ring depth
   using PR = ParamRows<PARAMS ? E::NP : 0, V>;
+  static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(AUTO || !cnt_is_stamp(CNT), "manual mode keeps the reference's own counters");
   static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
   extern __shared__ uint8_t smem_raw[];
@@ -954,6 +1021,10 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS) step_kernel_
           for (int c = 0; c < SD; ++c) ns[c] = p.reset_pool[(uint64_t)c * p.pool_len + k];
         } else {
           E::reset(philox_env(p.keys, gid, episode_start(t_now, lengths[j]), TAG_AUTO_RESET), ns);
+        }
+        if constexpr (REDRAW) {
+          redraw_params<E::NP>(p.keys, p.redraw, gid, episode_start(t_now, lengths[j]), TAG_REDRAW_AUTO,
+                               const_cast<float*>(p.params) + local, p.ld);
         }
 #pragma unroll
         for (int c = 0; c < SD; ++c) p.state[(uint64_t)c * p.ld + local] = ns[c];
@@ -1159,13 +1230,19 @@ constexpr int rollout_min_blocks() {
 // prefetched reset states) and picked up by every step: held in registers across the loop they would cost the
 // occupancy the loop is built for.  The action ring is half as deep then, so that CartPole's slots (24 KB), its
 // prefetched resets (16 KB) and the ring stay within the 48 KB of static shared memory.
-template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false>
-__global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kernel(const __grid_constant__ KParams<PARAMS> p) {
+// REDRAW (mgym_set_param_redraw): a reset also draws the finished env's parameters for its new episode, in the
+// divergent reset pass, straight into its slots (every later step of the tile runs the new episode's constants); the
+// slots are written back to the rows at the end of the tile.  Drawing them ahead of time like the reset states would
+// need 24 KB more of CartPole's slots, i.e. dynamic shared memory (DESIGN.md section 11.1).
+template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false, bool REDRAW = false>
+__global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
+    rollout_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
   using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   constexpr int SD = E::SD, OD = E::OD;
+  static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!FULL || (AUTO && V == 4), "the FULL form is built for the vector auto-reset path only");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
@@ -1291,6 +1368,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kerne
     // return value says whether the invariant behind it still holds (it can only break when a reset state
     // comes from an injected pool, and is re-checked right there, under the same rare branch).
     ResetPrefetch pre;
+    [[maybe_unused]] uint32_t redrawn = 0;  // REDRAW: slots whose parameters were redrawn in this tile
     // Redraws slot `slot` of EVERY lane (full warp): the state the lane's env in that slot restarts from when its
     // current episode ends.  t_next = index of the next step to run; g.steps = counts at its entry.
     [[maybe_unused]] auto draw_ahead = [&](uint32_t slot, uint64_t t_next) {
@@ -1405,6 +1483,10 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kerne
               }
             }
           }
+          if constexpr (REDRAW) {  // into this thread's slots: the next step of the tile reads them
+            redrawn |= pending;
+            redraw_pending<KIND, V>(p, base, t, pending, g, RedrawDst{&par_slots[0][threadIdx.x], (uint64_t)V * 256, 256});
+          }
           reset_pending<KIND, V>(p, base, t, pending, g, PREFETCH ? &pre : nullptr);
           if constexpr (TRUSTED && E::HAS_TRUSTED) {
             if (p.reset_pool) still = __all_sync(0xffffffffu, group_trusted<KIND, V>(g));
@@ -1493,6 +1575,17 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>()) rollout_kerne
 #pragma unroll
         for (int v = 0; v < V; ++v) er.v[v] = g.ret[v];
         stv<float, V>(p.ep_return + base, er);
+      }
+      if constexpr (REDRAW) {  // the parameters of the episodes that run on past this launch, if any were drawn
+        if (redrawn) {
+#pragma unroll
+          for (int c = 0; c < E::NP; ++c) {
+            Vec<float, V> r;
+#pragma unroll
+            for (int v = 0; v < V; ++v) r.v[v] = par_slots[c * V + v][threadIdx.x];
+            stv<float, V>(const_cast<float*>(p.params) + (uint64_t)c * p.ld + base, r);
+          }
+        }
       }
     }
   }
@@ -1638,12 +1731,8 @@ __global__ void steps_from_counters_kernel(const typename CounterType<CNT>::type
 }
 
 // ---- per-env parameters (mgym_set_params / mgym_sample_params / mgym_get_params) ----------------------------------
-constexpr int MAX_PARAMS = 8;
 struct ParamVec {
   float v[MAX_PARAMS];
-};
-struct ParamBox {  // U[lo, lo + range) per parameter, in f64 like the reset draws
-  double lo[MAX_PARAMS], range[MAX_PARAMS];
 };
 
 // Is every parameter finite, and every parameter c with bit c of `positive` set > 0?  Runs before anything is
@@ -1675,6 +1764,25 @@ __global__ void sample_params_kernel(float* params, uint64_t n, int np, const ui
   const uint64_t g = env_base + i;
   for (int b = 0; b * 4 < np; ++b) {
     const uint4 w = philox_env(seed, g, key, TAG_PARAMS + (uint32_t)b);
+    const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int c = 4 * b + j;
+      if (c < np) params[(uint64_t)c * n + i] = uniform_f64_to_f32(ws[j], box.lo[c], box.range[c]);
+    }
+  }
+}
+
+// Explicit resets of a handle with redraw ranges (mgym_reset / mgym_reset_masked), after the reset kernel: the
+// parameters of every reset env (mask[i] != 0, or all with mask == null) from the Philox blocks with the counter of
+// its reset state, (g, reset call index), and tags TAG_REDRAW_RESET + c / 4.  Cold: one thread per env.
+__global__ void reset_redraw_params_kernel(float* params, uint64_t n, int np, const uint8_t* mask, uint64_t seed,
+                                           uint64_t env_base, uint64_t reset_index, ParamBox box) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n || (mask && !mask[i])) return;
+  const uint64_t g = env_base + i;
+  for (int b = 0; b * 4 < np; ++b) {
+    const uint4 w = philox_env(seed, g, reset_index, TAG_REDRAW_RESET + (uint32_t)b);
     const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
     for (int j = 0; j < 4; ++j) {

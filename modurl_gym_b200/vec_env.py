@@ -344,7 +344,8 @@ class GpuVecEnv:
     def sample_params(self, low, high, mask=None, key=0):
         """Draw every env's parameters (or those with mask != 0) uniformly from [low, high) (P values each):
         Philox-keyed by (global env index, key), so independent of sharding.  Capturable into a CUDA graph once
-        parameters exist; per-episode randomisation is sample_params(..., mask=info.flags != 0, key=step)."""
+        parameters exist.  For new parameters at every new episode use set_param_redraw instead: it draws them on
+        the device inside the resets of step, rollout and reset, keyed by the episode rather than by the caller."""
         np_ = len(self.param_names(self.kind))
         if len(low) != np_ or len(high) != np_:
             raise ValueError(f"low and high need {np_} values each")
@@ -353,6 +354,40 @@ class GpuVecEnv:
         if mask is not None:
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         _lib.check(self._lib.mgym_sample_params(self._h, lo, hi, _ptr(mask), int(key), self._stream()))
+
+    def set_param_redraw(self, low, high=None):
+        """Per-episode domain randomisation: every reset of an env (auto-reset in step / rollout / step_host, and
+        reset()) also draws its parameters uniformly from [low, high), on the device, keyed by the episode (DESIGN.md
+        section 11).  low, high: P values each; or one dict name -> (low, high), where missing names keep their
+        default value ([default, default]); or None to stop redrawing (the rows stay).  Current episodes keep their
+        parameters: set_param_redraw(lo, hi); reset() starts every env on drawn ones.  Bad ranges raise and change
+        nothing.  A captured CUDA graph replays the ranges it was captured with."""
+        if low is None:
+            _lib.check(self._lib.mgym_set_param_redraw(self._h, None, None, self._stream()))
+            return
+        names = self.param_names(self.kind)
+        if isinstance(low, dict):
+            unknown = set(low) - set(names)
+            if unknown:
+                raise KeyError(f"{sorted(unknown)} are not parameters of {self.kind}: {names}")
+            d = self.param_defaults(self.kind)
+            pairs = [low.get(name, (d[c], d[c])) for c, name in enumerate(names)]
+            low, high = [p[0] for p in pairs], [p[1] for p in pairs]
+        if high is None or len(low) != len(names) or len(high) != len(names):
+            raise ValueError(f"low and high need {len(names)} values each")
+        lo = (C.c_float * max(1, len(names)))(*[float(x) for x in low])
+        hi = (C.c_float * max(1, len(names)))(*[float(x) for x in high])
+        _lib.check(self._lib.mgym_set_param_redraw(self._h, lo, hi, self._stream()))
+
+    def param_redraw(self):
+        """The redraw ranges as (low, high) tuples of P floats, or None when the handle does not redraw."""
+        np_ = max(1, len(self.param_names(self.kind)))
+        on, lo, hi = C.c_int(0), (C.c_float * np_)(), (C.c_float * np_)()
+        _lib.check(self._lib.mgym_get_param_redraw(self._h, C.byref(on), lo, hi))
+        if not on.value:
+            return None
+        p = len(self.param_names(self.kind))
+        return tuple(lo[:p]), tuple(hi[:p])
 
     @property
     def step_index(self):
