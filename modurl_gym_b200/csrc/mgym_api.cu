@@ -43,7 +43,7 @@ struct mgym_env {
   int device = 0;
   uint64_t seed = 0;
   mgym_config cfg{};
-  int cnt_mode = CNT_NONE;
+  int cnt_mode = CNT_U32;
   bool vec4 = false;  // n % 4 == 0 and env_index_base % 4 == 0
 
   float* state = nullptr;
@@ -136,9 +136,7 @@ static_assert(Env<0>::NP == 6 && Env<1>::NP == 2 && Env<2>::NP == 2 && Env<3>::N
               "parameter tables and Env<KIND>::NP disagree");
 
 bool valid_kind(int kind) { return kind >= 0 && kind < MGYM_NUM_KINDS; }
-size_t counter_width(int cnt_mode) {
-  return cnt_mode == CNT_NONE ? 0 : ((cnt_mode == CNT_U16 || cnt_mode == CNT_S16) ? 2 : 4);
-}
+size_t counter_width(int cnt_mode) { return cnt_mode == CNT_S16 ? 2 : 4; }
 size_t action_size(int kind) { return kContinuous[kind] ? sizeof(float) : sizeof(uint8_t); }
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
@@ -220,14 +218,6 @@ KernelParams base_params(const mgym_env* e) {
   return p;
 }
 
-int env_blocks_per_sm() {
-  static int v = [] {
-    const char* s = getenv("MGYM_BLOCKS_PER_SM");
-    return s ? atoi(s) : 0;
-  }();
-  return v;
-}
-
 // Occupancy of a kernel is a per-device constant: query it once per (kernel instantiation, device).
 constexpr int kMaxDevices = 64;
 
@@ -262,7 +252,6 @@ int launch_persistent(void (*kernel)(KP), const mgym_env* e, const KP& p, uint64
     if (per_sm < 1) per_sm = 1;
     g_occupancy.put(reinterpret_cast<const void*>(kernel), e->device, per_sm);
   }
-  if (env_blocks_per_sm() > 0) per_sm = env_blocks_per_sm();
   uint64_t blocks = (uint64_t)e->num_sms * per_sm;
   const uint64_t need = (groups + threads - 1) / threads;
   if (blocks > need) blocks = need;
@@ -289,7 +278,6 @@ int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cud
     if (per_sm < 1) per_sm = 1;
     if (e->device < kMaxDevices) cached_per_sm[e->device] = per_sm;
   }
-  if (env_blocks_per_sm() > 0) per_sm = env_blocks_per_sm();
   // persistent CTAs, tiles handed out by tickets (see the producer warp)
   const uint64_t slots = (uint64_t)e->num_sms * per_sm;
   const uint64_t tiles = p.n / TMA_TILE;
@@ -309,10 +297,6 @@ int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cud
     p.work_base = e->work_issued[e->work_slot];
     e->work_issued[e->work_slot] += tiles + blocks;
   }
-  static const bool pdl = [] {
-    const char* s = getenv("MGYM_NO_PDL");
-    return !(s && atoi(s) != 0);
-  }();
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)blocks);
   cfg.blockDim = dim3(threads);
@@ -322,17 +306,9 @@ int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cud
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   MGYM_CUDA(cudaLaunchKernelEx(&cfg, kernel, p));
   return MGYM_OK;
-}
-
-bool use_tma() {
-  static bool v = [] {
-    const char* s = getenv("MGYM_NO_TMA");
-    return !(s && atoi(s) != 0);
-  }();
-  return v;
 }
 
 // kind x vector width x auto/manual x counter representation (x per-env parameters (x per-episode redraw: auto-reset
@@ -344,11 +320,10 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStrea
   if constexpr (!ROLLOUT && V == 4) {
     // manual mode (the reference's protocol): counters are 32-bit, CartPole adds steps_beyond_terminated
     if constexpr (!REDRAW) {
-      if (!autor && use_tma() && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
+      if (!autor && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
     }
-    if (autor && use_tma() && p.n % TMA_TILE == 0) {
-      if constexpr (KIND == 0) {  // CartPole always counts (500-step truncation, cartpole.rs:297)
-        if (e->cnt_mode == CNT_U16) return launch_step_tma<KIND, CNT_U16, true, PARAMS, REDRAW>(e, p, st);
+    if (autor && p.n % TMA_TILE == 0) {
+      if constexpr (KIND == 0) {  // CartPole's handles are all CNT_S16 (500-step truncation, cartpole.rs:297)
         return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW>(e, p, st);
       } else {
         switch (e->cnt_mode) {
@@ -358,7 +333,7 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStrea
         }
       }
     }
-    if (use_tma() && p.n > TMA_TILE) {
+    if (p.n > TMA_TILE) {
       // ragged size: whole 1024-env tiles on the TMA kernel, the remaining (< 1024) envs on the vector kernel
       KParams<PARAMS, REDRAW> head = p, tail = p;
       head.adv_dt = 0;  // device clock: the tail launch (last of the call) moves the step index on
@@ -389,7 +364,6 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStrea
     if (!autor) MGYM_LAUNCH(false, CNT_U32);
   }
   if constexpr (KIND == 0) {
-    if (e->cnt_mode == CNT_U16) MGYM_LAUNCH(true, CNT_U16);
     MGYM_LAUNCH(true, CNT_S16);
   } else {
     switch (e->cnt_mode) {  // these kernels hold the count in registers: a lazy stamp is an ordinary one here
@@ -458,7 +432,6 @@ int launch_reset_kind(const mgym_env* e, const KernelParams& p, const uint8_t* m
     else reset_kernel<KIND, CNT_><<<blocks, 256, 0, st>>>(p, mask, e->n_resets);                \
   } while (0)
   switch (e->cnt_mode) {
-    case CNT_U16: MGYM_RESET(CNT_U16); break;
     case CNT_U32: MGYM_RESET(CNT_U32); break;
     case CNT_S16: MGYM_RESET(CNT_S16); break;
     default: MGYM_RESET(CNT_S32); break;  // CNT_S32 and CNT_S32_LAZY share the representation
@@ -694,10 +667,7 @@ int mgym_create(int kind, uint64_t num_envs, int device_ordinal, uint64_t seed, 
   if (!cfg.auto_reset) {
     e->cnt_mode = CNT_U32;  // the reference's steps_since_reset (cartpole.rs:24)
   } else if (kind == MGYM_CARTPOLE_V1) {
-    // <= 500 between resets: a 16-bit start stamp (read-only per step); MGYM_CARTPOLE_COUNTER=u16 selects the
-    // round-1 read+write counter for A/B measurements
-    const char* s = getenv("MGYM_CARTPOLE_COUNTER");
-    e->cnt_mode = (s && strcmp(s, "u16") == 0) ? CNT_U16 : CNT_S16;
+    e->cnt_mode = CNT_S16;  // <= 500 between resets: a 16-bit start stamp (read-only per step)
   } else if (cfg.max_episode_steps > 0 && cfg.max_episode_steps <= 65535) {
     e->cnt_mode = CNT_S16;
   } else if (cfg.max_episode_steps > 65535) {
@@ -717,10 +687,9 @@ int mgym_create(int kind, uint64_t num_envs, int device_ordinal, uint64_t seed, 
     const size_t n = (size_t)num_envs;
     MGYM_CUDA(cudaMalloc(&e->state, sizeof(float) * kStateDim[kind] * n));
     MGYM_CUDA(cudaMemset(e->state, 0, sizeof(float) * kStateDim[kind] * n));  // cartpole.rs:85 zero state
-    if (e->cnt_mode != CNT_NONE) {  // count 0, or start stamp 0 = the handle's step index right now
-      MGYM_CUDA(cudaMalloc(&e->steps, counter_width(e->cnt_mode) * n));
-      MGYM_CUDA(cudaMemset(e->steps, 0, counter_width(e->cnt_mode) * n));
-    }
+    // count 0, or start stamp 0 = the handle's step index right now
+    MGYM_CUDA(cudaMalloc(&e->steps, counter_width(e->cnt_mode) * n));
+    MGYM_CUDA(cudaMemset(e->steps, 0, counter_width(e->cnt_mode) * n));
     if (!cfg.auto_reset && kind == MGYM_CARTPOLE_V1) {
       MGYM_CUDA(cudaMalloc(&e->sbt, sizeof(uint32_t) * n));
       fill_u32_kernel<<<(unsigned)((n + 255) / 256), 256>>>(e->sbt, 1u, n);  // cartpole.rs:81 Some(0)
@@ -830,27 +799,24 @@ int mgym_set_state(mgym_env* e, const float* state, const uint32_t* steps, const
   const size_t n = (size_t)e->n;
   const unsigned blocks = (unsigned)((n + 255) / 256);
   MGYM_CUDA(cudaMemcpyAsync(e->state, state, sizeof(float) * kStateDim[e->kind] * n, cudaMemcpyDefault, st));
-  if (e->cnt_mode != CNT_NONE) {
-    // the caller's uint32 counts -> this handle's representation (a count, or a start stamp relative to t)
-    const uint32_t* src = steps;
-    uint32_t* tmp = nullptr;
-    if (steps && is_host_pointer(steps)) {  // set_state/get_state also accept host arrays
-      MGYM_CUDA(cudaMalloc(&tmp, sizeof(uint32_t) * n));
-      MGYM_CUDA(cudaMemcpyAsync(tmp, steps, sizeof(uint32_t) * n, cudaMemcpyHostToDevice, st));
-      src = tmp;
-    }
-    const unsigned long long* td = e->cfg.device_clock ? e->clock : nullptr;
-    switch (e->cnt_mode) {
-      case CNT_U16: counters_from_steps_kernel<CNT_U16><<<blocks, 256, 0, st>>>(src, (uint16_t*)e->steps, n, e->t, td); break;
-      case CNT_U32: counters_from_steps_kernel<CNT_U32><<<blocks, 256, 0, st>>>(src, (uint32_t*)e->steps, n, e->t, td); break;
-      case CNT_S16: counters_from_steps_kernel<CNT_S16><<<blocks, 256, 0, st>>>(src, (uint16_t*)e->steps, n, e->t, td); break;
-      default: counters_from_steps_kernel<CNT_S32><<<blocks, 256, 0, st>>>(src, (uint32_t*)e->steps, n, e->t, td); break;
-    }
-    MGYM_CUDA(cudaGetLastError());
-    if (tmp) {
-      MGYM_CUDA(cudaStreamSynchronize(st));
-      cudaFree(tmp);
-    }
+  // the caller's uint32 counts -> this handle's representation (a count, or a start stamp relative to t)
+  const uint32_t* src = steps;
+  uint32_t* tmp = nullptr;
+  if (steps && is_host_pointer(steps)) {  // set_state/get_state also accept host arrays
+    MGYM_CUDA(cudaMalloc(&tmp, sizeof(uint32_t) * n));
+    MGYM_CUDA(cudaMemcpyAsync(tmp, steps, sizeof(uint32_t) * n, cudaMemcpyHostToDevice, st));
+    src = tmp;
+  }
+  const unsigned long long* td = e->cfg.device_clock ? e->clock : nullptr;
+  switch (e->cnt_mode) {
+    case CNT_U32: counters_from_steps_kernel<CNT_U32><<<blocks, 256, 0, st>>>(src, (uint32_t*)e->steps, n, e->t, td); break;
+    case CNT_S16: counters_from_steps_kernel<CNT_S16><<<blocks, 256, 0, st>>>(src, (uint16_t*)e->steps, n, e->t, td); break;
+    default: counters_from_steps_kernel<CNT_S32><<<blocks, 256, 0, st>>>(src, (uint32_t*)e->steps, n, e->t, td); break;
+  }
+  MGYM_CUDA(cudaGetLastError());
+  if (tmp) {
+    MGYM_CUDA(cudaStreamSynchronize(st));
+    cudaFree(tmp);
   }
   if (e->sbt) {
     if (sbt) MGYM_CUDA(cudaMemcpyAsync(e->sbt, sbt, sizeof(uint32_t) * n, cudaMemcpyDefault, st));
@@ -868,31 +834,24 @@ int mgym_get_state(mgym_env* e, float* state, uint32_t* steps, uint32_t* sbt, vo
   const unsigned blocks = (unsigned)((n + 255) / 256);
   if (state) MGYM_CUDA(cudaMemcpyAsync(state, e->state, sizeof(float) * kStateDim[e->kind] * n, cudaMemcpyDefault, st));
   if (steps) {
-    if (e->cnt_mode != CNT_NONE) {
-      const bool host = is_host_pointer(steps);
-      uint32_t* dst = steps;
-      uint32_t* tmp = nullptr;
-      if (host) {
-        MGYM_CUDA(cudaMalloc(&tmp, sizeof(uint32_t) * n));
-        dst = tmp;
-      }
-      const unsigned long long* td = e->cfg.device_clock ? e->clock : nullptr;
-      switch (e->cnt_mode) {
-        case CNT_U16: steps_from_counters_kernel<CNT_U16><<<blocks, 256, 0, st>>>((const uint16_t*)e->steps, dst, n, e->t, td); break;
-        case CNT_U32: steps_from_counters_kernel<CNT_U32><<<blocks, 256, 0, st>>>((const uint32_t*)e->steps, dst, n, e->t, td); break;
-        case CNT_S16: steps_from_counters_kernel<CNT_S16><<<blocks, 256, 0, st>>>((const uint16_t*)e->steps, dst, n, e->t, td); break;
-        default: steps_from_counters_kernel<CNT_S32><<<blocks, 256, 0, st>>>((const uint32_t*)e->steps, dst, n, e->t, td); break;
-      }
-      MGYM_CUDA(cudaGetLastError());
-      if (host) {
-        MGYM_CUDA(cudaMemcpyAsync(steps, tmp, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st));
-        MGYM_CUDA(cudaStreamSynchronize(st));
-        cudaFree(tmp);
-      }
-    } else if (is_host_pointer(steps)) {
-      memset(steps, 0, sizeof(uint32_t) * n);
-    } else {
-      MGYM_CUDA(cudaMemsetAsync(steps, 0, sizeof(uint32_t) * n, st));
+    const bool host = is_host_pointer(steps);
+    uint32_t* dst = steps;
+    uint32_t* tmp = nullptr;
+    if (host) {
+      MGYM_CUDA(cudaMalloc(&tmp, sizeof(uint32_t) * n));
+      dst = tmp;
+    }
+    const unsigned long long* td = e->cfg.device_clock ? e->clock : nullptr;
+    switch (e->cnt_mode) {
+      case CNT_U32: steps_from_counters_kernel<CNT_U32><<<blocks, 256, 0, st>>>((const uint32_t*)e->steps, dst, n, e->t, td); break;
+      case CNT_S16: steps_from_counters_kernel<CNT_S16><<<blocks, 256, 0, st>>>((const uint16_t*)e->steps, dst, n, e->t, td); break;
+      default: steps_from_counters_kernel<CNT_S32><<<blocks, 256, 0, st>>>((const uint32_t*)e->steps, dst, n, e->t, td); break;
+    }
+    MGYM_CUDA(cudaGetLastError());
+    if (host) {
+      MGYM_CUDA(cudaMemcpyAsync(steps, tmp, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st));
+      MGYM_CUDA(cudaStreamSynchronize(st));
+      cudaFree(tmp);
     }
   }
   if (sbt) {

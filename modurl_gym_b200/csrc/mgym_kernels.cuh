@@ -18,26 +18,6 @@
 
 #include "mgym_device.cuh"
 
-#ifndef MGYM_MIN_BLOCKS
-#define MGYM_MIN_BLOCKS 1
-#endif
-#ifndef MGYM_EXP_MEMONLY
-#define MGYM_EXP_MEMONLY 0
-#endif
-#ifndef MGYM_ROLLOUT_MIN_BLOCKS
-#define MGYM_ROLLOUT_MIN_BLOCKS 0  // 0 = per kind, see rollout_min_blocks
-#endif
-#ifndef MGYM_TMA_MIN_BLOCKS
-#define MGYM_TMA_MIN_BLOCKS 2
-#endif
-
-#ifndef MGYM_STEP_BATCH_PAIRS
-#define MGYM_STEP_BATCH_PAIRS false  // true: step_kernel_tma runs Acrobot as two batches of two envs (see step_group)
-#endif
-#ifndef MGYM_ACT_RING
-#define MGYM_ACT_RING 8  // rollout: steps of action look-ahead staged in shared memory (power of two)
-#endif
-
 namespace mgym {
 
 // cp.async (LDGSTS): global -> shared without passing through registers; completion is tracked per thread in
@@ -57,11 +37,11 @@ __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(PENDING) : "memory");
 }
 
-// Per-env episode step count, as the handle keeps it between launches:
-//   CNT_NONE      nothing.  Not used by handles any more: an auto-reset handle always knows the length of a finished
-//                 episode (it keys the reset stream, see reset_pending), a manual one keeps the reference's counters
-//   CNT_U16/U32   the count itself, read AND written by every step (manual mode = the reference's steps_since_reset,
-//                 cartpole.rs:24; CNT_U16 is the round-1 CartPole form, kept for A/B measurements)
+// Per-env episode step count, as the handle keeps it between launches.  Every handle keeps one: an auto-reset
+// handle needs the length of a finished episode (it keys the reset stream, see reset_pending), a manual one keeps the
+// reference's counters.
+//   CNT_U32       the count itself, read AND written by every step (manual mode = the reference's steps_since_reset,
+//                 cartpole.rs:24)
 //   CNT_S16/S32   a START STAMP: the handle's step index t at which the episode began (mod 2^16 / 2^32).  The count is
 //                 (t - stamp), so a step only READS the stamp; it is written when an episode ends (by the lane that
 //                 owns the finished env) -- 2 or 4 bytes read per env-step instead of a read and a write.
@@ -69,15 +49,16 @@ __device__ __forceinline__ void cp_async_wait() {
 //                 (statistics, reset stream): not even read by a step unless the env finished (MountainCar-v0: 22 B per env-step,
 //                 the SURVEY 8(d) contract figure, instead of 30).  Kernels that keep the count in registers anyway
 //                 (rollout, the LDG step form) treat it as CNT_S32.
-enum CounterMode : int { CNT_NONE = 0, CNT_U16 = 1, CNT_U32 = 2, CNT_S16 = 3, CNT_S32 = 4, CNT_S32_LAZY = 5 };
+// The values are stored in checkpoints (the header's cnt_mode): never renumber them.
+enum CounterMode : int { CNT_U32 = 2, CNT_S16 = 3, CNT_S32 = 4, CNT_S32_LAZY = 5 };
 __host__ __device__ constexpr bool cnt_is_stamp(int c) { return c >= CNT_S16; }
 __host__ __device__ constexpr bool cnt_is_lazy(int c) { return c == CNT_S32_LAZY; }
-__host__ __device__ constexpr bool cnt_staged(int c) { return c != CNT_NONE && c != CNT_S32_LAZY; }  // read by every step
+__host__ __device__ constexpr bool cnt_staged(int c) { return c != CNT_S32_LAZY; }  // read by every step
 
 struct KernelParams {
   // resident env state (owned by the handle)
   float* state;        // [SD][n]
-  void* steps;         // uint16_t[n] or uint32_t[n] or null, see CounterMode
+  void* steps;         // uint16_t[n] or uint32_t[n], see CounterMode
   uint32_t* sbt;       // manual CartPole only: steps_beyond_terminated (0 = None, k+1 = Some(k))
   float* ep_return;    // per-env running return (kinds without an analytic return), or null
   // caller buffers
@@ -481,9 +462,8 @@ __device__ __noinline__ LaneIO<KIND, V> dynamics_reference_lane(LaneIO<KIND, V> 
 // REDRAW (RESET_IN_PLACE, p is a KernelParamsR): the reset also redraws the finished envs' parameter rows in global
 // memory (the step itself ran on the old ones, in prm).
 template <int KIND, int V, bool AUTO, bool WANT_FINAL, bool TALLY_LEN = true, int RESET = RESET_IN_PLACE,
-          bool TRUSTED = false, bool OBS_VALID = false, bool BATCH_PAIRS = false, typename PR = NoParams,
-          bool REDRAW = false>
-__device__ __forceinline__ uint32_t step_group(const KernelParams& p, bool count, uint64_t base, uint64_t t,
+          bool TRUSTED = false, bool OBS_VALID = false, typename PR = NoParams, bool REDRAW = false>
+__device__ __forceinline__ void step_group(const KernelParams& p, bool count, uint64_t base, uint64_t t,
                                            const typename Env<KIND>::act_t (&action)[V], bool track_ret,
                                            Group<KIND, V>& g, StatAcc& acc, const PR& prm = PR{}) {
   using E = Env<KIND>;
@@ -525,21 +505,7 @@ __device__ __forceinline__ uint32_t step_group(const KernelParams& p, bool count
 #pragma unroll
       for (int c = 0; c < E::SD; ++c) old[v][c] = g.st[v][c];
     }
-    if constexpr (BATCH_PAIRS && V == 4) {
-      // two batches of two: half the loop body (Acrobot's rolled RK4 loop then stalls less on instruction
-      // fetch) for half the instruction-level parallelism.  With the scalar derivative this was +7 % in the
-      // per-call step kernel (-2 % in the rollout); with the packed f32x2 derivative a batch of two is ONE chain
-      // of packed operations, and the batch of four wins again (+4 %), so nobody asks for it now.
-      using act_t = typename E::act_t;
-      bool ok2[2];
-      const act_t a01[2] = {action[0], action[1]}, a23[2] = {action[2], action[3]};
-      E::template dynamics_fast_batch<2>(*reinterpret_cast<float(*)[2][E::SD]>(&g.st[0]), a01, p.k, ok2);
-      ok[0] = ok2[0], ok[1] = ok2[1];
-      E::template dynamics_fast_batch<2>(*reinterpret_cast<float(*)[2][E::SD]>(&g.st[2]), a23, p.k, ok2);
-      ok[2] = ok2[0], ok[3] = ok2[1];
-    } else {
-      E::template dynamics_fast_batch<V>(g.st, action, p.k, ok);
-    }
+    E::template dynamics_fast_batch<V>(g.st, action, p.k, ok);
 #pragma unroll
     for (int v = 0; v < V; ++v) all_ok = all_ok && ok[v];
     if (!all_ok) {
@@ -637,16 +603,11 @@ __device__ __forceinline__ uint32_t step_group(const KernelParams& p, bool count
     redraw_pending<KIND, V>(p, base, t, pending, g, rd);
   }
   if constexpr (AUTO && RESET == RESET_IN_PLACE) reset_pending<KIND, V>(p, base, t, pending, g);
-  return 0u;
 }
 
 template <int MODE>
 struct CounterType {
   using type = uint32_t;
-};
-template <>
-struct CounterType<CNT_U16> {
-  using type = uint16_t;
 };
 template <>
 struct CounterType<CNT_S16> {
@@ -671,7 +632,7 @@ __device__ __forceinline__ typename CounterType<CNT>::type cnt_encode(uint32_t s
 // =============================================================================================
 // REDRAW: every reset also redraws the env's parameter rows (mgym_set_param_redraw; auto-reset with rows only).
 template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false, bool REDRAW = false>
-__global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
+__global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
@@ -679,7 +640,6 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
   constexpr int SD = E::SD, OD = E::OD;
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
-  static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
   StatAcc acc;
   const uint64_t groups = p.n / V;
   const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -705,8 +665,7 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
 #pragma unroll
       for (int c = 0; c < SD; ++c) s[c] = ldv<float, V>(p.state + (uint64_t)c * p.ld + base);
       const Vec<act_t, V> a = ldv<act_t, V>(reinterpret_cast<const act_t*>(p.actions) + base);
-      Vec<cnt_t, V> cnt;
-      if constexpr (CNT != CNT_NONE) cnt = ldv<cnt_t, V>(reinterpret_cast<const cnt_t*>(p.steps) + base);
+      const Vec<cnt_t, V> cnt = ldv<cnt_t, V>(reinterpret_cast<const cnt_t*>(p.steps) + base);
       Vec<uint32_t, V> sb;
       if constexpr (!AUTO && KIND == 0) sb = ldv<uint32_t, V>(p.sbt + base);
       Vec<float, V> er;
@@ -716,20 +675,18 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
 #pragma unroll
         for (int c = 0; c < SD; ++c) g.st[v][c] = s[c].v[v];
         action[v] = a.v[v];
-        g.steps[v] = 0;
+        g.steps[v] = cnt_decode<CNT>(cnt.v[v], t_now);
         g.sbt[v] = SBT_NONE;
-        if constexpr (CNT != CNT_NONE) g.steps[v] = cnt_decode<CNT>(cnt.v[v], t_now);
         if constexpr (!AUTO && KIND == 0) g.sbt[v] = sb.v[v];
         g.ret[v] = track_ret ? er.v[v] : 0.0f;
       }
     }
     if (want_final)
-      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, false, PR, REDRAW>(p, true, base, t_now, action,
-                                                                                            track_ret, g, acc, prm);
+      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, PR, REDRAW>(p, true, base, t_now, action, track_ret,
+                                                                                     g, acc, prm);
     else
-      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, false, PR, REDRAW>(p, true, base, t_now,
-                                                                                             action, track_ret, g, acc,
-                                                                                             prm);
+      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, PR, REDRAW>(p, true, base, t_now, action, track_ret,
+                                                                                      g, acc, prm);
 
     {
       Vec<float, V> s[SD];
@@ -740,14 +697,12 @@ __global__ void __launch_bounds__(256, MGYM_MIN_BLOCKS) step_kernel(const __grid
         stv<float, V>(p.state + (uint64_t)c * p.ld + base, s[c]);
       }
     }
-    if constexpr (CNT != CNT_NONE) {
-      // a start stamp only changes when an episode ended (the count of a finished env is 0 again by now)
-      if (!cnt_is_stamp(CNT) || packed_flags<KIND, V>(g) != 0u) {
-        Vec<cnt_t, V> cnt;
+    // a start stamp only changes when an episode ended (the count of a finished env is 0 again by now)
+    if (!cnt_is_stamp(CNT) || packed_flags<KIND, V>(g) != 0u) {
+      Vec<cnt_t, V> cnt;
 #pragma unroll
-        for (int v = 0; v < V; ++v) cnt.v[v] = cnt_encode<CNT>(g.steps[v], t_now + 1);
-        stv<cnt_t, V>(reinterpret_cast<cnt_t*>(p.steps) + base, cnt);
-      }
+      for (int v = 0; v < V; ++v) cnt.v[v] = cnt_encode<CNT>(g.steps[v], t_now + 1);
+      stv<cnt_t, V>(reinterpret_cast<cnt_t*>(p.steps) + base, cnt);
     }
     if constexpr (!AUTO && KIND == 0) {
       Vec<uint32_t, V> sb;
@@ -838,10 +793,7 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 }
 }  // namespace tma
 
-#ifndef MGYM_TMA_STAGES
-#define MGYM_TMA_STAGES 4
-#endif
-constexpr int TMA_STAGES = MGYM_TMA_STAGES;
+constexpr int TMA_STAGES = 4;
 constexpr int TMA_CONSUMER_WARPS = 8;
 constexpr int TMA_THREADS = (TMA_CONSUMER_WARPS + 2) * 32;  // + one producer warp + one reset warp
 constexpr int TMA_RESET_BUFFERS = 2;                         // request queues in flight
@@ -905,7 +857,7 @@ struct TmaLayout {
 // with the staged (old) rows; no other tile of the launch holds the env, and the next launch's producer reads the
 // rows only after griddepcontrol.wait.  Stage layout and stage count are those of the PARAMS form.
 template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false>
-__global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS)
+__global__ void __launch_bounds__(TMA_THREADS, 2)
     step_kernel_tma(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
   using E = Env<KIND>;
   using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
@@ -916,7 +868,6 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS)
   using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(AUTO || !cnt_is_stamp(CNT), "manual mode keeps the reference's own counters");
-  static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (tma::smem_u32(smem_raw) + 127u) & ~127u;
   const uint32_t warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);  // warp-uniform for the compiler
@@ -1101,27 +1052,17 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS)
       __syncwarp();  // every lane of this warp has its values in registers
       if (lane == 0) tma::mbar_arrive(empty0 + 8 * s);
 
-#if MGYM_EXP_MEMONLY
-      // experiment: the memory traffic of the step without its arithmetic (profiles/README.md)
-#pragma unroll
-      for (int v = 0; v < V; ++v) {
-        g.reward[v] = g.st[v][0] + (float)action[v];
-        g.flags[v] = g.steps[v] & 1u;
-        g.steps[v] += 1;
-      }
-#else
       if (want_final)
-        step_group<KIND, V, AUTO, true, true, RESET_BY_CALLER, false, false, MGYM_STEP_BATCH_PAIRS, PR>(p, true, base, t_now, action, track_ret, g,
-                                                                                   acc, prm);
+        step_group<KIND, V, AUTO, true, true, RESET_BY_CALLER, false, false, PR>(p, true, base, t_now, action, track_ret,
+                                                                                  g, acc, prm);
       else
-        step_group<KIND, V, AUTO, false, true, RESET_BY_CALLER, false, false, MGYM_STEP_BATCH_PAIRS, PR>(p, true, base, t_now, action, track_ret,
-                                                                                    g, acc, prm);
-#endif
+        step_group<KIND, V, AUTO, false, true, RESET_BY_CALLER, false, false, PR>(p, true, base, t_now, action, track_ret,
+                                                                                   g, acc, prm);
       // Everything about this lane's finished envs sits in one branch: statistics from the packed flags word,
       // counters cleared, and their index inside the tile appended to the reset queue.
       const uint32_t fw = packed_flags<KIND, V>(g);
-      // the memory-only experiment finishes nothing; in manual mode finished envs wait for the caller's reset
-      const uint32_t fin = (MGYM_EXP_MEMONLY || !AUTO) ? 0u : fw;
+      // in manual mode finished envs wait for the caller's reset
+      const uint32_t fin = AUTO ? fw : 0u;
       if (fin) {
         if constexpr (cnt_is_lazy(CNT)) {
           // the episode length is only needed now: the stamps of this lane's envs come straight from global memory
@@ -1158,7 +1099,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS)
         for (int v = 0; v < V; ++v) o.v[v] = g.st[v][c];
         stv<float, V>(p.state + (uint64_t)c * p.ld + base, o);
       }
-      if constexpr (CNT != CNT_NONE && !cnt_is_stamp(CNT)) {
+      if constexpr (!cnt_is_stamp(CNT)) {
         Vec<cnt_t, V> cnt;
 #pragma unroll
         for (int v = 0; v < V; ++v) cnt.v[v] = (cnt_t)g.steps[v];
@@ -1223,7 +1164,7 @@ __global__ void __launch_bounds__(TMA_THREADS, MGYM_TMA_MIN_BLOCKS)
 // the kinds fit 80 registers without spilling (measured: +8..11 % at 3 CTAs); Acrobot's RK4 does not (-6 %).
 template <int KIND>
 constexpr int rollout_min_blocks() {
-  return MGYM_ROLLOUT_MIN_BLOCKS > 0 ? MGYM_ROLLOUT_MIN_BLOCKS : (KIND == 4 ? 2 : 3);
+  return KIND == 4 ? 2 : 3;
 }
 
 // PARAMS: the NP parameters of each env are read once per warp tile into per-thread shared-memory slots (like the
@@ -1245,8 +1186,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!FULL || (AUTO && V == 4), "the FULL form is built for the vector auto-reset path only");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
-  static_assert(!AUTO || CNT != CNT_NONE, "auto-reset needs the episode length: it keys the reset stream");
-  constexpr int ACT_RING = PARAMS ? MGYM_ACT_RING / 2 : MGYM_ACT_RING;
+  constexpr int ACT_RING = PARAMS ? 4 : 8;  // steps of action look-ahead staged in shared memory
   __shared__ float par_slots[PARAMS ? E::NP * V : 1][PARAMS ? 256 : 1];  // [c * V + v][thread]
   static_assert((ACT_RING & (ACT_RING - 1)) == 0, "power of two");
   constexpr uint32_t RING_STRIDE = 256 * V * sizeof(act_t);  // one row of the CTA: 256 threads x V actions
@@ -1295,11 +1235,9 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
 #pragma unroll
         for (int v = 0; v < V; ++v) g.st[v][c] = s.v[v];
       }
-      if constexpr (CNT != CNT_NONE) {
-        const Vec<cnt_t, V> cnt = ldv<cnt_t, V>(reinterpret_cast<const cnt_t*>(p.steps) + base);
+      const Vec<cnt_t, V> cnt = ldv<cnt_t, V>(reinterpret_cast<const cnt_t*>(p.steps) + base);
 #pragma unroll
-        for (int v = 0; v < V; ++v) g.steps[v] = cnt_decode<CNT>(cnt.v[v], t_first);
-      }
+      for (int v = 0; v < V; ++v) g.steps[v] = cnt_decode<CNT>(cnt.v[v], t_first);
       if constexpr (!AUTO && KIND == 0) {
         const Vec<uint32_t, V> sb = ldv<uint32_t, V>(p.sbt + base);
 #pragma unroll
@@ -1327,7 +1265,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
 #pragma unroll
       for (int v = 0; v < V; ++v) E::obs(g.st[v], g.obs[v]);
     }
-    // Actions are staged MGYM_ACT_RING steps ahead in shared memory with cp.async: every lane copies its own
+    // Actions are staged ACT_RING steps ahead in shared memory with cp.async: every lane copies its own
     // 4 (uint8) or 16 (float) bytes of the row ACT_RING steps ahead and later reads back exactly those bytes, so no
     // cross-lane synchronisation is needed, only its own commit groups.  A load issued one step ahead into a
     // register (round 1, plus an L1 prefetch four rows ahead) arrived late under the write-heavy DRAM traffic of a
@@ -1351,9 +1289,8 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
 
     // Sum of the lengths of the episodes an env finishes during this launch = steps_before + K - steps_after,
     // so the per-step tally is not needed here (counters saturate only after 4e9 steps).
-    constexpr bool kLenIdentity = AUTO && CNT != CNT_NONE;
     uint32_t steps_before = 0;
-    if constexpr (kLenIdentity) {
+    if constexpr (AUTO) {
 #pragma unroll
       for (int v = 0; v < V; ++v) steps_before += g.steps[v];
     }
@@ -1437,8 +1374,8 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
           for (int v = 0; v < V; ++v) prm.r[c][v] = *static_cast<volatile const float*>(&par_slots[c * V + v][threadIdx.x]);
         }
       }
-      step_group<KIND, V, AUTO, false, false, RESET_BY_CALLER, TRUSTED, true, false, PR>(p, active, base, t, action,
-                                                                                         track_ret, g, acc, prm);
+      step_group<KIND, V, AUTO, false, false, RESET_BY_CALLER, TRUSTED, true, PR>(p, active, base, t, action, track_ret,
+                                                                                  g, acc, prm);
 
       // ---- trajectory stores (before the resets: reward and flags belong to the finishing step; the
       // observation is stored after them, it is the post-reset one) ----
@@ -1466,7 +1403,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
       if (__ballot_sync(0xffffffffu, wf != 0u) != 0u) {
         dones += __popc((wf | (wf >> 1)) & 0x01010101u);
         if constexpr (AUTO) {
-          tally_packed<KIND, V, !kLenIdentity>(wf, g, acc);
+          tally_packed<KIND, V, false>(wf, g, acc);
           uint32_t pending = 0;
 #pragma unroll
           for (int v = 0; v < V; ++v) pending |= ((wf >> (8 * v)) & 0xffu) ? (1u << v) : 0u;
@@ -1541,7 +1478,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
     if constexpr (STAGED) {
       if (!policy) cp_async_wait<0>();  // the ring is reused by this warp's next tile
     }
-    if constexpr (kLenIdentity) {
+    if constexpr (AUTO) {
       if (active) {
         uint32_t steps_after = 0;
 #pragma unroll
@@ -1558,12 +1495,10 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
         for (int v = 0; v < V; ++v) s.v[v] = g.st[v][c];
         stv<float, V>(p.state + (uint64_t)c * p.ld + base, s);
       }
-      if constexpr (CNT != CNT_NONE) {
-        Vec<cnt_t, V> cnt;
+      Vec<cnt_t, V> cnt;
 #pragma unroll
-        for (int v = 0; v < V; ++v) cnt.v[v] = cnt_encode<CNT>(g.steps[v], t_first + p.K);
-        stv<cnt_t, V>(reinterpret_cast<cnt_t*>(p.steps) + base, cnt);
-      }
+      for (int v = 0; v < V; ++v) cnt.v[v] = cnt_encode<CNT>(g.steps[v], t_first + p.K);
+      stv<cnt_t, V>(reinterpret_cast<cnt_t*>(p.steps) + base, cnt);
       if constexpr (!AUTO && KIND == 0) {
         Vec<uint32_t, V> sb;
 #pragma unroll
@@ -1613,7 +1548,7 @@ __device__ __forceinline__ void reset_one(const KernelParams& p, uint64_t i, uin
   }
 #pragma unroll
   for (int c = 0; c < E::SD; ++c) p.state[(uint64_t)c * p.ld + i] = st[c];
-  if constexpr (CNT != CNT_NONE) reinterpret_cast<cnt_t*>(p.steps)[i] = cnt_encode<CNT>(0u, launch_t(p));  // cartpole.rs:243
+  reinterpret_cast<cnt_t*>(p.steps)[i] = cnt_encode<CNT>(0u, launch_t(p));  // cartpole.rs:243
   if (p.sbt) p.sbt[i] = SBT_NONE;                                            // cartpole.rs:239
   if (p.ep_return) p.ep_return[i] = 0.0f;
   if (p.obs_out) {
