@@ -137,6 +137,21 @@ impl GpuVecEnv {
                    flags_traj: *mut u8, done_count: *mut u64) -> Result<(), MgymError> {
         check(unsafe { sys::mgym_rollout(self.h, k, actions, obs_traj, reward_traj, flags_traj, done_count, self.stream) })
     }
+    /// `rollout` plus the observation every finished episode ended on (auto-reset handles): where flags_traj[k][i]
+    /// != 0, final_obs_traj[k][c][i] is env i's observation before its reset at step k; other entries are not
+    /// written.  `final_obs_len` is the length in floats of the device buffer `final_obs_traj`, checked against the
+    /// k * obs_dim * N the kernel may write.
+    pub fn rollout_final(&mut self, k: u32, actions: *const c_void, obs_traj: *mut f32, reward_traj: *mut f32,
+                         flags_traj: *mut u8, final_obs_traj: *mut f32, final_obs_len: usize, done_count: *mut u64)
+                         -> Result<(), MgymError> {
+        assert!(!final_obs_traj.is_null(), "final_obs_traj: a device buffer (use rollout without one)");
+        assert!(final_obs_len >= k as usize * self.obs_dim() * self.num_envs as usize,
+                "final_obs_traj: K * obs_dim * N floats, time-major");
+        check(unsafe {
+            sys::mgym_rollout_final(self.h, k, actions, obs_traj, reward_traj, flags_traj, final_obs_traj, done_count,
+                                    self.stream)
+        })
+    }
     /// Host-buffer step for scalar adapters and tests: H2D actions, step, D2H results, synchronises.
     /// Every slice length is checked against what the C side reads or writes (N actions of the kind's own type,
     /// obs_dim * N observations, N rewards, N flags), so this safe function cannot reach out of bounds.

@@ -77,6 +77,9 @@ extern "C" {
     pub fn mgym_rollout(env: *mut mgym_env, k: u32, actions: *const c_void, obs_traj: *mut f32,
                         reward_traj: *mut f32, flags_traj: *mut u8, done_count_out: *mut u64,
                         stream: *mut c_void) -> c_int;
+    pub fn mgym_rollout_final(env: *mut mgym_env, k: u32, actions: *const c_void, obs_traj: *mut f32,
+                              reward_traj: *mut f32, flags_traj: *mut u8, final_obs_traj: *mut f32,
+                              done_count_out: *mut u64, stream: *mut c_void) -> c_int;
     pub fn mgym_sample_actions(env: *mut mgym_env, actions_out: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn mgym_step_host(env: *mut mgym_env, actions_host: *const c_void, obs_host: *mut f32,
                           reward_host: *mut f32, flags_host: *mut u8, stream: *mut c_void) -> c_int;

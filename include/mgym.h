@@ -37,6 +37,8 @@
  *                   an env whose step returns terminated or truncated is reset in the
  *                   same call; obs_out holds the post-reset observation, reward/flags the
  *                   finishing step's values, final_obs_out (optional) the pre-reset obs.
+ *                   mgym_rollout_final keeps the same pre-reset obs for a fused rollout, stored only
+ *                   where an env finished.
  *   Reset states come from a counter-based Philox4x32-10 stream keyed by the seed; the counter is
  *   (global env index, reset call index) for mgym_reset and (global env index, step index at which
  *   the episode that just finished BEGAN) for a same-step auto-reset, so results do not depend on
@@ -186,6 +188,8 @@ int mgym_checkpoint_load(mgym_env *env, const void *host_blob, size_t blob_bytes
 
 /* ---- the hot path ------------------------------------------------------------------ */
 /* One Gym::step for all N envs.  obs_out, reward_out, flags_out, final_obs_out may be NULL.
+ * final_obs_out is DENSE: every env's entry is written (the pre-reset observation where the env finished, the
+ * observation itself elsewhere).  mgym_rollout_final's final_obs_traj is SPARSE: only finished envs are written.
  * CUDA graphs: by default the step index that keys the Philox resets and the tile tickets are per-call launch
  * parameters, so on a capturing stream mgym_step / mgym_rollout / mgym_sample_actions return
  * MGYM_ERR_BAD_ARGUMENT instead of recording a launch whose replay would be wrong.  A handle created with
@@ -199,6 +203,23 @@ int mgym_step(mgym_env *env, const void *actions, float *obs_out, float *reward_
  * done_count_out (device uint64, optional) receives the number of finished env-steps. */
 int mgym_rollout(mgym_env *env, uint32_t K, const void *actions, float *obs_traj, float *reward_traj,
                  uint8_t *flags_traj, unsigned long long *done_count_out, void *stream);
+/* mgym_rollout plus the observation every finished episode ended on.
+ * final_obs_traj: device float[K][obs_dim][N], time-major like obs_traj.  Where flags_traj[k][i] != 0 (env i
+ * finished at step k), final_obs_traj[k][c][i] = the observation step k produced BEFORE the auto-reset: the value
+ * mgym_step's final_obs_out would hold for that env at that step.  Every other entry is NOT written: it keeps what
+ * the caller put there (unlike mgym_step's dense final_obs_out: a dense copy would write every observation twice,
+ * sparse stores cost only where an env finished).  next_obs of transition k is therefore
+ * flags[k] ? final_obs_traj[k] : obs_traj[k].
+ * final_obs_traj == NULL: exactly mgym_rollout.  Everything else (obs_traj, reward_traj, flags_traj, done_count,
+ * state, counters, running returns, statistics, parameter rows and redraws, step index) is bit-identical to
+ * mgym_rollout with the same arguments.  The finishing step runs on the env's old parameters, so with redraw ranges
+ * the final observation is the one those produced; a reset pool changes reset states only.  Needs 4-byte alignment
+ * only.  auto_reset = 0 handles: MGYM_ERR_BAD_ARGUMENT (nothing resets inside the rollout; obs_traj already holds the
+ * final observations).  final_obs_traj == obs_traj: MGYM_ERR_BAD_ARGUMENT.  validate_actions = 1 rejects a bad batch
+ * before anything, final_obs_traj included, is written.  Capturable under the same rules as mgym_rollout
+ * (device_clock handles). */
+int mgym_rollout_final(mgym_env *env, uint32_t K, const void *actions, float *obs_traj, float *reward_traj,
+                       uint8_t *flags_traj, float *final_obs_traj, unsigned long long *done_count_out, void *stream);
 /* Space::sample for all envs at the current step index (same stream mgym_rollout uses). */
 int mgym_sample_actions(mgym_env *env, void *actions_out, void *stream);
 

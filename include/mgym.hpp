@@ -161,6 +161,13 @@ class GpuVecEnv {
                unsigned long long* done_count_device = nullptr) {
     check(mgym_rollout(h_, K, actions_device, obs_traj, reward_traj, flags_traj, done_count_device, stream_));
   }
+  // rollout plus the observation each finished episode ended on: final_obs_traj [K][obs_dim][N] (device) is written
+  // only where flags_traj != 0 (mgym_rollout_final); auto-reset handles only
+  void rollout_final(uint32_t K, const void* actions_device, float* obs_traj, float* reward_traj, uint8_t* flags_traj,
+                     float* final_obs_traj, unsigned long long* done_count_device = nullptr) {
+    check(mgym_rollout_final(h_, K, actions_device, obs_traj, reward_traj, flags_traj, final_obs_traj,
+                             done_count_device, stream_));
+  }
   void sample_actions(void* actions_device) { check(mgym_sample_actions(h_, actions_device, stream_)); }
 
   // ---- Testable (cartpole.rs:436-447) and checkpointing ---------------------------------------------

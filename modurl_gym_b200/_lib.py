@@ -79,6 +79,7 @@ SYMBOLS = {
     "mgym_checkpoint_load": (_i, [_vp, _vp, C.c_size_t, _vp]),
     "mgym_step": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mgym_rollout": (_i, [_vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mgym_rollout_final": (_i, [_vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mgym_sample_actions": (_i, [_vp, _vp, _vp]),
     "mgym_step_host": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "mgym_num_params": (_i, [_i]),

@@ -312,9 +312,11 @@ int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cud
 }
 
 // kind x vector width x auto/manual x counter representation (x per-env parameters (x per-episode redraw: auto-reset
-// handles only, the host never asks for a manual form of it))
-template <int KIND, int V, bool ROLLOUT, bool PARAMS = false, bool REDRAW = false>
+// handles only, the host never asks for a manual form of it)) (x final observations: auto-reset rollouts only,
+// mgym_rollout_final refuses manual handles before it gets here)
+template <int KIND, int V, bool ROLLOUT, bool PARAMS = false, bool REDRAW = false, bool FINAL = false>
 int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStream_t st) {
+  static_assert(!FINAL || ROLLOUT, "final observations are a rollout form");
   const uint64_t groups = p.n / V;
   const bool autor = e->cfg.auto_reset != 0;
   if constexpr (!ROLLOUT && V == 4) {
@@ -353,14 +355,14 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStrea
     if constexpr (ROLLOUT) {                                                                             \
       if constexpr (AUTO_ && V == 4) {                                                                   \
         if (full)                                                                                        \
-          return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS, REDRAW>, e, p, groups, st); \
+          return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS, REDRAW, FINAL>, e, p, groups, st); \
       }                                                                                                  \
-      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS, REDRAW>, e, p, groups, st); \
+      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS, REDRAW, FINAL>, e, p, groups, st); \
     } else {                                                                                             \
       return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS, REDRAW>, e, p, groups, st);     \
     }                                                                                                    \
   } while (0)
-  if constexpr (!REDRAW) {
+  if constexpr (!REDRAW && !FINAL) {
     if (!autor) MGYM_LAUNCH(false, CNT_U32);
   }
   if constexpr (KIND == 0) {
@@ -386,7 +388,7 @@ ParamBox redraw_box(const mgym_env* e) {
 
 // A handle with per-env parameters runs the PARAMS instantiations (kinds that have parameters only), an auto-reset
 // one with redraw ranges the PARAMS + REDRAW instantiations (manual-mode steps never reset).
-template <int KIND, bool ROLLOUT>
+template <int KIND, bool ROLLOUT, bool FINAL>
 int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
   if constexpr (Env<KIND>::NP > 0) {
     if (e->params) {
@@ -397,20 +399,23 @@ int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStrea
         KernelParamsR pr;
         static_cast<KernelParamsP&>(pr) = pp;
         pr.redraw = redraw_box(e);
-        return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true, true>(e, pr, st)
-                    : dispatch_mode<KIND, 1, ROLLOUT, true, true>(e, pr, st);
+        return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true, true, FINAL>(e, pr, st)
+                    : dispatch_mode<KIND, 1, ROLLOUT, true, true, FINAL>(e, pr, st);
       }
-      return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true>(e, pp, st) : dispatch_mode<KIND, 1, ROLLOUT, true>(e, pp, st);
+      return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true, false, FINAL>(e, pp, st)
+                  : dispatch_mode<KIND, 1, ROLLOUT, true, false, FINAL>(e, pp, st);
     }
   }
-  return vec4 ? dispatch_mode<KIND, 4, ROLLOUT>(e, p, st) : dispatch_mode<KIND, 1, ROLLOUT>(e, p, st);
+  return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, false, false, FINAL>(e, p, st)
+              : dispatch_mode<KIND, 1, ROLLOUT, false, false, FINAL>(e, p, st);
 }
 
-template <bool ROLLOUT>
+// FINAL: the rollout forms that also store final observations (mgym_rollout_final)
+template <bool ROLLOUT, bool FINAL = false>
 int dispatch(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
 #define MGYM_KIND(K_)                                               \
   case K_:                                                          \
-    return dispatch_kind<K_, ROLLOUT>(e, p, vec4, st)
+    return dispatch_kind<K_, ROLLOUT, FINAL>(e, p, vec4, st)
   switch (e->kind) {
     MGYM_KIND(0);
     MGYM_KIND(1);
@@ -1072,13 +1077,22 @@ int mgym_step(mgym_env* e, const void* actions, float* obs_out, float* reward_ou
   return advance_clock(e, 1, st, /*fused=*/true);
 }
 
-int mgym_rollout(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
-                 uint8_t* flags_traj, unsigned long long* done_count_out, void* stream) {
-  if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_rollout: env is NULL");
+// mgym_rollout and mgym_rollout_final: a non-null final_obs_traj selects the FINAL kernel forms, null launches exactly
+// what mgym_rollout launches
+static int run_rollout(const char* fn, mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
+                       uint8_t* flags_traj, float* final_obs_traj, unsigned long long* done_count_out, void* stream) {
+  if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "%s: env is NULL", fn);
+  if (final_obs_traj) {
+    if (!e->cfg.auto_reset)
+      return fail(MGYM_ERR_BAD_ARGUMENT, "%s: a manual-mode handle resets nothing inside the rollout; obs_traj "
+                  "already holds the final observations", fn);
+    if (final_obs_traj == obs_traj)
+      return fail(MGYM_ERR_BAD_ARGUMENT, "%s: final_obs_traj must not be obs_traj", fn);
+  }
   if (K == 0) return MGYM_OK;
   DeviceGuard guard(e->device);
   cudaStream_t st = (cudaStream_t)stream;
-  if (int rc = refuse_capture(e, st, "mgym_rollout", true)) return rc;
+  if (int rc = refuse_capture(e, st, fn, true)) return rc;
   if (int rc = validate_device_actions(e, actions, (uint64_t)K * e->n, st)) return rc;
   e->call_tickets = 0;
   KernelParams p = base_params(e);
@@ -1097,9 +1111,26 @@ int mgym_rollout(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, 
   p.work_counter = e->work + 3;
   p.work_base = 0;
   MGYM_CUDA(cudaMemsetAsync(e->work + 3, 0, sizeof(unsigned long long), st));
-  int rc = dispatch<true>(e, p, vec4, st);
+  int rc;
+  if (final_obs_traj) {
+    p.final_obs_out = final_obs_traj;  // float alignment suffices: stored one scalar at a time
+    rc = dispatch<true, true>(e, p, vec4, st);
+  } else {
+    rc = dispatch<true>(e, p, vec4, st);
+  }
   if (rc != MGYM_OK) return rc;
   return advance_clock(e, K, st, /*fused=*/true);
+}
+
+int mgym_rollout(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
+                 uint8_t* flags_traj, unsigned long long* done_count_out, void* stream) {
+  return run_rollout("mgym_rollout", e, K, actions, obs_traj, reward_traj, flags_traj, nullptr, done_count_out, stream);
+}
+
+int mgym_rollout_final(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
+                       uint8_t* flags_traj, float* final_obs_traj, unsigned long long* done_count_out, void* stream) {
+  return run_rollout("mgym_rollout_final", e, K, actions, obs_traj, reward_traj, flags_traj, final_obs_traj,
+                 done_count_out, stream);
 }
 
 int mgym_sample_actions(mgym_env* e, void* actions_out, void* stream) {

@@ -66,7 +66,7 @@ struct KernelParams {
   float* obs_out;       // step: [OD][n]; rollout: [K][OD][n]
   float* reward_out;    // step: [n];     rollout: [K][n]
   uint8_t* flags_out;   // step: [n];     rollout: [K][n]
-  float* final_obs_out; // step only: pre-reset observation [OD][n]
+  float* final_obs_out; // step: pre-reset observation [OD][n]; rollout (FINAL forms): [K][OD][n], finished envs only
   // reset source
   const float* reset_pool;  // [SD][pool_len] or null
   uint64_t pool_len;
@@ -1175,7 +1175,10 @@ constexpr int rollout_min_blocks() {
 // divergent reset pass, straight into its slots (every later step of the tile runs the new episode's constants); the
 // slots are written back to the rows at the end of the tile.  Drawing them ahead of time like the reset states would
 // need 24 KB more of CartPole's slots, i.e. dynamic shared memory (DESIGN.md section 11.1).
-template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false, bool REDRAW = false>
+// FINAL (mgym_rollout_final, auto-reset forms only): the divergent reset pass also stores the observation each
+// finished env ended on, before the reset overwrites it, to p.final_obs_out [K][OD][ld].  Only finished envs are
+// written; the address is computed there from (kk, base), so the hot loop carries no extra pointer.
+template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false, bool REDRAW = false, bool FINAL = false>
 __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
     rollout_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
   using E = Env<KIND>;
@@ -1185,6 +1188,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
   constexpr int SD = E::SD, OD = E::OD;
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!FULL || (AUTO && V == 4), "the FULL form is built for the vector auto-reset path only");
+  static_assert(!FINAL || AUTO, "final observations exist only where the rollout resets");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   constexpr int ACT_RING = PARAMS ? 4 : 8;  // steps of action look-ahead staged in shared memory
   __shared__ float par_slots[PARAMS ? E::NP * V : 1][PARAMS ? 256 : 1];  // [c * V + v][thread]
@@ -1407,6 +1411,16 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
           uint32_t pending = 0;
 #pragma unroll
           for (int v = 0; v < V; ++v) pending |= ((wf >> (8 * v)) & 0xffu) ? (1u << v) : 0u;
+          if constexpr (FINAL) {  // g.st / g.obs still hold what the finishing step produced
+#pragma unroll
+            for (int v = 0; v < V; ++v) {
+              if (pending & (1u << v)) {
+                float* dst = p.final_obs_out + (uint64_t)kk * OD * p.ld + base + v;
+#pragma unroll
+                for (int c = 0; c < OD; ++c) dst[(uint64_t)c * p.ld] = E::OBS_IS_STATE ? g.st[v][c < SD ? c : 0] : g.obs[v][c];
+              }
+            }
+          }
           if constexpr (PREFETCH) {
             // Slots about to be consumed whose state is not there (never drawn in this tile, or consumed since):
             // redraw those slots for the WHOLE warp, so that the divergent pass below only ever picks states up.

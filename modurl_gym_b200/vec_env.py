@@ -191,11 +191,20 @@ class GpuVecEnv:
         _lib.check(self._lib.mgym_step(self._h, _ptr(actions), _ptr(obs_out), _ptr(reward_out), _ptr(flags_out),
                                        _ptr(final_obs_out), self._stream()))
 
-    def rollout(self, K, actions=None, obs=None, reward=None, flags=None, want_obs=True, count_done=True):
+    def rollout(self, K, actions=None, obs=None, reward=None, flags=None, want_obs=True, count_done=True,
+                final_obs=None, want_final_obs=False):
         """K fused steps (the caller's step loop, cartpole.rs:460-471).  actions: [K, N] or None for the
-        device-side uniform random policy.  Returns time-major trajectories."""
+        device-side uniform random policy.  Returns time-major trajectories.
+
+        want_final_obs=True (auto-reset handles): returns (Rollout, final_obs), where final_obs [K, obs_dim, N]
+        (`final_obs`, or a new buffer) holds the observation each episode ended on, before its auto-reset.  Only the
+        entries of envs that finished at that step (flags != 0) are written; the others keep what the buffer held.
+        The next observation of every transition is then
+            next_obs = torch.where((out.flags != 0).unsqueeze(1), final_obs, out.obs)"""
         K = int(K)
         n = self.num_envs
+        if final_obs is not None and not want_final_obs:
+            raise ValueError("final_obs is the buffer of want_final_obs=True")
         if actions is not None:
             self._check_actions(actions, (K,))
         if obs is None and want_obs:
@@ -205,25 +214,39 @@ class GpuVecEnv:
         if flags is None:
             flags = torch.empty((K, n), dtype=torch.uint8, device=self.device)
         dc = torch.zeros(1, dtype=torch.int64, device=self.device) if count_done else None
+        if want_final_obs:
+            if final_obs is None:
+                final_obs = torch.empty((K, self.obs_dim, n), dtype=torch.float32, device=self.device)
+            elif (final_obs.dtype != torch.float32 or final_obs.device != self.device or not final_obs.is_contiguous()
+                  or tuple(final_obs.shape) != (K, self.obs_dim, n)):
+                raise ValueError(f"final_obs must be contiguous float32 on {self.device} with shape "
+                                 f"{(K, self.obs_dim, n)}")
+            _lib.check(self._lib.mgym_rollout_final(self._h, K, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(flags),
+                                                    _ptr(final_obs), _ptr(dc), self._stream()))
+            return Rollout(obs, reward, flags, dc), final_obs
         _lib.check(self._lib.mgym_rollout(self._h, K, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(flags), _ptr(dc),
                                           self._stream()))
         return Rollout(obs, reward, flags, dc)
 
-    def iter_rollout(self, total_steps, chunk=32, actions=None, want_obs=True):
+    def iter_rollout(self, total_steps, chunk=32, actions=None, want_obs=True, want_final_obs=False):
         """A long rollout (e.g. MountainCar's 1000 steps, BASELINE configs[2]) as fused launches of `chunk` steps
         over ONE reused trajectory ring: the full trajectory of 2^24 envs x 1000 steps would be 218 GB.
         Yields (first_step, Rollout) per launch; the Rollout tensors are overwritten by the next launch.
-        actions: None (device policy) or a callable first_step, n_steps -> [n_steps, N] tensor."""
+        actions: None (device policy) or a callable first_step, n_steps -> [n_steps, N] tensor.
+        want_final_obs=True yields (first_step, (Rollout, final_obs)) with one reused [chunk, obs_dim, N] final buffer
+        (see rollout: only entries with flags != 0 are valid)."""
         n, K = self.num_envs, int(chunk)
         obs = torch.empty((K, self.obs_dim, n), dtype=torch.float32, device=self.device) if want_obs else None
         reward = torch.empty((K, n), dtype=torch.float32, device=self.device)
         flags = torch.empty((K, n), dtype=torch.uint8, device=self.device)
+        final = torch.empty((K, self.obs_dim, n), dtype=torch.float32, device=self.device) if want_final_obs else None
         done = 0
         while done < total_steps:
             k = min(K, total_steps - done)
             a = None if actions is None else actions(done, k)
             out = self.rollout(k, a, obs=None if obs is None else obs[:k], reward=reward[:k], flags=flags[:k],
-                               want_obs=want_obs)
+                               want_obs=want_obs, final_obs=None if final is None else final[:k],
+                               want_final_obs=want_final_obs)
             yield done, out
             done += k
 
