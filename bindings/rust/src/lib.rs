@@ -152,6 +152,38 @@ impl GpuVecEnv {
                                     self.stream)
         })
     }
+    /// `step` plus the return and length of every episode that ended in it (auto-reset handles): where
+    /// flags_out[i] != 0, ep_return[i] / ep_length[i] are env i's finished episode; other entries are not written.
+    /// Either buffer may be null; `ep_return_len` / `ep_length_len` are the lengths in elements of the device buffers,
+    /// checked against the N the kernel may write.
+    pub fn step_episodes(&mut self, actions: *const c_void, obs_out: *mut f32, reward_out: *mut f32,
+                         flags_out: *mut u8, ep_return: *mut f32, ep_return_len: usize, ep_length: *mut u32,
+                         ep_length_len: usize) -> Result<VecStepInfo, MgymError> {
+        let n = self.num_envs as usize;
+        assert!(ep_return.is_null() || ep_return_len >= n, "ep_return: N floats");
+        assert!(ep_length.is_null() || ep_length_len >= n, "ep_length: N u32");
+        check(unsafe {
+            sys::mgym_step_episodes(self.h, actions, obs_out, reward_out, flags_out, ptr::null_mut(), ep_return,
+                                    ep_length, self.stream)
+        })?;
+        Ok(VecStepInfo { state: obs_out, reward: reward_out, flags: flags_out })
+    }
+    /// `rollout` plus the return and length of every episode that ended in it (auto-reset handles): where
+    /// flags_traj[k][i] != 0, ep_return_traj[k][i] / ep_length_traj[k][i] are the episode env i finished at step k;
+    /// other entries are not written.  Either buffer may be null; their lengths in elements are checked against the
+    /// K * N the kernel may write.
+    pub fn rollout_episodes(&mut self, k: u32, actions: *const c_void, obs_traj: *mut f32, reward_traj: *mut f32,
+                            flags_traj: *mut u8, ep_return_traj: *mut f32, ep_return_len: usize,
+                            ep_length_traj: *mut u32, ep_length_len: usize, done_count: *mut u64)
+                            -> Result<(), MgymError> {
+        let kn = k as usize * self.num_envs as usize;
+        assert!(ep_return_traj.is_null() || ep_return_len >= kn, "ep_return_traj: K * N floats, time-major");
+        assert!(ep_length_traj.is_null() || ep_length_len >= kn, "ep_length_traj: K * N u32, time-major");
+        check(unsafe {
+            sys::mgym_rollout_episodes(self.h, k, actions, obs_traj, reward_traj, flags_traj, ptr::null_mut(),
+                                       ep_return_traj, ep_length_traj, done_count, self.stream)
+        })
+    }
     /// Host-buffer step for scalar adapters and tests: H2D actions, step, D2H results, synchronises.
     /// Every slice length is checked against what the C side reads or writes (N actions of the kind's own type,
     /// obs_dim * N observations, N rewards, N flags), so this safe function cannot reach out of bounds.

@@ -80,6 +80,13 @@ extern "C" {
     pub fn mgym_rollout_final(env: *mut mgym_env, k: u32, actions: *const c_void, obs_traj: *mut f32,
                               reward_traj: *mut f32, flags_traj: *mut u8, final_obs_traj: *mut f32,
                               done_count_out: *mut u64, stream: *mut c_void) -> c_int;
+    pub fn mgym_step_episodes(env: *mut mgym_env, actions: *const c_void, obs_out: *mut f32, reward_out: *mut f32,
+                              flags_out: *mut u8, final_obs_out: *mut f32, ep_return_out: *mut f32,
+                              ep_length_out: *mut u32, stream: *mut c_void) -> c_int;
+    pub fn mgym_rollout_episodes(env: *mut mgym_env, k: u32, actions: *const c_void, obs_traj: *mut f32,
+                                 reward_traj: *mut f32, flags_traj: *mut u8, final_obs_traj: *mut f32,
+                                 ep_return_traj: *mut f32, ep_length_traj: *mut u32, done_count_out: *mut u64,
+                                 stream: *mut c_void) -> c_int;
     pub fn mgym_sample_actions(env: *mut mgym_env, actions_out: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn mgym_step_host(env: *mut mgym_env, actions_host: *const c_void, obs_host: *mut f32,
                           reward_host: *mut f32, flags_host: *mut u8, stream: *mut c_void) -> c_int;

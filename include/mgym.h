@@ -38,7 +38,8 @@
  *                   same call; obs_out holds the post-reset observation, reward/flags the
  *                   finishing step's values, final_obs_out (optional) the pre-reset obs.
  *                   mgym_rollout_final keeps the same pre-reset obs for a fused rollout, stored only
- *                   where an env finished.
+ *                   where an env finished; mgym_step_episodes / mgym_rollout_episodes store the
+ *                   return and length of each episode that ends, the same way.
  *   Reset states come from a counter-based Philox4x32-10 stream keyed by the seed; the counter is
  *   (global env index, reset call index) for mgym_reset and (global env index, step index at which
  *   the episode that just finished BEGAN) for a same-step auto-reset, so results do not depend on
@@ -220,6 +221,32 @@ int mgym_rollout(mgym_env *env, uint32_t K, const void *actions, float *obs_traj
  * (device_clock handles). */
 int mgym_rollout_final(mgym_env *env, uint32_t K, const void *actions, float *obs_traj, float *reward_traj,
                        uint8_t *flags_traj, float *final_obs_traj, unsigned long long *done_count_out, void *stream);
+/* Per-episode returns and lengths (Gymnasium's RecordEpisodeStatistics: info["episode"]["r"], ["l"]).
+ * mgym_step_episodes is mgym_step, mgym_rollout_episodes is mgym_rollout_final, each plus two device outputs aligned
+ * with the flags: ep_return_out float[N] / ep_length_out uint32[N] for the step, ep_return_traj float[K][N] /
+ * ep_length_traj uint32[K][N] (time-major like reward_traj) for the rollout.  Where flags[i] != 0 (flags[k][i] != 0),
+ * entry i ([k][i]) holds the episode that env just finished; every other entry is NOT written: it keeps what the
+ * caller put there (SPARSE, for the step too, unlike its dense final_obs_out).
+ *   ep_length = the step count the finishing step reached: the value the statistics add to length_sum for that
+ *               episode (counts injected by mgym_set_state included; CartPole reports 500 on truncation).
+ *   ep_return = the value the statistics add to return_sum for that episode, as f32: CartPole the length
+ *               (sutton_barto_reward: +1 if truncated, -1 if terminated), MountainCar-v0 -length, Acrobot
+ *               (terminated ? 1 : 0) - length (exact below 2^24 steps), MountainCarContinuous and Pendulum the handle's
+ *               f32 running return as the finishing step leaves it.
+ * Either output may be NULL; with both NULL the calls are mgym_step and mgym_rollout_final (which with
+ * final_obs_traj == NULL is mgym_rollout).  Everything else (the other outputs, done count, state, counters, running
+ * returns, statistics, parameter rows and redraws, step index) is bit-identical to those calls with the same arguments.
+ * Results do not depend on sharding or launch geometry.  Needs 4-byte alignment only; neither output needs
+ * track_stats.  MGYM_ERR_BAD_ARGUMENT, before anything is written: an episode output on an auto_reset = 0 handle;
+ * ep_return for MountainCarContinuous or Pendulum on a handle without running returns (track_returns = 0 or
+ * track_stats = 0; ep_length alone is fine); ep_return == ep_length; final_obs_traj == obs_traj.  validate_actions = 1
+ * rejects a bad batch before anything is written.  Capturable under the same rules as mgym_step / mgym_rollout
+ * (device_clock handles). */
+int mgym_step_episodes(mgym_env *env, const void *actions, float *obs_out, float *reward_out, uint8_t *flags_out,
+                       float *final_obs_out, float *ep_return_out, uint32_t *ep_length_out, void *stream);
+int mgym_rollout_episodes(mgym_env *env, uint32_t K, const void *actions, float *obs_traj, float *reward_traj,
+                          uint8_t *flags_traj, float *final_obs_traj, float *ep_return_traj, uint32_t *ep_length_traj,
+                          unsigned long long *done_count_out, void *stream);
 /* Space::sample for all envs at the current step index (same stream mgym_rollout uses). */
 int mgym_sample_actions(mgym_env *env, void *actions_out, void *stream);
 

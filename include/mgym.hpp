@@ -144,6 +144,15 @@ class GpuVecEnv {
     check(mgym_step(h_, actions_device, alias ? nullptr : obs_, reward_, flags_, nullptr, stream_));
     return StepInfo{alias ? mgym_state_ptr(h_) : obs_, reward_, flags_};
   }
+  // step plus the return and length of every episode that ended in it (RecordEpisodeStatistics): ep_return [N] and
+  // ep_length [N] (device, either may be null) are written only where StepInfo.flags != 0 (mgym_step_episodes);
+  // auto-reset handles only
+  StepInfo step_episodes(const void* actions_device, float* ep_return_device, uint32_t* ep_length_device) {
+    const bool alias = obs_is_state();
+    check(mgym_step_episodes(h_, actions_device, alias ? nullptr : obs_, reward_, flags_, nullptr, ep_return_device,
+                             ep_length_device, stream_));
+    return StepInfo{alias ? mgym_state_ptr(h_) : obs_, reward_, flags_};
+  }
   BoxSpace observation_space() const {  // cartpole.rs:350-352
     BoxSpace b{std::vector<float>(obs_dim()), std::vector<float>(obs_dim())};
     check(mgym_space_observation(kind_, b.low.data(), b.high.data()));
@@ -167,6 +176,15 @@ class GpuVecEnv {
                      float* final_obs_traj, unsigned long long* done_count_device = nullptr) {
     check(mgym_rollout_final(h_, K, actions_device, obs_traj, reward_traj, flags_traj, final_obs_traj,
                              done_count_device, stream_));
+  }
+  // rollout plus the return and length of every episode that ended in it: ep_return_traj [K][N], ep_length_traj
+  // [K][N] (device, either may be null) and final_obs_traj (optional) are written only where flags_traj != 0
+  // (mgym_rollout_episodes); auto-reset handles only
+  void rollout_episodes(uint32_t K, const void* actions_device, float* obs_traj, float* reward_traj,
+                        uint8_t* flags_traj, float* final_obs_traj, float* ep_return_traj, uint32_t* ep_length_traj,
+                        unsigned long long* done_count_device = nullptr) {
+    check(mgym_rollout_episodes(h_, K, actions_device, obs_traj, reward_traj, flags_traj, final_obs_traj,
+                                ep_return_traj, ep_length_traj, done_count_device, stream_));
   }
   void sample_actions(void* actions_device) { check(mgym_sample_actions(h_, actions_device, stream_)); }
 

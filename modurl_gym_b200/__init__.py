@@ -6,7 +6,7 @@ from .spaces import BoxSpace, Discrete  # noqa: F401
 
 def __getattr__(name):
     # GpuVecEnv needs torch; keep `import modurl_gym_b200` light for symbol/ABI checks.
-    if name in ("GpuVecEnv", "StepInfo", "Rollout", "EpisodeStats", "KINDS", "CARTPOLE", "MOUNTAIN_CAR",
+    if name in ("GpuVecEnv", "StepInfo", "Rollout", "EpisodeStats", "Episodes", "KINDS", "CARTPOLE", "MOUNTAIN_CAR",
                 "MOUNTAIN_CAR_CONTINUOUS", "PENDULUM", "ACROBOT", "FLAG_TERMINATED", "FLAG_TRUNCATED"):
         from . import vec_env
 

@@ -117,6 +117,8 @@ constexpr int kStateDim[MGYM_NUM_KINDS] = {4, 2, 2, 2, 4};
 constexpr int kObsDim[MGYM_NUM_KINDS] = {4, 2, 2, 3, 6};
 constexpr int kContinuous[MGYM_NUM_KINDS] = {0, 0, 1, 1, 0};
 constexpr int kNumActions[MGYM_NUM_KINDS] = {2, 3, 0, 0, 3};
+// rewards are constants, so a return follows from the episode's length and outcome (Env::ANALYTIC_RETURN)
+constexpr int kAnalyticReturn[MGYM_NUM_KINDS] = {1, 1, 0, 0, 1};
 const char* const kNames[MGYM_NUM_KINDS] = {"CartPole-v1", "MountainCar-v0", "MountainCarContinuous-v0",
                                             "Pendulum-v1", "Acrobot-v1"};
 
@@ -262,12 +264,12 @@ int launch_persistent(void (*kernel)(KP), const mgym_env* e, const KP& p, uint64
 }
 
 // TMA-staged step kernel (auto-reset, vector path, N a multiple of the 128-env warp tile)
-template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false>
-int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cudaStream_t st) {
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false>
+int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW, EPISODES>& p_in, cudaStream_t st) {
   mgym_env* e = const_cast<mgym_env*>(ce);  // ticket accounting
-  KParams<PARAMS, REDRAW> p = p_in;
+  KParams<PARAMS, REDRAW, EPISODES> p = p_in;
   using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
-  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS, REDRAW>;
+  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS, REDRAW, EPISODES>;
   constexpr int threads = TMA_THREADS;
   // the opt-in to > 48 KB of dynamic shared memory and the occupancy are per device
   static int cached_per_sm[kMaxDevices] = {};
@@ -313,38 +315,41 @@ int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW>& p_in, cud
 
 // kind x vector width x auto/manual x counter representation (x per-env parameters (x per-episode redraw: auto-reset
 // handles only, the host never asks for a manual form of it)) (x final observations: auto-reset rollouts only,
-// mgym_rollout_final refuses manual handles before it gets here)
-template <int KIND, int V, bool ROLLOUT, bool PARAMS = false, bool REDRAW = false, bool FINAL = false>
-int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStream_t st) {
+// mgym_rollout_final refuses manual handles before it gets here) (x episode outputs: auto-reset steps and rollouts,
+// mgym_step_episodes / mgym_rollout_episodes refuse manual handles)
+template <int KIND, int V, bool ROLLOUT, bool PARAMS = false, bool REDRAW = false, bool FINAL = false,
+          bool EPISODES = false>
+int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW, EPISODES>& p, cudaStream_t st) {
   static_assert(!FINAL || ROLLOUT, "final observations are a rollout form");
+  static_assert(!(FINAL && EPISODES), "the EPISODES rollout forms store final observations themselves");
   const uint64_t groups = p.n / V;
   const bool autor = e->cfg.auto_reset != 0;
   if constexpr (!ROLLOUT && V == 4) {
     // manual mode (the reference's protocol): counters are 32-bit, CartPole adds steps_beyond_terminated
-    if constexpr (!REDRAW) {
+    if constexpr (!REDRAW && !EPISODES) {
       if (!autor && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
     }
     if (autor && p.n % TMA_TILE == 0) {
       if constexpr (KIND == 0) {  // CartPole's handles are all CNT_S16 (500-step truncation, cartpole.rs:297)
-        return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW>(e, p, st);
+        return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW, EPISODES>(e, p, st);
       } else {
         switch (e->cnt_mode) {
-          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW>(e, p, st);
-          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS, REDRAW>(e, p, st);
-          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS, REDRAW>(e, p, st);
+          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW, EPISODES>(e, p, st);
+          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS, REDRAW, EPISODES>(e, p, st);
+          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS, REDRAW, EPISODES>(e, p, st);
         }
       }
     }
     if (p.n > TMA_TILE) {
       // ragged size: whole 1024-env tiles on the TMA kernel, the remaining (< 1024) envs on the vector kernel
-      KParams<PARAMS, REDRAW> head = p, tail = p;
+      KParams<PARAMS, REDRAW, EPISODES> head = p, tail = p;
       head.adv_dt = 0;  // device clock: the tail launch (last of the call) moves the step index on
       head.n = p.n - p.n % TMA_TILE;
       tail.first = p.first + head.n;
       tail.n = p.n - head.n;
-      int rc = dispatch_mode<KIND, 4, false, PARAMS, REDRAW>(e, head, st);
+      int rc = dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES>(e, head, st);
       if (rc != MGYM_OK) return rc;
-      return dispatch_mode<KIND, 4, false, PARAMS, REDRAW>(e, tail, st);
+      return dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES>(e, tail, st);
     }
   }
   // rollout_kernel's FULL form: complete warp tiles and all three trajectory outputs
@@ -355,14 +360,16 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW>& p, cudaStrea
     if constexpr (ROLLOUT) {                                                                             \
       if constexpr (AUTO_ && V == 4) {                                                                   \
         if (full)                                                                                        \
-          return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS, REDRAW, FINAL>, e, p, groups, st); \
+          return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, true, PARAMS, REDRAW, FINAL, EPISODES>, e, p, \
+                                   groups, st);                                                          \
       }                                                                                                  \
-      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS, REDRAW, FINAL>, e, p, groups, st); \
+      return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS, REDRAW, FINAL, EPISODES>, e, p, \
+                               groups, st);                                                              \
     } else {                                                                                             \
-      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS, REDRAW>, e, p, groups, st);     \
+      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS, REDRAW, EPISODES>, e, p, groups, st); \
     }                                                                                                    \
   } while (0)
-  if constexpr (!REDRAW && !FINAL) {
+  if constexpr (!REDRAW && !FINAL && !EPISODES) {
     if (!autor) MGYM_LAUNCH(false, CNT_U32);
   }
   if constexpr (KIND == 0) {
@@ -388,8 +395,18 @@ ParamBox redraw_box(const mgym_env* e) {
 
 // A handle with per-env parameters runs the PARAMS instantiations (kinds that have parameters only), an auto-reset
 // one with redraw ranges the PARAMS + REDRAW instantiations (manual-mode steps never reset).
-template <int KIND, bool ROLLOUT, bool FINAL>
-int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
+template <int KIND, bool ROLLOUT, bool FINAL, bool EPISODES, bool PARAMS, bool REDRAW>
+int dispatch_width(const mgym_env* e, const KParamsBase<PARAMS, REDRAW>& pb, const EpisodeOut& ep, bool vec4,
+                   cudaStream_t st) {
+  KParams<PARAMS, REDRAW, EPISODES> p;
+  static_cast<KParamsBase<PARAMS, REDRAW>&>(p) = pb;
+  if constexpr (EPISODES) p.ep = ep;
+  return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, PARAMS, REDRAW, FINAL, EPISODES>(e, p, st)
+              : dispatch_mode<KIND, 1, ROLLOUT, PARAMS, REDRAW, FINAL, EPISODES>(e, p, st);
+}
+
+template <int KIND, bool ROLLOUT, bool FINAL, bool EPISODES>
+int dispatch_kind(const mgym_env* e, const KernelParams& p, const EpisodeOut& ep, bool vec4, cudaStream_t st) {
   if constexpr (Env<KIND>::NP > 0) {
     if (e->params) {
       KernelParamsP pp;
@@ -399,23 +416,23 @@ int dispatch_kind(const mgym_env* e, const KernelParams& p, bool vec4, cudaStrea
         KernelParamsR pr;
         static_cast<KernelParamsP&>(pr) = pp;
         pr.redraw = redraw_box(e);
-        return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true, true, FINAL>(e, pr, st)
-                    : dispatch_mode<KIND, 1, ROLLOUT, true, true, FINAL>(e, pr, st);
+        return dispatch_width<KIND, ROLLOUT, FINAL, EPISODES, true, true>(e, pr, ep, vec4, st);
       }
-      return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, true, false, FINAL>(e, pp, st)
-                  : dispatch_mode<KIND, 1, ROLLOUT, true, false, FINAL>(e, pp, st);
+      return dispatch_width<KIND, ROLLOUT, FINAL, EPISODES, true, false>(e, pp, ep, vec4, st);
     }
   }
-  return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, false, false, FINAL>(e, p, st)
-              : dispatch_mode<KIND, 1, ROLLOUT, false, false, FINAL>(e, p, st);
+  return dispatch_width<KIND, ROLLOUT, FINAL, EPISODES, false, false>(e, p, ep, vec4, st);
 }
 
-// FINAL: the rollout forms that also store final observations (mgym_rollout_final)
-template <bool ROLLOUT, bool FINAL = false>
-int dispatch(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st) {
+// FINAL: the rollout forms that also store final observations (mgym_rollout_final).  EPISODES: the step and rollout
+// forms that also store episode returns and lengths to `ep` (mgym_step_episodes, mgym_rollout_episodes); their
+// rollouts store final observations where p.final_obs_out is not null.
+template <bool ROLLOUT, bool FINAL = false, bool EPISODES = false>
+int dispatch(const mgym_env* e, const KernelParams& p, bool vec4, cudaStream_t st,
+             const EpisodeOut& ep = EpisodeOut{nullptr, nullptr}) {
 #define MGYM_KIND(K_)                                               \
   case K_:                                                          \
-    return dispatch_kind<K_, ROLLOUT, FINAL>(e, p, vec4, st)
+    return dispatch_kind<K_, ROLLOUT, FINAL, EPISODES>(e, p, ep, vec4, st)
   switch (e->kind) {
     MGYM_KIND(0);
     MGYM_KIND(1);
@@ -700,8 +717,7 @@ int mgym_create(int kind, uint64_t num_envs, int device_ordinal, uint64_t seed, 
       fill_u32_kernel<<<(unsigned)((n + 255) / 256), 256>>>(e->sbt, 1u, n);  // cartpole.rs:81 Some(0)
       MGYM_CUDA(cudaGetLastError());
     }
-    const bool analytic = kind == MGYM_CARTPOLE_V1 || kind == MGYM_MOUNTAIN_CAR_V0 || kind == MGYM_ACROBOT_V1;
-    if (cfg.auto_reset && cfg.track_stats && cfg.track_returns && !analytic) {
+    if (cfg.auto_reset && cfg.track_stats && cfg.track_returns && !kAnalyticReturn[kind]) {
       MGYM_CUDA(cudaMalloc(&e->ep_return, sizeof(float) * n));
       MGYM_CUDA(cudaMemset(e->ep_return, 0, sizeof(float) * n));
     }
@@ -1052,13 +1068,31 @@ int mgym_checkpoint_load(mgym_env* e, const void* blob, size_t blob_bytes, void*
 // ---------------------------------------------------------------------------------------------
 // hot path
 // ---------------------------------------------------------------------------------------------
-int mgym_step(mgym_env* e, const void* actions, float* obs_out, float* reward_out, uint8_t* flags_out,
-              float* final_obs_out, void* stream) {
-  if (!e || !actions) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_step: NULL argument");
+// The checks of the episode outputs shared by mgym_step_episodes and mgym_rollout_episodes (e is not null)
+static int check_episode_outputs(const char* fn, const mgym_env* e, const float* ep_return, const uint32_t* ep_length) {
+  if (!ep_return && !ep_length) return MGYM_OK;
+  if (!e->cfg.auto_reset)
+    return fail(MGYM_ERR_BAD_ARGUMENT, "%s: a manual-mode handle ends no episode itself and keeps no statistics; "
+                "ep_return and ep_length need auto_reset = 1", fn);
+  if (ep_return && !kAnalyticReturn[e->kind] && !e->ep_return)
+    return fail(MGYM_ERR_BAD_ARGUMENT, "%s: %s keeps no running return on this handle; ep_return needs a handle "
+                "created with track_returns = 1 and track_stats = 1 (ep_length alone does not)", fn, kNames[e->kind]);
+  if (ep_return && (const void*)ep_return == (const void*)ep_length)
+    return fail(MGYM_ERR_BAD_ARGUMENT, "%s: ep_return and ep_length must be different buffers", fn);
+  return MGYM_OK;
+}
+
+// mgym_step and mgym_step_episodes: a non-null episode output selects the EPISODES kernel forms, none launches exactly
+// what mgym_step launches
+static int run_step(const char* fn, mgym_env* e, const void* actions, float* obs_out, float* reward_out,
+                    uint8_t* flags_out, float* final_obs_out, float* ep_return_out, uint32_t* ep_length_out,
+                    void* stream) {
+  if (!e || !actions) return fail(MGYM_ERR_BAD_ARGUMENT, "%s: NULL argument", fn);
+  if (int rc = check_episode_outputs(fn, e, ep_return_out, ep_length_out)) return rc;
   e->work_slot = 0;
   DeviceGuard guard(e->device);
   cudaStream_t st = (cudaStream_t)stream;
-  if (int rc = refuse_capture(e, st, "mgym_step", true)) return rc;
+  if (int rc = refuse_capture(e, st, fn, true)) return rc;
   if (int rc = validate_device_actions(e, actions, e->n, st)) return rc;
   e->call_tickets = 0;
   KernelParams p = base_params(e);
@@ -1072,16 +1106,34 @@ int mgym_step(mgym_env* e, const void* actions, float* obs_out, float* reward_ou
   p.adv_dt = 1;
   const bool vec4 = e->vec4 && aligned16(actions) && aligned16(obs_out) && aligned16(reward_out) &&
                     aligned16(flags_out) && aligned16(final_obs_out);
-  int rc = dispatch<false>(e, p, vec4, st);
+  int rc;
+  if (ep_return_out || ep_length_out)  // stored one scalar at a time: float alignment suffices
+    rc = dispatch<false, false, true>(e, p, vec4, st, EpisodeOut{ep_return_out, ep_length_out});
+  else
+    rc = dispatch<false>(e, p, vec4, st);
   if (rc != MGYM_OK) return rc;
   return advance_clock(e, 1, st, /*fused=*/true);
 }
 
-// mgym_rollout and mgym_rollout_final: a non-null final_obs_traj selects the FINAL kernel forms, null launches exactly
-// what mgym_rollout launches
+int mgym_step(mgym_env* e, const void* actions, float* obs_out, float* reward_out, uint8_t* flags_out,
+              float* final_obs_out, void* stream) {
+  return run_step("mgym_step", e, actions, obs_out, reward_out, flags_out, final_obs_out, nullptr, nullptr, stream);
+}
+
+int mgym_step_episodes(mgym_env* e, const void* actions, float* obs_out, float* reward_out, uint8_t* flags_out,
+                       float* final_obs_out, float* ep_return_out, uint32_t* ep_length_out, void* stream) {
+  return run_step("mgym_step_episodes", e, actions, obs_out, reward_out, flags_out, final_obs_out, ep_return_out,
+                  ep_length_out, stream);
+}
+
+// mgym_rollout, mgym_rollout_final and mgym_rollout_episodes: a non-null episode output selects the EPISODES kernel
+// forms (which store final observations where final_obs_traj is not null), else a non-null final_obs_traj the FINAL
+// forms; neither launches exactly what mgym_rollout launches
 static int run_rollout(const char* fn, mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
-                       uint8_t* flags_traj, float* final_obs_traj, unsigned long long* done_count_out, void* stream) {
+                       uint8_t* flags_traj, float* final_obs_traj, float* ep_return_traj, uint32_t* ep_length_traj,
+                       unsigned long long* done_count_out, void* stream) {
   if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "%s: env is NULL", fn);
+  if (int rc = check_episode_outputs(fn, e, ep_return_traj, ep_length_traj)) return rc;
   if (final_obs_traj) {
     if (!e->cfg.auto_reset)
       return fail(MGYM_ERR_BAD_ARGUMENT, "%s: a manual-mode handle resets nothing inside the rollout; obs_traj "
@@ -1112,8 +1164,10 @@ static int run_rollout(const char* fn, mgym_env* e, uint32_t K, const void* acti
   p.work_base = 0;
   MGYM_CUDA(cudaMemsetAsync(e->work + 3, 0, sizeof(unsigned long long), st));
   int rc;
-  if (final_obs_traj) {
-    p.final_obs_out = final_obs_traj;  // float alignment suffices: stored one scalar at a time
+  p.final_obs_out = final_obs_traj;  // float alignment suffices: the sparse outputs are stored one scalar at a time
+  if (ep_return_traj || ep_length_traj) {
+    rc = dispatch<true, false, true>(e, p, vec4, st, EpisodeOut{ep_return_traj, ep_length_traj});
+  } else if (final_obs_traj) {
     rc = dispatch<true, true>(e, p, vec4, st);
   } else {
     rc = dispatch<true>(e, p, vec4, st);
@@ -1124,13 +1178,21 @@ static int run_rollout(const char* fn, mgym_env* e, uint32_t K, const void* acti
 
 int mgym_rollout(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
                  uint8_t* flags_traj, unsigned long long* done_count_out, void* stream) {
-  return run_rollout("mgym_rollout", e, K, actions, obs_traj, reward_traj, flags_traj, nullptr, done_count_out, stream);
+  return run_rollout("mgym_rollout", e, K, actions, obs_traj, reward_traj, flags_traj, nullptr, nullptr, nullptr,
+                     done_count_out, stream);
 }
 
 int mgym_rollout_final(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
                        uint8_t* flags_traj, float* final_obs_traj, unsigned long long* done_count_out, void* stream) {
-  return run_rollout("mgym_rollout_final", e, K, actions, obs_traj, reward_traj, flags_traj, final_obs_traj,
-                 done_count_out, stream);
+  return run_rollout("mgym_rollout_final", e, K, actions, obs_traj, reward_traj, flags_traj, final_obs_traj, nullptr,
+                     nullptr, done_count_out, stream);
+}
+
+int mgym_rollout_episodes(mgym_env* e, uint32_t K, const void* actions, float* obs_traj, float* reward_traj,
+                          uint8_t* flags_traj, float* final_obs_traj, float* ep_return_traj, uint32_t* ep_length_traj,
+                          unsigned long long* done_count_out, void* stream) {
+  return run_rollout("mgym_rollout_episodes", e, K, actions, obs_traj, reward_traj, flags_traj, final_obs_traj,
+                     ep_return_traj, ep_length_traj, done_count_out, stream);
 }
 
 int mgym_sample_actions(mgym_env* e, void* actions_out, void* stream) {

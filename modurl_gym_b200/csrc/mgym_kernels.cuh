@@ -66,7 +66,7 @@ struct KernelParams {
   float* obs_out;       // step: [OD][n]; rollout: [K][OD][n]
   float* reward_out;    // step: [n];     rollout: [K][n]
   uint8_t* flags_out;   // step: [n];     rollout: [K][n]
-  float* final_obs_out; // step: pre-reset observation [OD][n]; rollout (FINAL forms): [K][OD][n], finished envs only
+  float* final_obs_out; // step: pre-reset obs [OD][n]; rollout (FINAL, EPISODES forms): [K][OD][n], finished envs only
   // reset source
   const float* reset_pool;  // [SD][pool_len] or null
   uint64_t pool_len;
@@ -109,8 +109,23 @@ struct ParamBox {  // U[lo, lo + range) per parameter, in f64 like the reset dra
 struct KernelParamsR : KernelParamsP {
   ParamBox redraw;
 };
+// Per-episode outputs (mgym_step_episodes, mgym_rollout_episodes): the return and length of every episode that
+// ends, at the index of its flags entry (step: [n]; rollout: [K][n]); entries of envs that did not finish are not
+// written.  Either pointer may be null.
+struct EpisodeOut {
+  float* ret;
+  uint32_t* len;
+};
+// The launch parameters of the kernels instantiated with EPISODES: the two outputs on top of any of the above, so
+// that the types the other kernels take keep their layout.
+template <typename Base>
+struct KernelParamsE : Base {
+  EpisodeOut ep;
+};
 template <bool PARAMS, bool REDRAW = false>
-using KParams = std::conditional_t<REDRAW, KernelParamsR, std::conditional_t<PARAMS, KernelParamsP, KernelParams>>;
+using KParamsBase = std::conditional_t<REDRAW, KernelParamsR, std::conditional_t<PARAMS, KernelParamsP, KernelParams>>;
+template <bool PARAMS, bool REDRAW = false, bool EPISODES = false>
+using KParams = std::conditional_t<EPISODES, KernelParamsE<KParamsBase<PARAMS, REDRAW>>, KParamsBase<PARAMS, REDRAW>>;
 
 // The parameters of global env g for the episode whose reset state has counter (g, t): word c % 4 of the Philox
 // block (g, t) with tag tag0 + c / 4, mapped to U[lo, lo + range) as mgym_sample_params maps them.  Parameter c is
@@ -250,6 +265,33 @@ __device__ __forceinline__ double analytic_return_sum(const EnvConsts& k, double
   } else {
     return 0.0 * episodes;
   }
+}
+
+// The return of one finished episode as the statistics add it to return_sum: the per-episode form of
+// analytic_return_sum for kinds whose rewards are constants, the running return otherwise.  The integer is exact and
+// rounded to f32 once, as analytic_return_sum's f64 value would be (exact below 2^24 steps), without f64 registers
+// in the rollout's reset pass.
+template <int KIND>
+__device__ __forceinline__ float episode_return(const EnvConsts& k, uint32_t flags, uint32_t length, float ret) {
+  const int64_t term = flags & FLAG_TERMINATED, trunc = flags >> 1;
+  if constexpr (KIND == 0) {
+    return k.sutton_barto ? (float)(trunc - term) : (float)length;
+  } else if constexpr (KIND == 1) {
+    return -(float)length;
+  } else if constexpr (KIND == 4) {
+    return (float)(term - (int64_t)length);
+  } else {
+    static_assert(!Env<KIND>::ANALYTIC_RETURN, "a kind with constant rewards needs its per-episode form here");
+    return ret;
+  }
+}
+
+// Stores the return and length of the episode that env slot `i` of an output just finished (flags != 0).
+template <int KIND>
+__device__ __forceinline__ void store_episode(const EpisodeOut& ep, const EnvConsts& k, uint64_t i, uint32_t flags,
+                                              uint32_t length, float ret) {
+  if (ep.ret) ep.ret[i] = episode_return<KIND>(k, flags, length, ret);
+  if (ep.len) ep.len[i] = length;
 }
 
 template <int KIND>
@@ -461,11 +503,15 @@ __device__ __noinline__ LaneIO<KIND, V> dynamics_reference_lane(LaneIO<KIND, V> 
 // PR (ParamRows with NP > 0): every env steps with its own constants, prm.r[.][v] (Env::dynamics_p).
 // REDRAW (RESET_IN_PLACE, p is a KernelParamsR): the reset also redraws the finished envs' parameter rows in global
 // memory (the step itself ran on the old ones, in prm).
+// EPISODES (RESET_IN_PLACE, p is the KernelParamsE of the PR / REDRAW form): the tally also stores each finished env's
+// episode return and length.
 template <int KIND, int V, bool AUTO, bool WANT_FINAL, bool TALLY_LEN = true, int RESET = RESET_IN_PLACE,
-          bool TRUSTED = false, bool OBS_VALID = false, typename PR = NoParams, bool REDRAW = false>
+          bool TRUSTED = false, bool OBS_VALID = false, typename PR = NoParams, bool REDRAW = false,
+          bool EPISODES = false>
 __device__ __forceinline__ void step_group(const KernelParams& p, bool count, uint64_t base, uint64_t t,
                                            const typename Env<KIND>::act_t (&action)[V], bool track_ret,
                                            Group<KIND, V>& g, StatAcc& acc, const PR& prm = PR{}) {
+  static_assert(!EPISODES || (AUTO && RESET == RESET_IN_PLACE), "episodes are stored by the in-place tally");
   using E = Env<KIND>;
   float aux[V];
 #pragma unroll
@@ -596,6 +642,10 @@ __device__ __forceinline__ void step_group(const KernelParams& p, bool count, ui
       if constexpr (!E::ANALYTIC_RETURN) {
         if (tally) acc.return_sum += (double)g.ret[v];
       }
+      if constexpr (EPISODES) {
+        using KPE = KernelParamsE<KParamsBase<(PR::NP > 0), REDRAW>>;
+        if (done) store_episode<KIND>(static_cast<const KPE&>(p).ep, p.k, base + v, g.flags[v], g.steps[v], g.ret[v]);
+      }
     }
   }
   if constexpr (AUTO && RESET == RESET_IN_PLACE && REDRAW) {
@@ -631,14 +681,17 @@ __device__ __forceinline__ typename CounterType<CNT>::type cnt_encode(uint32_t s
 // Mode 1: per-call step kernel
 // =============================================================================================
 // REDRAW: every reset also redraws the env's parameter rows (mgym_set_param_redraw; auto-reset with rows only).
-template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false, bool REDRAW = false>
-__global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
+// EPISODES (mgym_step_episodes, auto-reset only): step_group's tally also stores each finished env's episode return
+// and length.
+template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false>
+__global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KParams<PARAMS, REDRAW, EPISODES> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
   using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   constexpr int SD = E::SD, OD = E::OD;
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
+  static_assert(!EPISODES || AUTO, "episodes end only where the step resets");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   StatAcc acc;
   const uint64_t groups = p.n / V;
@@ -682,11 +735,12 @@ __global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KP
       }
     }
     if (want_final)
-      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, PR, REDRAW>(p, true, base, t_now, action, track_ret,
-                                                                                     g, acc, prm);
+      step_group<KIND, V, AUTO, true, true, RESET_IN_PLACE, false, false, PR, REDRAW, EPISODES>(p, true, base, t_now, action,
+                                                                                               track_ret, g, acc, prm);
     else
-      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, PR, REDRAW>(p, true, base, t_now, action, track_ret,
-                                                                                      g, acc, prm);
+      step_group<KIND, V, AUTO, false, true, RESET_IN_PLACE, false, false, PR, REDRAW, EPISODES>(p, true, base, t_now,
+                                                                                                action, track_ret, g, acc,
+                                                                                                prm);
 
     {
       Vec<float, V> s[SD];
@@ -856,9 +910,12 @@ struct TmaLayout {
 // Philox block, two for CartPole) and writes them into the rows in global memory.  The consumers stepped that tile
 // with the staged (old) rows; no other tile of the launch holds the env, and the next launch's producer reads the
 // rows only after griddepcontrol.wait.  Stage layout and stage count are those of the PARAMS form.
-template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false>
+//
+// EPISODES (mgym_step_episodes, auto-reset only): the consumers' branch for finished envs also stores each one's
+// episode return and length, where the statistics read them (after the lazy stamp decode, before they are cleared).
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false>
 __global__ void __launch_bounds__(TMA_THREADS, 2)
-    step_kernel_tma(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
+    step_kernel_tma(const __grid_constant__ KParams<PARAMS, REDRAW, EPISODES> p) {
   using E = Env<KIND>;
   using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
   using act_t = typename E::act_t;
@@ -868,6 +925,7 @@ __global__ void __launch_bounds__(TMA_THREADS, 2)
   using PR = ParamRows<PARAMS ? E::NP : 0, V>;
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(AUTO || !cnt_is_stamp(CNT), "manual mode keeps the reference's own counters");
+  static_assert(!EPISODES || AUTO, "episodes end only where the step resets");
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (tma::smem_u32(smem_raw) + 127u) & ~127u;
   const uint32_t warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);  // warp-uniform for the compiler
@@ -1077,6 +1135,7 @@ __global__ void __launch_bounds__(TMA_THREADS, 2)
 #pragma unroll
         for (int v = 0; v < V; ++v) {
           if ((fin >> (8 * v)) & 0xffu) {
+            if constexpr (EPISODES) store_episode<KIND>(p.ep, p.k, base + v, g.flags[v], g.steps[v], g.ret[v]);
             items[pos] = (uint16_t)(tid * V + v);
             lengths[pos++] = g.steps[v];
             g.steps[v] = 0u;
@@ -1178,9 +1237,13 @@ constexpr int rollout_min_blocks() {
 // FINAL (mgym_rollout_final, auto-reset forms only): the divergent reset pass also stores the observation each
 // finished env ended on, before the reset overwrites it, to p.final_obs_out [K][OD][ld].  Only finished envs are
 // written; the address is computed there from (kk, base), so the hot loop carries no extra pointer.
-template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false, bool REDRAW = false, bool FINAL = false>
+// EPISODES (mgym_rollout_episodes, auto-reset forms only): the same pass also stores each finished env's episode return
+// and length to p.ep [K][ld], and its final observation where p.final_obs_out is not null, so one set of forms serves
+// the calls with and without final observations.
+template <int KIND, int V, bool AUTO, int CNT, bool FULL, bool PARAMS = false, bool REDRAW = false, bool FINAL = false,
+          bool EPISODES = false>
 __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
-    rollout_kernel(const __grid_constant__ KParams<PARAMS, REDRAW> p) {
+    rollout_kernel(const __grid_constant__ KParams<PARAMS, REDRAW, EPISODES> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
   using cnt_t = typename CounterType<CNT>::type;
@@ -1189,6 +1252,7 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!FULL || (AUTO && V == 4), "the FULL form is built for the vector auto-reset path only");
   static_assert(!FINAL || AUTO, "final observations exist only where the rollout resets");
+  static_assert(!EPISODES || (AUTO && !FINAL), "the EPISODES forms test for final observations at run time");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
   constexpr int ACT_RING = PARAMS ? 4 : 8;  // steps of action look-ahead staged in shared memory
   __shared__ float par_slots[PARAMS ? E::NP * V : 1][PARAMS ? 256 : 1];  // [c * V + v][thread]
@@ -1411,13 +1475,18 @@ __global__ void __launch_bounds__(256, rollout_min_blocks<KIND>())
           uint32_t pending = 0;
 #pragma unroll
           for (int v = 0; v < V; ++v) pending |= ((wf >> (8 * v)) & 0xffu) ? (1u << v) : 0u;
-          if constexpr (FINAL) {  // g.st / g.obs still hold what the finishing step produced
+          if constexpr (FINAL || EPISODES) {  // g.st / g.obs / g.steps / g.ret still hold what the finishing step left
 #pragma unroll
             for (int v = 0; v < V; ++v) {
               if (pending & (1u << v)) {
-                float* dst = p.final_obs_out + (uint64_t)kk * OD * p.ld + base + v;
+                if (FINAL || p.final_obs_out) {
+                  float* dst = p.final_obs_out + (uint64_t)kk * OD * p.ld + base + v;
 #pragma unroll
-                for (int c = 0; c < OD; ++c) dst[(uint64_t)c * p.ld] = E::OBS_IS_STATE ? g.st[v][c < SD ? c : 0] : g.obs[v][c];
+                  for (int c = 0; c < OD; ++c) dst[(uint64_t)c * p.ld] = E::OBS_IS_STATE ? g.st[v][c < SD ? c : 0] : g.obs[v][c];
+                }
+                if constexpr (EPISODES)
+                  store_episode<KIND>(p.ep, p.k, (uint64_t)kk * p.ld + base + v, (wf >> (8 * v)) & 0xffu, g.steps[v],
+                                      g.ret[v]);
               }
             }
           }

@@ -62,6 +62,9 @@ class _DeviceArray:
 
 Rollout = namedtuple("Rollout", ["obs", "reward", "flags", "done_count"])
 EpisodeStats = namedtuple("EpisodeStats", ["episodes", "terminated", "truncated", "length_sum", "return_sum"])
+# Return (float32) and length (int32 view of the library's uint32) of every episode that ended, aligned with the
+# flags of the same call: valid only where flags != 0, e.g. `ep.ret[flags != 0]`
+Episodes = namedtuple("Episodes", ["ret", "length"])
 
 
 def _ptr(t):
@@ -172,19 +175,41 @@ class GpuVecEnv:
         if tuple(actions.shape) != tuple(lead) + (self.num_envs,) or not actions.is_contiguous():
             raise ValueError(f"actions must be contiguous with shape {tuple(lead) + (self.num_envs,)}")
 
-    def step(self, actions, want_final_obs=False):
+    def _check_buffer(self, t, name, dtype, shape):
+        if t.dtype != dtype or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != tuple(shape):
+            raise ValueError(f"{name} must be contiguous {str(dtype).replace('torch.', '')} on {self.device} with "
+                             f"shape {tuple(shape)}")
+
+    def step(self, actions, want_final_obs=False, want_episodes=False):
         """Gym::step for all envs.  actions: uint8[N] (Discrete) or float32[N] (Box).
 
         Returns StepInfo(state=[obs_dim, N] f32, reward=[N] f32, done=[N] bool, truncated=[N] bool).
-        The tensors are views of buffers reused by the next call."""
+        The tensors are views of buffers reused by the next call.
+
+        want_final_obs=True also returns final [obs_dim, N], the observation before the auto-reset (dense).
+        want_episodes=True (auto-reset handles) also returns Episodes(ret [N] f32, length [N] i32): the return and
+        length of the episode each env finished in this step (RecordEpisodeStatistics' info["episode"]), the values
+        the statistics add.  Valid only where info.flags != 0, e.g. `ep.ret[info.flags != 0]`; the other entries keep
+        what an earlier step left (the buffers are reused by the next call).  MountainCarContinuous and Pendulum need
+        track_returns=True for ret.  Returns info, (info, final), (info, episodes) or (info, final, episodes)."""
         self._check_actions(actions)
         final = None
         if want_final_obs:
             final = torch.empty_like(self._obs)
-        _lib.check(self._lib.mgym_step(self._h, _ptr(actions), self._p_obs, self._p_reward, self._p_flags, _ptr(final),
-                                       self._stream()))
+        if not want_episodes:
+            _lib.check(self._lib.mgym_step(self._h, _ptr(actions), self._p_obs, self._p_reward, self._p_flags,
+                                           _ptr(final), self._stream()))
+            info = StepInfo(self._obs, self._reward, self._flags)
+            return (info, final) if want_final_obs else info
+        if getattr(self, "_episodes", None) is None:
+            n = self.num_envs
+            self._episodes = Episodes(torch.zeros(n, dtype=torch.float32, device=self.device),
+                                      torch.zeros(n, dtype=torch.int32, device=self.device))
+        ep = self._episodes
+        _lib.check(self._lib.mgym_step_episodes(self._h, _ptr(actions), self._p_obs, self._p_reward, self._p_flags,
+                                                _ptr(final), _ptr(ep.ret), _ptr(ep.length), self._stream()))
         info = StepInfo(self._obs, self._reward, self._flags)
-        return (info, final) if want_final_obs else info
+        return (info, final, ep) if want_final_obs else (info, ep)
 
     def step_raw(self, actions, obs_out=None, reward_out=None, flags_out=None, final_obs_out=None):
         """mgym_step with caller-owned (possibly absent) outputs; returns nothing."""
@@ -192,7 +217,7 @@ class GpuVecEnv:
                                        _ptr(final_obs_out), self._stream()))
 
     def rollout(self, K, actions=None, obs=None, reward=None, flags=None, want_obs=True, count_done=True,
-                final_obs=None, want_final_obs=False):
+                final_obs=None, want_final_obs=False, ep_return=None, ep_length=None, want_episodes=False):
         """K fused steps (the caller's step loop, cartpole.rs:460-471).  actions: [K, N] or None for the
         device-side uniform random policy.  Returns time-major trajectories.
 
@@ -200,11 +225,19 @@ class GpuVecEnv:
         (`final_obs`, or a new buffer) holds the observation each episode ended on, before its auto-reset.  Only the
         entries of envs that finished at that step (flags != 0) are written; the others keep what the buffer held.
         The next observation of every transition is then
-            next_obs = torch.where((out.flags != 0).unsqueeze(1), final_obs, out.obs)"""
+            next_obs = torch.where((out.flags != 0).unsqueeze(1), final_obs, out.obs)
+
+        want_episodes=True (auto-reset handles): also returns Episodes(ret [K, N] f32, length [K, N] i32)
+        (`ep_return` / `ep_length`, or new buffers): the return and length of the episode env i finished at step k,
+        the values the statistics add.  Valid only where out.flags != 0, e.g. `ep.ret[out.flags != 0]`; the other
+        entries keep what the buffers held.  MountainCarContinuous and Pendulum need track_returns=True.  Returns
+        (Rollout, episodes), or (Rollout, final_obs, episodes) with want_final_obs."""
         K = int(K)
         n = self.num_envs
         if final_obs is not None and not want_final_obs:
             raise ValueError("final_obs is the buffer of want_final_obs=True")
+        if (ep_return is not None or ep_length is not None) and not want_episodes:
+            raise ValueError("ep_return / ep_length are the buffers of want_episodes=True")
         if actions is not None:
             self._check_actions(actions, (K,))
         if obs is None and want_obs:
@@ -217,10 +250,23 @@ class GpuVecEnv:
         if want_final_obs:
             if final_obs is None:
                 final_obs = torch.empty((K, self.obs_dim, n), dtype=torch.float32, device=self.device)
-            elif (final_obs.dtype != torch.float32 or final_obs.device != self.device or not final_obs.is_contiguous()
-                  or tuple(final_obs.shape) != (K, self.obs_dim, n)):
-                raise ValueError(f"final_obs must be contiguous float32 on {self.device} with shape "
-                                 f"{(K, self.obs_dim, n)}")
+            else:
+                self._check_buffer(final_obs, "final_obs", torch.float32, (K, self.obs_dim, n))
+        if want_episodes:
+            if ep_return is None:
+                ep_return = torch.empty((K, n), dtype=torch.float32, device=self.device)
+            else:
+                self._check_buffer(ep_return, "ep_return", torch.float32, (K, n))
+            if ep_length is None:
+                ep_length = torch.empty((K, n), dtype=torch.int32, device=self.device)
+            else:
+                self._check_buffer(ep_length, "ep_length", torch.int32, (K, n))
+            _lib.check(self._lib.mgym_rollout_episodes(self._h, K, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(flags),
+                                                       _ptr(final_obs), _ptr(ep_return), _ptr(ep_length), _ptr(dc),
+                                                       self._stream()))
+            out, ep = Rollout(obs, reward, flags, dc), Episodes(ep_return, ep_length)
+            return (out, final_obs, ep) if want_final_obs else (out, ep)
+        if want_final_obs:
             _lib.check(self._lib.mgym_rollout_final(self._h, K, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(flags),
                                                     _ptr(final_obs), _ptr(dc), self._stream()))
             return Rollout(obs, reward, flags, dc), final_obs
@@ -228,25 +274,30 @@ class GpuVecEnv:
                                           self._stream()))
         return Rollout(obs, reward, flags, dc)
 
-    def iter_rollout(self, total_steps, chunk=32, actions=None, want_obs=True, want_final_obs=False):
+    def iter_rollout(self, total_steps, chunk=32, actions=None, want_obs=True, want_final_obs=False,
+                     want_episodes=False):
         """A long rollout (e.g. MountainCar's 1000 steps, BASELINE configs[2]) as fused launches of `chunk` steps
         over ONE reused trajectory ring: the full trajectory of 2^24 envs x 1000 steps would be 218 GB.
         Yields (first_step, Rollout) per launch; the Rollout tensors are overwritten by the next launch.
         actions: None (device policy) or a callable first_step, n_steps -> [n_steps, N] tensor.
         want_final_obs=True yields (first_step, (Rollout, final_obs)) with one reused [chunk, obs_dim, N] final buffer
-        (see rollout: only entries with flags != 0 are valid)."""
+        (see rollout: only entries with flags != 0 are valid).  want_episodes=True appends Episodes to that tuple,
+        over one reused [chunk, N] pair (valid only where flags != 0: `ep.ret[out.flags != 0]`)."""
         n, K = self.num_envs, int(chunk)
         obs = torch.empty((K, self.obs_dim, n), dtype=torch.float32, device=self.device) if want_obs else None
         reward = torch.empty((K, n), dtype=torch.float32, device=self.device)
         flags = torch.empty((K, n), dtype=torch.uint8, device=self.device)
         final = torch.empty((K, self.obs_dim, n), dtype=torch.float32, device=self.device) if want_final_obs else None
+        ep_ret = torch.empty((K, n), dtype=torch.float32, device=self.device) if want_episodes else None
+        ep_len = torch.empty((K, n), dtype=torch.int32, device=self.device) if want_episodes else None
         done = 0
         while done < total_steps:
             k = min(K, total_steps - done)
             a = None if actions is None else actions(done, k)
             out = self.rollout(k, a, obs=None if obs is None else obs[:k], reward=reward[:k], flags=flags[:k],
                                want_obs=want_obs, final_obs=None if final is None else final[:k],
-                               want_final_obs=want_final_obs)
+                               want_final_obs=want_final_obs, ep_return=None if ep_ret is None else ep_ret[:k],
+                               ep_length=None if ep_len is None else ep_len[:k], want_episodes=want_episodes)
             yield done, out
             done += k
 
