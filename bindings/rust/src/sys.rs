@@ -69,6 +69,8 @@ extern "C" {
                           stream: *mut c_void) -> c_int;
     pub fn mgym_get_obs(env: *mut mgym_env, obs_out: *mut f32, stream: *mut c_void) -> c_int;
     pub fn mgym_state_ptr(env: *mut mgym_env) -> *mut f32;
+    pub fn mgym_reward_ptr(env: *mut mgym_env) -> *mut f32;
+    pub fn mgym_reward_constant(env: *mut mgym_env, value: *mut f32) -> c_int;
     pub fn mgym_checkpoint_size(env: *const mgym_env) -> usize;
     pub fn mgym_checkpoint_save(env: *mut mgym_env, blob: *mut c_void, bytes: usize, stream: *mut c_void) -> c_int;
     pub fn mgym_checkpoint_load(env: *mut mgym_env, blob: *const c_void, bytes: usize, stream: *mut c_void) -> c_int;

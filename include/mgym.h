@@ -177,6 +177,18 @@ int mgym_get_obs(mgym_env *env, float *obs_out, void *stream); /* current observ
 /* Zero-copy view of the resident state rows ([state_dim][N]); for kinds whose observation is the
  * state (CartPole, MountainCar, MountainCarContinuous) this IS the observation buffer. */
 float *mgym_state_ptr(mgym_env *env);
+/* The handle's own reward row, device float[N], allocated with the handle and freed by mgym_destroy: pass it as
+ * reward_out of mgym_step / mgym_step_episodes.  On a handle whose rewards are all one value (mgym_reward_constant
+ * returns 1) the row is filled with that value at creation and a step given the row stores nothing into it (4 bytes
+ * per env-step less); no reset, state or parameter change, checkpoint load or graph replay writes it either, so what a
+ * caller writes into it stays.  On any other handle every step given the row writes it, like any caller buffer.  Any
+ * other reward_out is written by every step on every handle. */
+float *mgym_reward_ptr(mgym_env *env);
+/* 1 and *value (may be NULL) = the reward when every reward this handle's steps can produce is that one value:
+ * CartPole-v1 with auto_reset = 1 and sutton_barto_reward = 0 (1.0), MountainCar-v0 (-1.0).  0 for every other kind
+ * or configuration (*value untouched); MGYM_ERR_BAD_ARGUMENT for a NULL handle.  Parameters and redraws do not change
+ * the answer: they change the physics only. */
+int mgym_reward_constant(mgym_env *env, float *value);
 
 /* Checkpoint / resume: the whole handle (state rows, counters, running returns, statistics, step and reset
  * indices, per-env parameters and redraw ranges if set) as one opaque HOST blob.  mgym_checkpoint_size gives the byte

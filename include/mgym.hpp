@@ -275,7 +275,8 @@ class GpuVecEnv {
     check(mgym_create(kind, n, device, seed, &cfg, &h_));
     check_cuda(cudaSetDevice(device), "cudaSetDevice");
     check_cuda(cudaMalloc(reinterpret_cast<void**>(&obs_), sizeof(float) * obs_dim() * n), "cudaMalloc obs");
-    check_cuda(cudaMalloc(reinterpret_cast<void**>(&reward_), sizeof(float) * n), "cudaMalloc reward");
+    // the handle's own reward row: a constant-reward handle's steps store nothing into it (mgym_reward_ptr)
+    reward_ = mgym_reward_ptr(h_);
     check_cuda(cudaMalloc(reinterpret_cast<void**>(&flags_), n), "cudaMalloc flags");
   }
   std::vector<float> download(const float* dev, size_t count) {
@@ -287,7 +288,6 @@ class GpuVecEnv {
   void release() {
     if (h_) mgym_destroy(h_);
     if (obs_) cudaFree(obs_);
-    if (reward_) cudaFree(reward_);
     if (flags_) cudaFree(flags_);
     if (act_) cudaFree(act_);
     h_ = nullptr, obs_ = nullptr, reward_ = nullptr, flags_ = nullptr, act_ = nullptr;

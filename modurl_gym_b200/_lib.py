@@ -74,6 +74,8 @@ SYMBOLS = {
     "mgym_get_state": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "mgym_get_obs": (_i, [_vp, _vp, _vp]),
     "mgym_state_ptr": (_vp, [_vp]),
+    "mgym_reward_ptr": (_vp, [_vp]),
+    "mgym_reward_constant": (_i, [_vp, C.POINTER(C.c_float)]),
     "mgym_checkpoint_size": (C.c_size_t, [_vp]),
     "mgym_checkpoint_save": (_i, [_vp, _vp, C.c_size_t, _vp]),
     "mgym_checkpoint_load": (_i, [_vp, _vp, C.c_size_t, _vp]),

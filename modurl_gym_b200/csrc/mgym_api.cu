@@ -47,6 +47,11 @@ struct mgym_env {
   bool vec4 = false;  // n % 4 == 0 and env_index_base % 4 == 0
 
   float* state = nullptr;
+  // the handle's own reward row [n] (mgym_reward_ptr).  Where every reward is one value (reward_const) it is filled
+  // with that value at creation and a step given the row stores nothing into it.
+  float* reward = nullptr;
+  bool reward_const = false;
+  float reward_value = 0.0f;
   void* steps = nullptr;
   uint32_t* sbt = nullptr;
   float* ep_return = nullptr;
@@ -198,6 +203,22 @@ EnvConsts make_consts(int kind, const mgym_config& cfg) {
   return k;
 }
 
+// Whether every reward a step of this configuration can produce is one value, read off the constants the kernels use
+// (Env<KIND>::outcome).  CartPole: truncated ? R_TRUNCATED : !terminated ? r_alive : fresh ? r_fell : r_after, where an
+// auto-reset env is always fresh (it is reset in the step that ends its episode, so r_after never occurs).
+// MountainCar-v0: one constant.  Every other kind or configuration has rewards that depend on the step.
+bool constant_reward(int kind, const mgym_config& cfg, const EnvConsts& k, float* value) {
+  if (kind == MGYM_CARTPOLE_V1 && cfg.auto_reset && k.r_alive == k.r_fell && k.r_alive == Env<0>::R_TRUNCATED) {
+    *value = Env<0>::R_TRUNCATED;
+    return true;
+  }
+  if (kind == MGYM_MOUNTAIN_CAR_V0) {
+    *value = Env<1>::REWARD;
+    return true;
+  }
+  return false;
+}
+
 KernelParams base_params(const mgym_env* e) {
   KernelParams p{};
   p.state = e->state;
@@ -264,12 +285,13 @@ int launch_persistent(void (*kernel)(KP), const mgym_env* e, const KP& p, uint64
 }
 
 // TMA-staged step kernel (auto-reset, vector path, N a multiple of the 128-env warp tile)
-template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false>
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false,
+          bool REWARD = true>
 int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW, EPISODES>& p_in, cudaStream_t st) {
   mgym_env* e = const_cast<mgym_env*>(ce);  // ticket accounting
   KParams<PARAMS, REDRAW, EPISODES> p = p_in;
   using L = TmaLayout<KIND, CNT, AUTO, PARAMS>;
-  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS, REDRAW, EPISODES>;
+  auto kernel = step_kernel_tma<KIND, CNT, AUTO, PARAMS, REDRAW, EPISODES, REWARD>;
   constexpr int threads = TMA_THREADS;
   // the opt-in to > 48 KB of dynamic shared memory and the occupancy are per device
   static int cached_per_sm[kMaxDevices] = {};
@@ -316,27 +338,31 @@ int launch_step_tma(const mgym_env* ce, const KParams<PARAMS, REDRAW, EPISODES>&
 // kind x vector width x auto/manual x counter representation (x per-env parameters (x per-episode redraw: auto-reset
 // handles only, the host never asks for a manual form of it)) (x final observations: auto-reset rollouts only,
 // mgym_rollout_final refuses manual handles before it gets here) (x episode outputs: auto-reset steps and rollouts,
-// mgym_step_episodes / mgym_rollout_episodes refuse manual handles)
+// mgym_step_episodes / mgym_rollout_episodes refuse manual handles) (x REWARD = false: steps of constant-reward
+// handles that store no reward, see dispatch_width)
 template <int KIND, int V, bool ROLLOUT, bool PARAMS = false, bool REDRAW = false, bool FINAL = false,
-          bool EPISODES = false>
+          bool EPISODES = false, bool REWARD = true>
 int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW, EPISODES>& p, cudaStream_t st) {
   static_assert(!FINAL || ROLLOUT, "final observations are a rollout form");
   static_assert(!(FINAL && EPISODES), "the EPISODES rollout forms store final observations themselves");
+  static_assert(REWARD || !ROLLOUT, "the reward-less forms are step forms");
   const uint64_t groups = p.n / V;
   const bool autor = e->cfg.auto_reset != 0;
   if constexpr (!ROLLOUT && V == 4) {
     // manual mode (the reference's protocol): counters are 32-bit, CartPole adds steps_beyond_terminated
-    if constexpr (!REDRAW && !EPISODES) {
-      if (!autor && p.n % TMA_TILE == 0) return launch_step_tma<KIND, CNT_U32, false, PARAMS>(e, p, st);
+    if constexpr (!REDRAW && !EPISODES && (REWARD || has_constant_reward(KIND, false))) {
+      if (!autor && p.n % TMA_TILE == 0)
+        return launch_step_tma<KIND, CNT_U32, false, PARAMS, false, false, REWARD>(e, p, st);
     }
     if (autor && p.n % TMA_TILE == 0) {
       if constexpr (KIND == 0) {  // CartPole's handles are all CNT_S16 (500-step truncation, cartpole.rs:297)
-        return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW, EPISODES>(e, p, st);
+        return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW, EPISODES, REWARD>(e, p, st);
       } else {
         switch (e->cnt_mode) {
-          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW, EPISODES>(e, p, st);
-          case CNT_S32_LAZY: return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS, REDRAW, EPISODES>(e, p, st);
-          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS, REDRAW, EPISODES>(e, p, st);
+          case CNT_S16: return launch_step_tma<KIND, CNT_S16, true, PARAMS, REDRAW, EPISODES, REWARD>(e, p, st);
+          case CNT_S32_LAZY:
+            return launch_step_tma<KIND, CNT_S32_LAZY, true, PARAMS, REDRAW, EPISODES, REWARD>(e, p, st);
+          default: return launch_step_tma<KIND, CNT_S32, true, PARAMS, REDRAW, EPISODES, REWARD>(e, p, st);
         }
       }
     }
@@ -347,9 +373,9 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW, EPISODES>& p,
       head.n = p.n - p.n % TMA_TILE;
       tail.first = p.first + head.n;
       tail.n = p.n - head.n;
-      int rc = dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES>(e, head, st);
+      int rc = dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES, REWARD>(e, head, st);
       if (rc != MGYM_OK) return rc;
-      return dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES>(e, tail, st);
+      return dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES, REWARD>(e, tail, st);
     }
   }
   // rollout_kernel's FULL form: complete warp tiles and all three trajectory outputs
@@ -366,10 +392,11 @@ int dispatch_mode(const mgym_env* e, const KParams<PARAMS, REDRAW, EPISODES>& p,
       return launch_persistent(rollout_kernel<KIND, V, AUTO_, CNT_, false, PARAMS, REDRAW, FINAL, EPISODES>, e, p, \
                                groups, st);                                                              \
     } else {                                                                                             \
-      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS, REDRAW, EPISODES>, e, p, groups, st); \
+      return launch_persistent(step_kernel<KIND, V, AUTO_, CNT_, PARAMS, REDRAW, EPISODES, REWARD>, e, p, groups, \
+                               st);                                                                      \
     }                                                                                                    \
   } while (0)
-  if constexpr (!REDRAW && !FINAL && !EPISODES) {
+  if constexpr (!REDRAW && !FINAL && !EPISODES && (REWARD || has_constant_reward(KIND, false))) {
     if (!autor) MGYM_LAUNCH(false, CNT_U32);
   }
   if constexpr (KIND == 0) {
@@ -394,13 +421,19 @@ ParamBox redraw_box(const mgym_env* e) {
 }
 
 // A handle with per-env parameters runs the PARAMS instantiations (kinds that have parameters only), an auto-reset
-// one with redraw ranges the PARAMS + REDRAW instantiations (manual-mode steps never reset).
+// one with redraw ranges the PARAMS + REDRAW instantiations (manual-mode steps never reset).  A step of a handle whose
+// rewards are all one value that stores no reward (its own row, or none asked for) runs the REWARD = false forms.
 template <int KIND, bool ROLLOUT, bool FINAL, bool EPISODES, bool PARAMS, bool REDRAW>
 int dispatch_width(const mgym_env* e, const KParamsBase<PARAMS, REDRAW>& pb, const EpisodeOut& ep, bool vec4,
                    cudaStream_t st) {
   KParams<PARAMS, REDRAW, EPISODES> p;
   static_cast<KParamsBase<PARAMS, REDRAW>&>(p) = pb;
   if constexpr (EPISODES) p.ep = ep;
+  if constexpr (!ROLLOUT && has_constant_reward(KIND, true)) {
+    if (e->reward_const && !p.reward_out)
+      return vec4 ? dispatch_mode<KIND, 4, false, PARAMS, REDRAW, false, EPISODES, false>(e, p, st)
+                  : dispatch_mode<KIND, 1, false, PARAMS, REDRAW, false, EPISODES, false>(e, p, st);
+  }
   return vec4 ? dispatch_mode<KIND, 4, ROLLOUT, PARAMS, REDRAW, FINAL, EPISODES>(e, p, st)
               : dispatch_mode<KIND, 1, ROLLOUT, PARAMS, REDRAW, FINAL, EPISODES>(e, p, st);
 }
@@ -631,6 +664,7 @@ int mgym_destroy(mgym_env* e) {
   DeviceGuard guard(e->device);
   cudaFree(e->clock);
   cudaFree(e->state);
+  cudaFree(e->reward);
   cudaFree(e->steps);
   cudaFree(e->sbt);
   cudaFree(e->ep_return);
@@ -683,6 +717,7 @@ int mgym_create(int kind, uint64_t num_envs, int device_ordinal, uint64_t seed, 
   e->seed = seed;
   e->cfg = cfg;
   e->k = make_consts(kind, cfg);
+  e->reward_const = constant_reward(kind, cfg, e->k, &e->reward_value);
   e->vec4 = (num_envs % 4 == 0) && (cfg.env_index_base % 4 == 0);
 
   // counter representation (DESIGN.md section 4, CounterMode in mgym_kernels.cuh)
@@ -709,6 +744,15 @@ int mgym_create(int kind, uint64_t num_envs, int device_ordinal, uint64_t seed, 
     const size_t n = (size_t)num_envs;
     MGYM_CUDA(cudaMalloc(&e->state, sizeof(float) * kStateDim[kind] * n));
     MGYM_CUDA(cudaMemset(e->state, 0, sizeof(float) * kStateDim[kind] * n));  // cartpole.rs:85 zero state
+    MGYM_CUDA(cudaMalloc(&e->reward, sizeof(float) * n));
+    if (e->reward_const) {  // the only write the row of a constant-reward handle ever gets from the library
+      uint32_t bits;
+      memcpy(&bits, &e->reward_value, sizeof(bits));
+      fill_u32_kernel<<<(unsigned)((n + 255) / 256), 256>>>(reinterpret_cast<uint32_t*>(e->reward), bits, n);
+      MGYM_CUDA(cudaGetLastError());
+    } else {
+      MGYM_CUDA(cudaMemset(e->reward, 0, sizeof(float) * n));
+    }
     // count 0, or start stamp 0 = the handle's step index right now
     MGYM_CUDA(cudaMalloc(&e->steps, counter_width(e->cnt_mode) * n));
     MGYM_CUDA(cudaMemset(e->steps, 0, counter_width(e->cnt_mode) * n));
@@ -761,6 +805,12 @@ uint64_t mgym_step_index(const mgym_env* ce) {
   return e->t;
 }
 float* mgym_state_ptr(mgym_env* e) { return e ? e->state : nullptr; }
+float* mgym_reward_ptr(mgym_env* e) { return e ? e->reward : nullptr; }
+int mgym_reward_constant(mgym_env* e, float* value) {
+  if (!e) return fail(MGYM_ERR_BAD_ARGUMENT, "mgym_reward_constant: env is NULL");
+  if (e->reward_const && value) *value = e->reward_value;
+  return e->reward_const ? 1 : 0;
+}
 
 // ---------------------------------------------------------------------------------------------
 // reset
@@ -1099,7 +1149,8 @@ static int run_step(const char* fn, mgym_env* e, const void* actions, float* obs
   p.actions = actions;
   // zero-copy observation: for kinds whose observation is the state, obs_out == state rows is a no-op
   p.obs_out = (obs_out == e->state) ? nullptr : obs_out;
-  p.reward_out = reward_out;
+  // zero-copy reward: the row of a constant-reward handle already holds every reward a step can produce
+  p.reward_out = (reward_out == e->reward && e->reward_const) ? nullptr : reward_out;
   p.flags_out = flags_out;
   p.final_obs_out = final_obs_out;
   p.adv_clock = e->cfg.device_clock ? e->clock : nullptr;

@@ -55,6 +55,10 @@ __host__ __device__ constexpr bool cnt_is_stamp(int c) { return c >= CNT_S16; }
 __host__ __device__ constexpr bool cnt_is_lazy(int c) { return c == CNT_S32_LAZY; }
 __host__ __device__ constexpr bool cnt_staged(int c) { return c != CNT_S32_LAZY; }  // read by every step
 
+// The kinds and modes whose handles can have every reward equal to one value (constant_reward in mgym_api.cu): only
+// these instantiate the step forms without a reward (REWARD = false)
+__host__ __device__ constexpr bool has_constant_reward(int kind, bool autor) { return kind == 1 || (kind == 0 && autor); }
+
 struct KernelParams {
   // resident env state (owned by the handle)
   float* state;        // [SD][n]
@@ -683,7 +687,9 @@ __device__ __forceinline__ typename CounterType<CNT>::type cnt_encode(uint32_t s
 // REDRAW: every reset also redraws the env's parameter rows (mgym_set_param_redraw; auto-reset with rows only).
 // EPISODES (mgym_step_episodes, auto-reset only): step_group's tally also stores each finished env's episode return
 // and length.
-template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false>
+// REWARD = false (handles whose rewards are all one value, given no reward buffer): no reward is computed or stored.
+template <int KIND, int V, bool AUTO, int CNT, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false,
+          bool REWARD = true>
 __global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KParams<PARAMS, REDRAW, EPISODES> p) {
   using E = Env<KIND>;
   using act_t = typename E::act_t;
@@ -693,6 +699,7 @@ __global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KP
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(!EPISODES || AUTO, "episodes end only where the step resets");
   static_assert(!cnt_is_lazy(CNT) && (AUTO || !cnt_is_stamp(CNT)), "the host maps CNT_S32_LAZY to CNT_S32 here");
+  static_assert(REWARD || has_constant_reward(KIND, AUTO), "only constant-reward handles skip the reward");
   StatAcc acc;
   const uint64_t groups = p.n / V;
   const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -788,7 +795,7 @@ __global__ void __launch_bounds__(256, 1) step_kernel(const __grid_constant__ KP
         stv<float, V>(p.final_obs_out + (uint64_t)c * p.ld + base, o);
       }
     }
-    if (p.reward_out) {
+    if (REWARD && p.reward_out) {
       Vec<float, V> rw;
 #pragma unroll
       for (int v = 0; v < V; ++v) rw.v[v] = g.reward[v];
@@ -913,7 +920,11 @@ struct TmaLayout {
 //
 // EPISODES (mgym_step_episodes, auto-reset only): the consumers' branch for finished envs also stores each one's
 // episode return and length, where the statistics read them (after the lazy stamp decode, before they are cleared).
-template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false>
+//
+// REWARD = false (a handle whose rewards are all one value, stepped into its own reward row, which already holds that
+// value; or given no reward buffer): no reward is selected, tested for or stored -- 4 bytes less per env-step.
+template <int KIND, int CNT, bool AUTO = true, bool PARAMS = false, bool REDRAW = false, bool EPISODES = false,
+          bool REWARD = true>
 __global__ void __launch_bounds__(TMA_THREADS, 2)
     step_kernel_tma(const __grid_constant__ KParams<PARAMS, REDRAW, EPISODES> p) {
   using E = Env<KIND>;
@@ -926,6 +937,7 @@ __global__ void __launch_bounds__(TMA_THREADS, 2)
   static_assert(!REDRAW || (PARAMS && AUTO), "redraw is a form of the auto-reset parameter kernels");
   static_assert(AUTO || !cnt_is_stamp(CNT), "manual mode keeps the reference's own counters");
   static_assert(!EPISODES || AUTO, "episodes end only where the step resets");
+  static_assert(REWARD || has_constant_reward(KIND, AUTO), "only constant-reward handles skip the reward");
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (tma::smem_u32(smem_raw) + 127u) & ~127u;
   const uint32_t warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);  // warp-uniform for the compiler
@@ -1196,7 +1208,7 @@ __global__ void __launch_bounds__(TMA_THREADS, 2)
           stv<float, V>(p.final_obs_out + (uint64_t)c * p.ld + base, o);
         }
       }
-      if (p.reward_out) {
+      if (REWARD && p.reward_out) {
         Vec<float, V> rw;
 #pragma unroll
         for (int v = 0; v < V; ++v) rw.v[v] = g.reward[v];

@@ -117,7 +117,15 @@ class GpuVecEnv:
         self._act_space = spaces.action_space(self.kind)
         n = self.num_envs
         with torch.cuda.device(self.device):
-            self._reward = torch.empty(n, dtype=torch.float32, device=self.device)
+            # the handle's own reward row [N].  Where every reward is one value (CartPole-v1 with auto-reset and the
+            # default rewards, MountainCar-v0) the library filled it at creation and a step given it stores nothing
+            # (36 instead of 40 bytes per CartPole env-step); reward_constant is that value, else None
+            self._reward = torch.as_tensor(_DeviceArray(self._lib.mgym_reward_ptr(self._h), (n,)), device=self.device)
+            value = C.c_float()
+            rc = self._lib.mgym_reward_constant(self._h, C.byref(value))
+            if rc < 0:
+                _lib.check(rc)
+            self.reward_constant = value.value if rc == 1 else None
             self._flags = torch.empty(n, dtype=torch.uint8, device=self.device)
             # the resident state rows [state_dim, N] as a tensor (valid while this env is open)
             self.state_view = torch.as_tensor(_DeviceArray(self._lib.mgym_state_ptr(self._h), (self.state_dim, n)),
@@ -134,7 +142,8 @@ class GpuVecEnv:
 
     # -- lifecycle ---------------------------------------------------------------------------
     def close(self):
-        """Frees the handle; `state_view` (and observations returned for obs_is_state kinds) dangle afterwards."""
+        """Frees the handle; `state_view`, observations returned for obs_is_state kinds and rewards returned by step
+        dangle afterwards."""
         if getattr(self, "_h", None) is not None and self._h:
             self._lib.mgym_destroy(self._h)
             self._h = C.c_void_p()
@@ -184,7 +193,10 @@ class GpuVecEnv:
         """Gym::step for all envs.  actions: uint8[N] (Discrete) or float32[N] (Box).
 
         Returns StepInfo(state=[obs_dim, N] f32, reward=[N] f32, done=[N] bool, truncated=[N] bool).
-        The tensors are views of buffers reused by the next call.
+        The tensors are views of buffers reused by the next call.  For obs_is_state kinds `state` is `state_view`, the
+        resident state rows.  `reward` is a view of the handle's reward row; on a handle whose rewards are all one
+        value (reward_constant is not None) that row is filled once at creation and no step stores into it, so it is
+        live: writing into it changes what later steps return.
 
         want_final_obs=True also returns final [obs_dim, N], the observation before the auto-reset (dense).
         want_episodes=True (auto-reset handles) also returns Episodes(ret [N] f32, length [N] i32): the return and
